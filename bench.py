@@ -2,7 +2,7 @@
 """bench.py -- agent-steps/s of the swarm hot path (world step + per-step graph + GAT-Q forward + greedy
 argmax) on N B200s, next to the reference-structured CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1] / SURVEY.md 8d "C2"): ObstacleAvoidance, 12 agents, 4 096 envs per GPU,
@@ -11,6 +11,10 @@ complete graph + (0,0) self loop (E = 133), weights of experiment_ObstacleAvoida
 episode of all envs: reset_grid launch + one fused rollout launch (state stays on chip for the 100 ticks).
 ``value`` is timed with the inputs resident in HBM; ``e2e`` goes through the public API with pinned host
 buffers (centres in, per-agent returns + per-env hit counts out) inside the timed region.
+``--dump-outputs DIR`` writes what the last timed ``e2e`` step handed back to its caller (rank 0's envs) as
+``DIR/state.npy`` f32[B,N,4], ``DIR/returns.npy`` f32[B,N] and ``DIR/hits.npy`` f64[B]: the inputs are seeded, so
+two builds run with the same arguments can be compared output for output.  The ``e2e`` leg runs the same rollout from
+the same centres as the ``value`` leg, whose returns and hits buffers instead accumulate over all its steps.
 """
 from __future__ import annotations
 
@@ -272,6 +276,9 @@ def run_ours(args):
     barrier()
     kernel_ms = sum(a.elapsed_time(b) for a, b in kev) / args.steps
     ms_e2e = timed(step_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"state": pack_host[:B * N * 4].view(B, N, 4), "returns": returns_host,
+                                         "hits": pack_host[B * N * 5:].view(torch.int32)})
     dqn_stats = measure_dqn(sb, ops, dev, cfg, weights, centers, dist, barrier, stream, rank, world)
     strong = None
     if world > 1:
@@ -353,6 +360,14 @@ def run_ours(args):
     emit(line)
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(where: str, arrays: dict) -> None:
+    """Each host tensor as ``where/<name>.npy``: float32 stays float32, integers become float64 (exact)."""
+    os.makedirs(where, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.numpy()
+        np.save(os.path.join(where, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 def measure_extra(sb, ops, dev):
@@ -616,7 +631,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed e2e step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     # stdout carries exactly ONE JSON line: everything else a library prints there (e.g. NCCL's version banner)
     # is diverted to stderr; the JSON line is written to the original descriptor at the end.
     global _JSON_OUT

@@ -3,7 +3,7 @@ dependencies (oracle/refstub: vmas / torch_geometric restated with the pinned or
 
     python tests/golden/make_reference_runs.py        ->  tests/golden/reference_runs.npz
 
-Needs the reference sources (/root/reference, or the staged copy tests/_refsrc).  What is recorded:
+Needs the reference sources (the copy build() stages into oracle/_ref).  What is recorded:
 
   flocking/n{N}/..., cohesion/n{N}/...
       FlockingScenario / CohesionScenario (src/scenarios/flocking_scenario.py, cohesion_scenario.py) stepped through

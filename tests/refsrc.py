@@ -1,8 +1,9 @@
 """Locating and importing the reference's OWN Python files (unmodified) on top of a stand-in for its two pip
 dependencies: ``oracle/refstub`` (CPU, pinned oracle arithmetic) or ``shim`` (the CUDA product).
 
-The sources are read from the git-ignored staging copy ``tests/_refsrc`` (scripts/stage_reference.py; travels to the
-GPU box) or, in the build container, straight from ``/root/reference``.
+The sources are not part of this repository: ``__graft_entry__.build()`` stages them from the reference checkout
+(scripts/stage_reference.py) into the git-ignored ``oracle/_ref``, and they are read from there.  Where no checkout was
+present at build time, the tests that execute them skip.
 """
 import contextlib
 import hashlib
@@ -12,7 +13,7 @@ import os
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-STAGED = os.path.join(ROOT, "tests", "_refsrc")
+STAGED = os.path.join(ROOT, "oracle", "_ref")
 BACKENDS = {"refstub": os.path.join(ROOT, "oracle", "refstub"), "shim": os.path.join(ROOT, "shim")}
 _REF_MODULES = ("go_to_position_scenario", "obstacle_avoidance_scenario", "flocking_scenario", "cohesion_scenario",
                 "train_gcn_dqn", "simulator")
@@ -26,8 +27,6 @@ def reference_root():
             if hashlib.sha256(open(os.path.join(STAGED, rel), "rb").read()).hexdigest() != digest:
                 raise AssertionError(f"staged reference file {rel} was modified after staging")
         return STAGED
-    if os.path.isdir("/root/reference/src"):
-        return "/root/reference"
     return None
 
 
@@ -44,7 +43,7 @@ def reference_modules(backend: str):
     imported fresh with ``vmas`` / ``torch_geometric`` resolving to the chosen stand-in."""
     root = reference_root()
     if root is None:
-        raise FileNotFoundError("reference sources not staged (run scripts/stage_reference.py where /root/reference exists)")
+        raise FileNotFoundError("reference sources not staged in oracle/_ref (build() stages them where the checkout exists)")
     paths = [BACKENDS[backend], os.path.join(root, "src", "scenarios"), os.path.join(root, "src", "training"),
              os.path.join(root, "src", "simulation")]
     saved = list(sys.path)

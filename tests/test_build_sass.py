@@ -14,12 +14,14 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 @pytest.fixture(scope="module")
 def sass():
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
     import swarm_b200 as sb
+    # cuobjdump ships beside nvcc, which the build also finds when the CUDA bin directory is not on PATH
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(sb._build._nvcc()), "cuobjdump")
+    if not os.path.exists(cuobjdump):
+        pytest.skip("cuobjdump not found")
     lib = sb._build.build()
-    elfs = subprocess.run(["cuobjdump", "-lelf", lib], capture_output=True, text=True, check=True).stdout
-    text = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
+    elfs = subprocess.run([cuobjdump, "-lelf", lib], capture_output=True, text=True, check=True).stdout
+    text = subprocess.run([cuobjdump, "-sass", lib], capture_output=True, text=True, check=True).stdout
     funcs, cur = {}, None
     for line in text.splitlines():
         m = re.search(r"Function : (\S+)", line)

@@ -5,7 +5,7 @@ hard-coded `device='cpu'` (train_gcn_dqn.py:262, tests/test_*.py:33) from the B2
 host tensors, `env.step` is `swarm_sim_step`, `GATConv` is the CUDA layer (forward and backward).  The expected outputs
 are what the SAME files produce on the CPU stand-ins of their dependencies (oracle/refstub; tests/golden/
 make_reference_runs.py -> tests/golden/reference_runs.npz), which in turn reproduce the reference's shipped goldens
-(tests/test_refstub.py).  The sources come from the git-ignored staging copy tests/_refsrc (scripts/stage_reference.py).
+(tests/test_refstub.py).  The sources come from the git-ignored staging copy oracle/_ref (scripts/stage_reference.py).
 """
 import os
 import re

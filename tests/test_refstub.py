@@ -5,7 +5,7 @@
     with -- the shipped simulator.py:19 says 10, SURVEY.md Appendix B);
   * the committed fixture tests/golden/reference_runs.npz (what the reference's Flocking / Cohesion reward() source
     and its scripts produce) is reproducible from the sources.
-Skipped where the reference sources are neither staged (tests/_refsrc) nor present (/root/reference).
+Skipped where build() found no reference checkout to stage into oracle/_ref.
 """
 import os
 
