@@ -64,15 +64,22 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
 
-// bounded wait (a lost arrival traps instead of hanging the GPU)
+__device__ __forceinline__ uint32_t mbar_try_wait(uint64_t* bar, uint32_t parity) {
+  uint32_t done;
+  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+               : "=r"(done)
+               : "r"(smem_u32(bar)), "r"(parity)
+               : "memory");
+  return done;
+}
+
+// bounded wait (a lost arrival traps instead of hanging the GPU).  The first try_wait sits outside the counted loop:
+// it suspends the thread until the phase completes or a hardware time limit passes, which covers the usual wait, so
+// the counter and the trap test stay off the common path.
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
+  if (mbar_try_wait(bar, parity)) return;
   uint32_t done = 0;
-  for (int it = 0; it < (1 << 26) && !done; ++it) {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done)
-                 : "r"(smem_u32(bar)), "r"(parity)
-                 : "memory");
-  }
+  for (int it = 0; it < (1 << 26) && !done; ++it) done = mbar_try_wait(bar, parity);
   if (!done) __trap();
 }
 

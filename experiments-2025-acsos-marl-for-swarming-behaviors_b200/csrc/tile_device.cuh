@@ -52,10 +52,13 @@ __device__ __forceinline__ TileThread tile_thread(int n_agents, int epb, long lo
 }
 
 // One world step for the agent of this thread: action decode, contact forces (obstacle first, then
-// agents in entity order), integration.  `pos` = pre-step states of the tile.
+// agents in entity order), integration.  `pos` = pre-step states of the tile.  NT: swarm size at compile time (0 = the
+// run-time value), so that the partner sweep unrolls.
+template <int NT = 0>
 __device__ __forceinline__ void tile_world_step(const TileParams& p, const TileThread& t, const float4* pos, int action,
                                                 float4& s, uint8_t& flags, uint32_t& cmask) {
   const SwarmConfig& c = p.cfg;
+  const int N = NT > 0 ? NT : c.n_agents;
   float fx, fy, gx, gy;
   decode_action(action, fx, fy);          // F = 0 + u
   if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
@@ -68,7 +71,7 @@ __device__ __forceinline__ void tile_world_step(const TileParams& p, const TileT
       }
     }
   }
-  agent_contacts(pos + t.envbase, c.n_agents, t.i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin,
+  agent_contacts(pos + t.envbase, N, t.i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin,
                  fx, fy, cmask);
   integrate(s, fx, fy, c.dt, p.one_minus_drag);
 }

@@ -26,7 +26,11 @@ namespace swarm {
 // NT: swarm size as a compile-time constant (0 = the run-time value): index arithmetic, attention loops and the partner
 // sweep of the shapes the reference's experiments use unroll completely (the streaming world step gained 25-40 % from
 // the same specialisation).
-template <int MODE, bool TC, bool DENSE, bool FLOCK = false, int NT = 0>
+// PLAIN (MODE_ROLLOUT, TC only): the greedy evaluation rollout -- complete graph, no trace, no replay push, no forced
+// actions, no device-side control block, epsilon 0 (launch_tile_q checks all of it).  The kNN / radius paths, the
+// other attention heads and every per-tick test of an optional pointer are compiled out, which leaves the tick a
+// straight line of about a quarter of the generic kernel's code.  Same arithmetic, same bits.
+template <int MODE, bool TC, bool DENSE, bool FLOCK = false, int NT = 0, bool PLAIN = false>
 __global__ void __launch_bounds__(kTileThreads, (MODE == MODE_GRAPH || MODE == MODE_STEP) ? 8 : ((TC && !DENSE) ? 3 : 4))
 tile_kernel(const __grid_constant__ TileParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
@@ -37,9 +41,10 @@ tile_kernel(const __grid_constant__ TileParams p) {
   const SwarmConfig& c = p.cfg;
   const int T = kTileThreads;
   const int N = NT > 0 ? NT : c.n_agents;
+  static_assert(!PLAIN || (MODE == MODE_ROLLOUT && TC && !FLOCK), "PLAIN is the tensor-core greedy rollout");
   const int K = c.knn_k;
-  const bool knn = (c.graph_mode == SWARM_GRAPH_KNN) && (kQ || MODE == MODE_GRAPH);
-  const bool radius = (c.graph_mode == SWARM_GRAPH_RADIUS) && (kQ || MODE == MODE_GRAPH);
+  const bool knn = !PLAIN && (c.graph_mode == SWARM_GRAPH_KNN) && (kQ || MODE == MODE_GRAPH);
+  const bool radius = !PLAIN && (c.graph_mode == SWARM_GRAPH_RADIUS) && (kQ || MODE == MODE_GRAPH);
   const TileThread t = tile_thread(N, p.epb, c.num_envs, p.bal_q, p.bal_r);
   const int tid = t.tid;
   const long long BN = (long long)c.num_envs * N;
@@ -69,7 +74,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
   if (FLOCK && t.active) shp = p.shaping[t.gidx];
   float epsilon = p.epsilon;
   long long rng_tick0 = p.rng_tick0, replay_cursor = p.replay_cursor;
-  if (MODE == MODE_ROLLOUT && p.ctl) {
+  if (MODE == MODE_ROLLOUT && !PLAIN && p.ctl) {
     epsilon = p.ctl->epsilon;
     rng_tick0 = p.ctl->tick + 1;
     replay_cursor = p.ctl->ring_cursor;
@@ -109,8 +114,9 @@ tile_kernel(const __grid_constant__ TileParams p) {
   float ret = 0.0f;
   int myhits = 0;
 
-
+  SWARM_PHASE_RESET();
   for (int tick = 0; tick < p.ticks; ++tick) {
+    SWARM_PHASE_START();
     const float4* pos = sst + (tick & 1) * T;
     sst[(tick & 1) * T + tid] = s;
     float adst_tc = 0.0f;
@@ -122,6 +128,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
       g.sas[tid] = asrc;
     }
     __syncthreads();
+    SWARM_PHASE(PH_PUBLISH);
 
     int action = 0;
 
@@ -142,7 +149,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
     if (radius && kQ && t.active) deg = tile_in_edges_radius(g, t, pos, s, N, p.qmax_r);
     if (MODE == MODE_GRAPH && radius) {
       tile_write_edges_radius(t, pos, s, N, p.qmax_r, p.edges_per_env, p.edges_out, p.counts_out, reinterpret_cast<int*>(sred));
-    } else if (kGraphOut) {
+    } else if (kGraphOut && !PLAIN) {
       int32_t* eout = nullptr;
       if (MODE == MODE_GRAPH) eout = p.edges_out;
       else if (p.trace.edges) eout = p.trace.edges + (long long)tick * c.num_envs * 2 * p.edges_per_env;
@@ -172,7 +179,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
       float q[9];
       if (TC) {
         if (complete)
-          action = tile_q_forward_tc<ATT_COMPLETE>(g, ts, t, tmem, pos, N, deg, 0u, adst_tc, c.goal_x, c.goal_y, parity, q);
+          action = tile_q_forward_tc<ATT_COMPLETE, NT>(g, ts, t, tmem, pos, N, deg, 0u, adst_tc, c.goal_x, c.goal_y, parity, q);
         else if (knn_small)
           action = tile_q_forward_tc<ATT_COUNTS>(g, ts, t, tmem, pos, N, deg, knn_counts, adst_tc, c.goal_x, c.goal_y, parity, q);
         else
@@ -191,7 +198,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
             for (int a = 0; a < 9; ++a) p.q_out[t.gidx * 9 + a] = q[a];
           }
           if (p.act_out) p.act_out[t.gidx] = action;
-        } else if (p.trace.q) {
+        } else if (!PLAIN && p.trace.q) {
           float* tq = p.trace.q + ((long long)tick * BN + t.gidx) * 9;
 #pragma unroll
           for (int a = 0; a < 9; ++a) tq[a] = q[a];
@@ -205,7 +212,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
       if (t.active) {
         if (MODE == MODE_STEP) {
           action = p.actions_in[t.gidx];
-        } else {
+        } else if (!PLAIN) {
           if (epsilon > 0.0f) {
             // train:164-165: one coin per tick for the whole swarm, then one uniform action per agent
             const unsigned long long genv = (unsigned long long)(p.env_offset + t.env);
@@ -221,7 +228,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
         const float4 s_prev = s;
         uint8_t flags = 0;
         uint32_t cmask = 0;
-        tile_world_step(p, t, pos, action, s, flags, cmask);
+        tile_world_step<NT>(p, t, pos, action, s, flags, cmask);
 
         // scenario.reward(agent) on the post-step state
         const float dgoal = goal_distance(s.x, s.y, c);
@@ -242,7 +249,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
             o[0] = s.x; o[1] = s.y; o[2] = s.z; o[3] = s.w; o[4] = c.goal_x; o[5] = c.goal_y;
           }
           if (p.dist_out) reinterpret_cast<float2*>(p.dist_out)[t.gidx] = make_float2(dgoal, dobs);
-        } else {
+        } else if (!PLAIN) {
           const long long tb = (long long)tick * BN + t.gidx;
           if (p.trace.state) reinterpret_cast<float4*>(p.trace.state)[tb] = s;
           if (p.trace.actions) p.trace.actions[tb] = action;
@@ -298,7 +305,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
         ret = __fadd_rn(ret, reward);
         if (MODE == MODE_STEP) {
           if (p.rewards_out) p.rewards_out[t.gidx] = reward;
-        } else {
+        } else if (!PLAIN) {
           if (p.trace.rewards) p.trace.rewards[(long long)tick * BN + t.gidx] = reward;
           if (p.replay.state) {
             const long long slot = (replay_cursor + (long long)tick * c.num_envs + t.env) % p.replay.capacity;
@@ -307,7 +314,9 @@ tile_kernel(const __grid_constant__ TileParams p) {
         }
       }
     }
+    SWARM_PHASE(PH_WORLD);
   }
+  SWARM_PHASE_FLUSH();
 
   if (MODE == MODE_ROLLOUT) {
     if (t.active) {
@@ -391,17 +400,18 @@ cudaError_t launch_replay_gather(const SwarmReplay& r, const int64_t* indices, i
 }
 
 // explicit instantiations + launcher
-template <int MODE, bool TC, bool DENSE, bool FLOCK = false, int NT = 0>
+template <int MODE, bool TC, bool DENSE, bool FLOCK = false, int NT = 0, bool PLAIN = false>
 static cudaError_t launch_tile_impl(const TileParams& p, cudaStream_t stream) {
   const SwarmConfig& c = p.cfg;
   const TileLayout L = tile_layout(MODE, kTileThreads, c.n_agents, c.knn_k, p.maxdeg, c.graph_mode, TC);
   const int grid = p.bal_q > 0 ? (int)((c.num_envs - p.bal_r) / p.bal_q) : (c.num_envs + p.epb - 1) / p.epb;
   if (L.total > 48 * 1024) {
     cudaError_t err =
-        cudaFuncSetAttribute(tile_kernel<MODE, TC, DENSE, FLOCK, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total);
+        cudaFuncSetAttribute(tile_kernel<MODE, TC, DENSE, FLOCK, NT, PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             L.total);
     if (err != cudaSuccess) return err;
   }
-  tile_kernel<MODE, TC, DENSE, FLOCK, NT><<<grid, kTileThreads, L.total, stream>>>(p);
+  tile_kernel<MODE, TC, DENSE, FLOCK, NT, PLAIN><<<grid, kTileThreads, L.total, stream>>>(p);
   return cudaGetLastError();
 }
 
@@ -428,11 +438,26 @@ static bool tile_grid_plan(TileParams& p) {
   return dense;
 }
 
+// The launch takes the PLAIN rollout (see tile_kernel) when it asks for nothing but the greedy episode on the complete
+// graph: final states, returns and hit counts.
+static bool plain_rollout(const TileParams& p) {
+  const SwarmTrace& tr = p.trace;
+  const bool traced = tr.state || tr.actions || tr.q || tr.rewards || tr.flags || tr.contact || tr.edges || tr.dist;
+  const bool scenario = p.cfg.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE || p.cfg.scenario == SWARM_SCENARIO_GOTO;
+  return p.cfg.graph_mode == SWARM_GRAPH_COMPLETE && !traced && !p.replay.state && !p.actions_in && !p.ctl &&
+         p.epsilon == 0.0f && scenario;
+}
+
 template <int MODE>
 static cudaError_t launch_tile_q(const TileParams& p0, cudaStream_t stream) {
   if (!p0.use_tc) return launch_tile_impl<MODE, false, true>(p0, stream);
   TileParams p = p0;
   const bool dense = tile_grid_plan(p);
+  if constexpr (MODE == MODE_ROLLOUT) {
+    if (p.cfg.n_agents == 12 && plain_rollout(p))
+      return dense ? launch_tile_impl<MODE, true, true, false, 12, true>(p, stream)
+                   : launch_tile_impl<MODE, true, false, false, 12, true>(p, stream);
+  }
   if (MODE == MODE_ROLLOUT && p.cfg.n_agents == 12)       // the benchmark shape with the swarm size at compile time
     return dense ? launch_tile_impl<MODE, true, true, false, 12>(p, stream)
                  : launch_tile_impl<MODE, true, false, false, 12>(p, stream);
@@ -462,3 +487,12 @@ cudaError_t launch_tile(int mode, const TileParams& p, cudaStream_t stream) {
 }
 
 }  // namespace swarm
+
+#ifdef SWARM_PHASE_CLOCKS
+// per-warp phase cycles of the last tile-kernel launch, [warps][PH_COUNT] (scripts/time_rollout_phases.py)
+extern "C" int swarm_phase_cycles(unsigned long long* dst, int warps) {
+  if (warps > swarm::kPhaseWarps) warps = swarm::kPhaseWarps;
+  const cudaError_t e = cudaMemcpyFromSymbol(dst, swarm::g_phase_cycles, sizeof(unsigned long long) * swarm::PH_COUNT * warps);
+  return e == cudaSuccess ? warps : -1;
+}
+#endif

@@ -20,6 +20,49 @@
 
 namespace swarm {
 
+// Phase clocks of the rollout tick, compiled in only with -DSWARM_PHASE_CLOCKS (scripts/time_rollout_phases.py builds
+// such a library next to the regular one).  Lane 0 of every warp stamps clock64() at each phase boundary and adds the
+// cycles since the previous stamp to its warp's slot in shared memory; at the end of the launch the per-warp sums go to
+// g_phase_cycles[global warp][phase].  A phase's count includes the time its warp waits at the barriers inside it.
+enum { PH_PUBLISH = 0, PH_ATTEND, PH_PROJ, PH_TANH, PH_LIN1, PH_RELU, PH_LIN2, PH_WORLD, PH_COUNT };
+#ifdef SWARM_PHASE_CLOCKS
+constexpr int kPhaseWarps = 16384;
+__device__ unsigned long long g_phase_cycles[kPhaseWarps][PH_COUNT];   // (only tile_kernels.cu is built with the macro)
+__device__ __forceinline__ unsigned long long* phase_slots() {
+  __shared__ unsigned long long s[kTileThreads / 32][PH_COUNT + 1];     // [warp][phase]; [warp][PH_COUNT] = last stamp
+  return s[threadIdx.x >> 5];
+}
+__device__ __forceinline__ void phase_reset() {
+  if ((threadIdx.x & 31) == 0)
+    for (int k = 0; k < PH_COUNT; ++k) phase_slots()[k] = 0;
+}
+__device__ __forceinline__ void phase_start() {
+  if ((threadIdx.x & 31) == 0) phase_slots()[PH_COUNT] = clock64();
+}
+__device__ __forceinline__ void phase_mark(int k) {
+  if ((threadIdx.x & 31) == 0) {
+    unsigned long long* s = phase_slots();
+    const unsigned long long now = clock64();
+    s[k] += now - s[PH_COUNT];
+    s[PH_COUNT] = now;
+  }
+}
+__device__ __forceinline__ void phase_flush() {
+  const long long w = (long long)blockIdx.x * (kTileThreads / 32) + (threadIdx.x >> 5);
+  if ((threadIdx.x & 31) == 0 && w < kPhaseWarps)
+    for (int k = 0; k < PH_COUNT; ++k) g_phase_cycles[w][k] = phase_slots()[k];
+}
+#define SWARM_PHASE_RESET() phase_reset()
+#define SWARM_PHASE_START() phase_start()
+#define SWARM_PHASE(k) phase_mark(k)
+#define SWARM_PHASE_FLUSH() phase_flush()
+#else
+#define SWARM_PHASE_RESET() ((void)0)
+#define SWARM_PHASE_START() ((void)0)
+#define SWARM_PHASE(k) ((void)0)
+#define SWARM_PHASE_FLUSH() ((void)0)
+#endif
+
 // float offsets inside the small vector block
 // (v_s, v_d: W0^T att_src / W0^T att_dst, 7 entries + one zero each)
 enum { TV_VS = 0, TV_VD = 8, TV_B0 = 16, TV_B1 = 48, TV_B2 = 80, TV_COUNT = 96 };
@@ -196,7 +239,16 @@ __device__ __forceinline__ void tc_alpha_terms(const TileTcSmem& s, const float 
 //                 in-edge LIST (strided byte stores, two barriers) is never built
 enum { ATT_LIST = 0, ATT_COMPLETE = 1, ATT_COUNTS = 2 };
 
-template <int ATT>
+//
+// NT > 0 (ATT_COMPLETE only): the swarm size at compile time.  Every loop unrolls completely: the alpha_src row is read
+// as float4s (an env's row starts at a multiple of 16 bytes when NT % 4 == 0), its maximum is a tree, and all NT
+// exponentials are issued before the accumulation, so the dependent chains are the sums alone.  An inactive thread
+// computes on env 0 of its tile instead of skipping the loops and discards the result (its UMMA row is independent of
+// the others).  The sums keep the order of the run-time loop: den, acc_p, acc_v and acc_id run left to right in j, so
+// the result is the same to the bit.  The maximum is exact in any order; a tree can return -0 where the chain returns
+// +0 (or the reverse), but m only enters through exp(x - m), and x - (+0) and x - (-0) differ at most in the sign of a
+// zero, which exp maps to 1 either way.
+template <int ATT, int NT = 0>
 __device__ __forceinline__ void tile_attend_inputs(const TileGraphSmem& g, const TileThread& t, const float4* __restrict__ pos,
                                                    int N, int deg, uint32_t counts, float adst, float goal_x, float goal_y,
                                                    float (&xm)[8]) {
@@ -207,7 +259,53 @@ __device__ __forceinline__ void tile_attend_inputs(const TileGraphSmem& g, const
   float den = 0.0f, acc_id = 0.0f;
   float2 acc_p = make_float2(0.0f, 0.0f), acc_v = make_float2(0.0f, 0.0f);
   // LeakyReLU and the rounded add are monotone: max_e leaky(a_e + d) = leaky(max_e a_e + d)
-  if (ATT == ATT_COUNTS) {
+  if constexpr (COMPLETE && NT > 0) {
+    const int base = t.active ? t.envbase : 0;
+    const int self = (t.i == 0) ? -1 : t.i;
+    float a[NT];
+    if constexpr (NT % 4 == 0) {
+      const float4* __restrict__ sas4 = reinterpret_cast<const float4*>(g.sas + base);
+#pragma unroll
+      for (int k = 0; k < NT / 4; ++k) {
+        const float4 v = sas4[k];
+        a[4 * k] = v.x; a[4 * k + 1] = v.y; a[4 * k + 2] = v.z; a[4 * k + 3] = v.w;
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < NT; ++j) a[j] = g.sas[base + j];
+    }
+    float4 sj[NT];
+#pragma unroll
+    for (int j = 0; j < NT; ++j) sj[j] = pos[base + j];
+    // (where every term is NaN the tree returns NaN and the chain -inf: every weight is NaN either way)
+    float mx[NT];
+#pragma unroll
+    for (int j = 0; j < NT; ++j) mx[j] = (j == self) ? -INFINITY : a[j];
+#pragma unroll
+    for (int w = 1; w < NT; w *= 2) {
+#pragma unroll
+      for (int j = 0; j + w < NT; j += 2 * w) mx[j] = fmaxf(mx[j], mx[j + w]);
+    }
+    const float amax = mx[0];
+    const float zt = __fadd_rn(amax, adst);
+    const float m = fmaxf(zt, __fmul_rn(zt, 0.2f));
+    float wj[NT];
+#pragma unroll
+    for (int j = 0; j < NT; ++j) {
+      const float zz = __fadd_rn(a[j], adst);
+      const float ex = __expf(fmaxf(zz, __fmul_rn(zz, 0.2f)) - m);
+      wj[j] = (j == self) ? 0.0f : ex;
+    }
+#pragma unroll
+    for (int j = 0; j < NT; ++j) {
+      const float w = wj[j];
+      const float2 w2 = make_float2(w, w);
+      den = __fadd_rn(den, w);
+      acc_p = __ffma2_rn(w2, make_float2(sj[j].x, sj[j].y), acc_p);
+      acc_v = __ffma2_rn(w2, make_float2(sj[j].z, sj[j].w), acc_v);
+      acc_id = fmaf(w, (float)j, acc_id);
+    }
+  } else if (ATT == ATT_COUNTS) {
     const int n = t.active ? N : 0;
     float amax = -INFINITY;
     uint32_t cw = counts;
@@ -284,7 +382,7 @@ __device__ __forceinline__ void tile_attend_inputs(const TileGraphSmem& g, const
 
 // Full per-tick Q forward on the tensor cores.  The caller has published g.sas[tid] = alpha_src of every node and
 // passed a block barrier since (the tick's state barrier).  Contains 3 block barriers.  All 128 threads must call it.
-template <int ATT>
+template <int ATT, int NT = 0>
 __device__ __forceinline__ int tile_q_forward_tc(const TileGraphSmem& g, const TileTcSmem& s, const TileThread& t,
                                                  uint32_t tmem, const float4* __restrict__ pos, int N, int deg,
                                                  uint32_t counts, float adst, float goal_x, float goal_y, uint32_t& parity,
@@ -293,7 +391,8 @@ __device__ __forceinline__ int tile_q_forward_tc(const TileGraphSmem& g, const T
   // ---- attention in input space, then agg = mean W0^T (K padded 7 -> 8) ----
   {
     float xm[8];
-    tile_attend_inputs<ATT>(g, t, pos, N, deg, counts, adst, goal_x, goal_y, xm);
+    tile_attend_inputs<ATT, NT>(g, t, pos, N, deg, counts, adst, goal_x, goal_y, xm);
+    SWARM_PHASE(PH_ATTEND);
     float4 h0, l0, h1, l1;
     tc::split4(make_float4(xm[0], xm[1], xm[2], xm[3]), h0, l0);
     tc::split4(make_float4(xm[4], xm[5], xm[6], 0.0f), h1, l1);
@@ -308,6 +407,7 @@ __device__ __forceinline__ int tile_q_forward_tc(const TileGraphSmem& g, const T
   tc_mma_round(s, tmem, tmem, s.w0, kTcW0Bytes / 2, 32, 1, parity);
   float a1[32];
   tc::tmem_ld32(lane_addr, a1);
+  SWARM_PHASE(PH_PROJ);
   {
     // u = tanh(agg + b0) = 1 - 2 / (exp(2 (agg + b0)) + 1), two channels per packed instruction around the SFU ops
     const float4* b4 = reinterpret_cast<const float4*>(s.vec + TV_B0);
@@ -329,9 +429,11 @@ __device__ __forceinline__ int tile_q_forward_tc(const TileGraphSmem& g, const T
     }
   }
   tc_store_a_row(lane_addr, a1);
+  SWARM_PHASE(PH_TANH);
   // ---- lin1 + ReLU ----
   tc_mma_round(s, tmem, tmem + 32, s.w1, kTcW1Bytes / 2, 32, 4, parity);
   tc::tmem_ld32(lane_addr + 32, a1);
+  SWARM_PHASE(PH_LIN1);
   {
     const float4* b4 = reinterpret_cast<const float4*>(s.vec + TV_B1);
 #pragma unroll
@@ -344,6 +446,7 @@ __device__ __forceinline__ int tile_q_forward_tc(const TileGraphSmem& g, const T
     }
   }
   tc_store_a_row(lane_addr, a1);    // lin1 has completed (mbarrier), the A columns are free again
+  SWARM_PHASE(PH_RELU);
   // ---- lin2 ----
   tc_mma_round(s, tmem, tmem, s.w2, kTcW2Bytes / 2, 16, 4, parity);
   float qq[16];
@@ -358,6 +461,7 @@ __device__ __forceinline__ int tile_q_forward_tc(const TileGraphSmem& g, const T
       action = a;
     }
   }
+  SWARM_PHASE(PH_LIN2);
   return action;
 }
 
