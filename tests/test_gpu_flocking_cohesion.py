@@ -359,12 +359,15 @@ def _flocking_pair(B, n, T, seed):
     return sb, envs[0], envs[1], w
 
 
-@pytest.mark.parametrize("graph,n", [("complete", 7), ("knn", 12), ("complete", 2)])
-def test_fused_flocking_rollout_matches_env_stepping(graph, n):
+@pytest.mark.parametrize("graph,n,B", [("complete", 7, 37), ("knn", 12, 37), ("complete", 2, 37),
+                                       # the FLOCK, NT = 12 instantiation at 444 CTAs of 9-10 envs
+                                       ("complete", 12, 4096)],
+                         ids=["complete-7", "knn-12", "complete-2", "complete-12-4096"])
+def test_fused_flocking_rollout_matches_env_stepping(graph, n, B):
     """swarm_rollout with the Flocking option (graph -> GAT-Q -> epsilon-greedy -> world step -> Flocking reward, T ticks in
     one launch) against Environment.step on a second FlockingScenario env driven with the traced actions: states, rewards,
     returns, replay pushes and the shaping memory agree bit for bit."""
-    B, T = 37, 20
+    T = 20
     sb, env_a, env_b, w = _flocking_pair(B, n, T, seed=n)
     ops, L = sb.ops, sb._lib
     sc_a, sc_b = env_a.scenario, env_b.scenario
