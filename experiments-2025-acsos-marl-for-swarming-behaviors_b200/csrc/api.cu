@@ -9,8 +9,8 @@
 
 namespace swarm {
 cudaError_t launch_tile(int mode, const TileParams& p, cudaStream_t stream);
-cudaError_t launch_sim_step(const TileParams& p, cudaStream_t stream);
-cudaError_t launch_sim_step_large(const TileParams& p, cudaStream_t stream);
+cudaError_t launch_sim_step(SimStepArgs p, cudaStream_t stream);
+cudaError_t launch_sim_step_large(const SimStepArgs& p, cudaStream_t stream);
 cudaError_t launch_graph_large(const SwarmConfig& c, const float* state, int32_t* edges, int32_t* nbr, int edges_per_env,
                                cudaStream_t stream);
 cudaError_t launch_reset_grid(const SwarmConfig& c, int cols, int rows, const float* centers, float* state,
@@ -35,7 +35,7 @@ int stack_weight_count_host(const SwarmStackSpec& s);
 cudaError_t launch_gatstack_forward(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, const float* state,
                                     float* q, int32_t* actions, cudaStream_t stream);
 cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
-                                    int ticks, const TileParams& step, const SwarmRewardSpec* flock, float* shaping,
+                                    int ticks, const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
                                     float* returns, int32_t* hits, cudaStream_t stream);
 cudaError_t launch_stack_accumulate(long long total, int N, const float* rewards, int per_env, const uint8_t* flags,
                                     float* returns, int32_t* hits, cudaStream_t stream);
@@ -136,11 +136,7 @@ int fill_params(TileParams& p, const SwarmConfig* cfg, int mode) {
   const bool knn = cfg->graph_mode == SWARM_GRAPH_KNN;
   p.maxdeg = knn ? (n + cfg->knn_k + 1) : n;
   p.edges_per_env = (int32_t)swarm_edges_per_env(cfg);
-  p.one_minus_drag = (float)(1.0 - (double)cfg->drag);
-  p.dmin_aa = cfg->agent_radius + cfg->agent_radius;
-  p.dmin_ao = cfg->landmark_radius + cfg->agent_radius;
-  p.qmax_aa = sq_threshold(p.dmin_aa);
-  p.qmax_ao = sq_threshold(p.dmin_ao);
+  p.world = world_consts(*cfg);
   p.qmax_r = cfg->graph_mode == SWARM_GRAPH_RADIUS ? sq_threshold(cfg->graph_radius) : 0.0f;
   // dense contractions on the tensor cores (tcgen05 3xTF32) unless SWARM_TC=0 selects the CUDA-core FFMA path
   const char* tc_env = std::getenv("SWARM_TC");
@@ -154,6 +150,17 @@ int fill_params(TileParams& p, const SwarmConfig* cfg, int mode) {
   }
   if (L.total > 227 * 1024) return fail(SWARM_ERR_UNSUPPORTED, "shared-memory tile exceeds 227 KB for this (N, k)");
   return SWARM_OK;
+}
+
+SimStepArgs step_args(const SwarmConfig& c, const float* state_in, const int32_t* actions, float* state_out) {
+  SimStepArgs p;
+  std::memset(&p, 0, sizeof(p));
+  p.cfg = c;
+  p.world = world_consts(c);
+  p.state_in = reinterpret_cast<const float4*>(state_in);
+  p.actions = actions;
+  p.state_out = reinterpret_cast<float4*>(state_out);
+  return p;
 }
 }  // namespace
 }  // namespace swarm
@@ -212,21 +219,16 @@ int swarm_sim_step(const SwarmConfig* cfg, const float* state_in, const int32_t*
   if (int rc = validate(cfg, false, true)) return rc;
   if (!state_in || !actions || !state_out) return fail(SWARM_ERR_INVALID_ARG, "state_in/actions/state_out is NULL");
   if (contact && cfg->n_agents > 32) return fail(SWARM_ERR_UNSUPPORTED, "contact masks need n_agents <= 32");
-  TileParams p;
-  if (int rc = fill_params(p, cfg, MODE_STEP)) return rc;
-  p.state_in = state_in;
-  p.state_out = state_out;
-  p.actions_in = actions;
-  p.rewards_out = rewards;
-  p.flags_out = flags;
-  p.contact_out = contact;
-  p.obs_out = obs;
-  p.dist_out = dist;
-  // n_agents <= 64: lean streaming kernel (step_kernels.cu); <= 128: env-tile kernel; above: one env per CTA row
-  // (large_kernels.cu) -- all three run the same device arithmetic
-  if (cfg->n_agents <= 64) return check_cuda(launch_sim_step(p, (cudaStream_t)stream), "swarm_sim_step");
+  SimStepArgs p = step_args(*cfg, state_in, actions, state_out);
+  p.rewards = rewards;
+  p.flags = flags;
+  p.contact = contact;
+  p.obs = obs;
+  p.dist = reinterpret_cast<float2*>(dist);
+  // n_agents <= 128: whole envs per CTA, TMA-streamed for small swarms where the tiles allow (step_kernels.cu); above:
+  // one env per CTA (large_kernels.cu) -- both run the same device arithmetic
   if (cfg->n_agents > kTileThreads) return check_cuda(launch_sim_step_large(p, (cudaStream_t)stream), "swarm_sim_step");
-  return check_cuda(launch_tile(MODE_STEP, p, (cudaStream_t)stream), "swarm_sim_step");
+  return check_cuda(launch_sim_step(p, (cudaStream_t)stream), "swarm_sim_step");
 }
 
 int swarm_graph_build(const SwarmConfig* cfg, const float* state, int32_t* edges, int32_t* neighbours, void* stream) {
@@ -358,15 +360,12 @@ int swarm_rollout_large(const SwarmConfig* cfg, const float* weights, float* sta
     return fail(SWARM_ERR_UNSUPPORTED, "the env does not fit shared memory: step it with swarm_graph_build + "
                                        "swarm_csr_from_edges + swarm_gatq_forward_csr + swarm_sim_step");
   if (workspace_bytes < swarm_rollout_large_workspace_bytes(cfg)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  TileParams p;
-  if (int rc = fill_params(p, cfg, MODE_STEP)) return rc;
   const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
   uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
   int32_t* nbr = reinterpret_cast<int32_t*>(base);
   int32_t* actions = nbr + (knn ? bn * cfg->knn_k : 0);
-  p.state_in = state;
-  p.state_out = state;           // in place: one CTA owns a whole env and stages its positions first
-  p.actions_in = actions;
+  // in place: one CTA owns a whole env and stages its positions first
+  SimStepArgs p = step_args(*cfg, state, actions, state);
   p.returns = returns;
   p.hits = hits;
   cudaStream_t st = (cudaStream_t)stream;
@@ -376,7 +375,7 @@ int swarm_rollout_large(const SwarmConfig* cfg, const float* weights, float* sta
     // (radius / complete graph: the forward finds its own sources -- uniform-grid broad phase / every other agent --
     // so a tick is two launches)
     if (knn) {
-      if (cudaError_t e = launch_graph_large(*cfg, state, nullptr, nbr, p.edges_per_env, st); e != cudaSuccess)
+      if (cudaError_t e = launch_graph_large(*cfg, state, nullptr, nbr, (int)swarm_edges_per_env(cfg), st); e != cudaSuccess)
         return check_cuda(e, "swarm_rollout_large (graph)");
       if (cudaError_t e = xspace ? launch_gatq_knn_large_x(*cfg, weights, state, nbr, nullptr, actions, st)
                                  : launch_gatq_knn_large(*cfg, weights, state, nbr, nullptr, actions, st);
@@ -857,31 +856,26 @@ int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, cons
     rs.reset = 0;
     rs.env_index = -1;
   }
-  TileParams p;
-  if (int rc = fill_params(p, cfg, MODE_STEP)) return rc;
   const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
   uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
   int32_t* actions = reinterpret_cast<int32_t*>(base);
   float* rewards = reinterpret_cast<float*>(actions + bn);
   uint8_t* flags = reinterpret_cast<uint8_t*>(rewards + bn);
-  p.state_in = state;
-  p.state_out = state;
-  p.actions_in = actions;
-  p.rewards_out = rewards;
-  p.flags_out = flags;
   cudaStream_t st = (cudaStream_t)stream;
   // the whole loop is ONE launch with the state in registers (stack_kernels.cu gatstack_kernel<HP, true>);
   // SWARM_STACK_FUSED=0 takes the launch sequence below (forward, step, reward kernel, totals per tick)
   const char* fused_env = std::getenv("SWARM_STACK_FUSED");
   if (!(fused_env && fused_env[0] == '0'))
-    return check_cuda(launch_gatstack_rollout(*cfg, *spec, weights, state, ticks, p, reward ? &rs : nullptr, shaping, returns,
-                                              hits, st),
+    return check_cuda(launch_gatstack_rollout(*cfg, *spec, weights, state, ticks, world_consts(*cfg), reward ? &rs : nullptr,
+                                              shaping, returns, hits, st),
                       "swarm_rollout_stack");
+  SimStepArgs p = step_args(*cfg, state, actions, state);
+  p.rewards = rewards;
+  p.flags = flags;
   for (int t = 0; t < ticks; ++t) {
     if (cudaError_t e = launch_gatstack_forward(*cfg, *spec, weights, state, nullptr, actions, st); e != cudaSuccess)
       return check_cuda(e, "swarm_rollout_stack (forward)");
-    cudaError_t e = cfg->n_agents <= 64 ? launch_sim_step(p, st) : launch_tile(MODE_STEP, p, st);
-    if (e != cudaSuccess) return check_cuda(e, "swarm_rollout_stack (step)");
+    if (cudaError_t e = launch_sim_step(p, st); e != cudaSuccess) return check_cuda(e, "swarm_rollout_stack (step)");
     int per_env = 0;
     if (reward) {
       per_env = rs.kind == SWARM_REWARD_FLOCKING ? 1 : 0;

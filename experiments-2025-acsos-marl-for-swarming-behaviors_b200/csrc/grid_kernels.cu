@@ -238,22 +238,9 @@ cudaError_t launch_radius_csr(const SwarmConfig& c, const float* state, int32_t*
 // radius_csr_kernel does) because the reference adds the contact forces in entity order and float addition does not
 // commute -- same pair test, same contact_force, same order as the full sweep, hence the same bits.  An agent whose
 // neighbourhood holds more than kGridBruteAbove candidates (a collapsed swarm) falls back to the full sweep.
-struct GridStepParams {
-  SwarmConfig cfg;
-  const float4* state_in;
-  const int32_t* actions;
-  float4* state_out;
-  float* rewards;
-  uint8_t* flags;
-  float* obs;
-  float2* dist;
-  float one_minus_drag, dmin_aa, dmin_ao, qmax_aa, qmax_ao;
-  float* returns;
-  int32_t* hits;
-};
 constexpr int kGridBruteAbove = 96;
 
-__global__ void __launch_bounds__(kGridThreads) sim_step_grid_kernel(const __grid_constant__ GridStepParams p) {
+__global__ void __launch_bounds__(kGridThreads) sim_step_grid_kernel(const __grid_constant__ SimStepArgs p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_hits;
   const SwarmConfig& c = p.cfg;
@@ -272,24 +259,17 @@ __global__ void __launch_bounds__(kGridThreads) sim_step_grid_kernel(const __gri
   }
   __syncthreads();
   // every pre-step position is staged before any thread writes a post-step state: state_out may alias state_in
-  const CellGrid g = grid_build([&](int j) { return spos[j]; }, N, P, p.dmin_aa, keys, cbeg, cend, sred);
+  const WorldConsts& w = p.world;
+  const CellGrid g = grid_build([&](int j) { return spos[j]; }, N, P, w.dmin_aa, keys, cbeg, cend, sred);
   int my_hits = 0;
+  const bool oa = c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE;
   for (int i = threadIdx.x; i < N; i += kGridThreads) {
     const long long gidx = env * N + i;
     float4 s = env_state[i];               // only this thread ever writes index i
-    float fx, fy, gx, gy;
+    float fx, fy;
     decode_action(p.actions[gidx], fx, fy);
     uint8_t flags = 0;
-    if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-      const float dx = __fsub_rn(s.x, c.obstacle_x), dy = __fsub_rn(s.y, c.obstacle_y);
-      if (__fmaf_rn(dy, dy, __fmul_rn(dx, dx)) <= p.qmax_ao) {
-        if (contact_force(s.x, s.y, c.obstacle_x, c.obstacle_y, p.dmin_ao, c.collision_force, c.contact_margin, gx, gy)) {
-          fx = __fadd_rn(fx, gx);
-          fy = __fadd_rn(fy, gy);
-          flags |= SWARM_FLAG_OBSTACLE_CONTACT;
-        }
-      }
-    }
+    if (oa) obstacle_contact(s, c, w, fx, fy, flags);
     {
       const float2 neg = make_float2(-s.x, -s.y);
       const int cx = g.cx(s.x), cy = g.cy(s.y);
@@ -307,7 +287,7 @@ __global__ void __launch_bounds__(kGridThreads) sim_step_grid_kernel(const __gri
       }
       if (cand > kGridBruteAbove) {
         uint32_t cmask = 0;
-        agent_contacts(spos, N, i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin, fx, fy, cmask);
+        agent_contacts(spos, N, i, s.x, s.y, w.qmax_aa, w.dmin_aa, c.collision_force, c.contact_margin, fx, fy, cmask);
       } else {
         while (true) {
           uint32_t m = v[0];
@@ -322,8 +302,9 @@ __global__ void __launch_bounds__(kGridThreads) sim_step_grid_kernel(const __gri
             }
           }
           const float2 o = spos[m];
-          if ((int)m != i && grid_hit(o, neg, p.qmax_aa)) {
-            if (contact_force(s.x, s.y, o.x, o.y, p.dmin_aa, c.collision_force, c.contact_margin, gx, gy)) {
+          float gx, gy;
+          if ((int)m != i && grid_hit(o, neg, w.qmax_aa)) {
+            if (contact_force(s.x, s.y, o.x, o.y, w.dmin_aa, c.collision_force, c.contact_margin, gx, gy)) {
               fx = __fadd_rn(fx, gx);
               fy = __fadd_rn(fy, gy);
             }
@@ -331,25 +312,16 @@ __global__ void __launch_bounds__(kGridThreads) sim_step_grid_kernel(const __gri
         }
       }
     }
-    integrate(s, fx, fy, c.dt, p.one_minus_drag);
-    const float dgoal = goal_distance(s.x, s.y, c);
-    float dobs = 0.0f;
-    if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-      dobs = obstacle_distance(s.x, s.y, c);
-      const float reward = oa_reward(dgoal, dobs, c, flags);
+    integrate(s, fx, fy, c.dt, w.one_minus_drag);
+    float dgoal, dobs;
+    const float reward = post_step_reward(s, oa, c, dgoal, dobs, flags);
+    if (oa) {
       if (p.rewards) p.rewards[gidx] = reward;
       if (p.returns) p.returns[gidx] = __fadd_rn(p.returns[gidx], reward);
       my_hits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
     }
     p.state_out[gidx] = s;
-    if (p.flags) p.flags[gidx] = flags;
-    if (p.obs) {
-      float2* o = reinterpret_cast<float2*>(p.obs + gidx * 6);
-      o[0] = make_float2(s.x, s.y);
-      o[1] = make_float2(s.z, s.w);
-      o[2] = make_float2(c.goal_x, c.goal_y);
-    }
-    if (p.dist) p.dist[gidx] = make_float2(dgoal, dobs);
+    store_step_outputs(p, gidx, s, dgoal, dobs, flags, 0u);     // no contact masks above 32 agents
   }
   if (p.hits) {
     if (my_hits) atomicAdd(&s_hits, my_hits);          // integer: order-independent
@@ -367,24 +339,8 @@ bool sim_step_grid_enabled(int n_agents) {
   return n_agents >= 512;
 }
 
-cudaError_t launch_sim_step_grid(const TileParams& tp, cudaStream_t stream) {
-  const SwarmConfig& c = tp.cfg;
-  GridStepParams p;
-  p.cfg = c;
-  p.state_in = reinterpret_cast<const float4*>(tp.state_in);
-  p.actions = tp.actions_in;
-  p.state_out = reinterpret_cast<float4*>(tp.state_out);
-  p.rewards = tp.rewards_out;
-  p.flags = tp.flags_out;
-  p.obs = tp.obs_out;
-  p.dist = reinterpret_cast<float2*>(tp.dist_out);
-  p.one_minus_drag = tp.one_minus_drag;
-  p.dmin_aa = tp.dmin_aa;
-  p.dmin_ao = tp.dmin_ao;
-  p.qmax_aa = tp.qmax_aa;
-  p.qmax_ao = tp.qmax_ao;
-  p.returns = tp.returns;
-  p.hits = tp.hits;
+cudaError_t launch_sim_step_grid(const SimStepArgs& p, cudaStream_t stream) {
+  const SwarmConfig& c = p.cfg;
   const size_t smem = radius_csr_smem_bytes(c.n_agents);
   cudaError_t err = cudaFuncSetAttribute(sim_step_grid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return err;

@@ -20,24 +20,10 @@ namespace swarm {
 
 constexpr int kLargeThreads = 256;
 
-struct LargeStepParams {
-  SwarmConfig cfg;
-  const float4* state_in;
-  const int32_t* actions;
-  float4* state_out;
-  float* rewards;
-  uint8_t* flags;
-  float* obs;
-  float2* dist;
-  float one_minus_drag, dmin_aa, dmin_ao, qmax_aa, qmax_ao;
-  float* returns;          // optional: per-agent running return += reward (swarm_rollout_large)
-  int32_t* hits;           // optional: per-env obstacle hits += number of agents inside hit_distance this tick
-};
-
 // grid = envs: ONE CTA owns a whole env.  It stages every pre-step position of the env in shared memory before any
 // thread writes a post-step state, so state_out may alias state_in (the in-place use of World.step / rollout_large);
 // a (chunk, env) grid would let a later-scheduled chunk read partner positions that an earlier chunk already stepped.
-__global__ void __launch_bounds__(kLargeThreads) sim_step_large_kernel(const __grid_constant__ LargeStepParams p) {
+__global__ void __launch_bounds__(kLargeThreads) sim_step_large_kernel(const __grid_constant__ SimStepArgs p) {
   extern __shared__ float2 spos[];
   __shared__ int s_hits;
   const SwarmConfig& c = p.cfg;
@@ -51,43 +37,24 @@ __global__ void __launch_bounds__(kLargeThreads) sim_step_large_kernel(const __g
     spos[j] = make_float2(s.x, s.y);
   }
   __syncthreads();
+  const bool oa = c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE;
   for (int i = threadIdx.x; i < N; i += kLargeThreads) {
-  const long long gidx = env * N + i;
-  float4 s = env_state[i];               // only this thread ever writes index i: no hazard with the in-place store below
-  float fx, fy, gx, gy;
-  decode_action(p.actions[gidx], fx, fy);
-  uint8_t flags = 0;
-  uint32_t cmask = 0;
-  if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-    const float dx = __fsub_rn(s.x, c.obstacle_x), dy = __fsub_rn(s.y, c.obstacle_y);
-    if (__fmaf_rn(dy, dy, __fmul_rn(dx, dx)) <= p.qmax_ao) {
-      if (contact_force(s.x, s.y, c.obstacle_x, c.obstacle_y, p.dmin_ao, c.collision_force, c.contact_margin, gx, gy)) {
-        fx = __fadd_rn(fx, gx);
-        fy = __fadd_rn(fy, gy);
-        flags |= SWARM_FLAG_OBSTACLE_CONTACT;
-      }
+    const long long gidx = env * N + i;
+    float4 s = env_state[i];               // only this thread ever writes index i: no hazard with the in-place store below
+    float2 u;
+    decode_action(p.actions[gidx], u.x, u.y);
+    uint8_t flags = 0;
+    uint32_t cmask = 0;
+    agent_step(s, u, spos, N, i, oa, c, p.world, flags, cmask);
+    float dgoal, dobs;
+    const float reward = post_step_reward(s, oa, c, dgoal, dobs, flags);
+    if (oa) {
+      if (p.rewards) p.rewards[gidx] = reward;
+      if (p.returns) p.returns[gidx] = __fadd_rn(p.returns[gidx], reward);
+      my_hits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
     }
-  }
-  agent_contacts(spos, N, i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin, fx, fy, cmask);
-  integrate(s, fx, fy, c.dt, p.one_minus_drag);
-  const float dgoal = goal_distance(s.x, s.y, c);
-  float dobs = 0.0f;
-  if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-    dobs = obstacle_distance(s.x, s.y, c);
-    const float reward = oa_reward(dgoal, dobs, c, flags);
-    if (p.rewards) p.rewards[gidx] = reward;
-    if (p.returns) p.returns[gidx] = __fadd_rn(p.returns[gidx], reward);
-    my_hits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
-  }
-  p.state_out[gidx] = s;
-  if (p.flags) p.flags[gidx] = flags;
-  if (p.obs) {
-    float2* o = reinterpret_cast<float2*>(p.obs + gidx * 6);
-    o[0] = make_float2(s.x, s.y);
-    o[1] = make_float2(s.z, s.w);
-    o[2] = make_float2(c.goal_x, c.goal_y);
-  }
-  if (p.dist) p.dist[gidx] = make_float2(dgoal, dobs);
+    p.state_out[gidx] = s;
+    store_step_outputs(p, gidx, s, dgoal, dobs, flags, 0u);     // no contact masks above 32 agents
   }
   if (p.hits) {
     if (my_hits) atomicAdd(&s_hits, my_hits);          // integer: order-independent
@@ -630,35 +597,19 @@ cudaError_t launch_gatq_knn_large(const SwarmConfig& c, const float* weights, co
 
 // ---- launchers ------------------------------------------------------------------------------
 bool sim_step_grid_enabled(int n_agents);
-cudaError_t launch_sim_step_grid(const TileParams& tp, cudaStream_t stream);
+cudaError_t launch_sim_step_grid(const SimStepArgs& p, cudaStream_t stream);
 
-cudaError_t launch_sim_step_large(const TileParams& tp, cudaStream_t stream) {
-  const SwarmConfig& c = tp.cfg;
-  LargeStepParams p;
-  p.cfg = c;
-  p.state_in = reinterpret_cast<const float4*>(tp.state_in);
-  p.actions = tp.actions_in;
-  p.state_out = reinterpret_cast<float4*>(tp.state_out);
-  p.rewards = tp.rewards_out;
-  p.flags = tp.flags_out;
-  p.obs = tp.obs_out;
-  p.dist = reinterpret_cast<float2*>(tp.dist_out);
-  p.one_minus_drag = tp.one_minus_drag;
-  p.dmin_aa = tp.dmin_aa;
-  p.dmin_ao = tp.dmin_ao;
-  p.qmax_aa = tp.qmax_aa;
-  p.qmax_ao = tp.qmax_ao;
-  p.returns = tp.returns;
-  p.hits = tp.hits;
+cudaError_t launch_sim_step_large(const SimStepArgs& p, cudaStream_t stream) {
+  const SwarmConfig& c = p.cfg;
   // contact partners from the uniform grid (grid_kernels.cu; same bits) unless SWARM_STEP_GRID=0 asks for the full sweep
   if (sim_step_grid_enabled(c.n_agents) && c.n_agents <= 4096) {
-    if (cudaError_t e = launch_sim_step_grid(tp, stream); e != cudaSuccess) return e;
+    if (cudaError_t e = launch_sim_step_grid(p, stream); e != cudaSuccess) return e;
   } else {
     sim_step_large_kernel<<<c.num_envs, kLargeThreads, c.n_agents * sizeof(float2), stream>>>(p);
   }
-  if (c.scenario == SWARM_SCENARIO_GOTO && (tp.rewards_out || tp.returns))
+  if (c.scenario == SWARM_SCENARIO_GOTO && (p.rewards || p.returns))
     goto_reward_large_kernel<<<c.num_envs, kLargeThreads, c.n_agents * sizeof(float), stream>>>(
-        c, reinterpret_cast<const float4*>(tp.state_out), tp.rewards_out, tp.returns);
+        c, p.state_out, p.rewards, p.returns);
   return cudaGetLastError();
 }
 

@@ -28,7 +28,7 @@ struct StackParams {
   int32_t epb, maxdeg;
   float qmax_r;
   // fused rollout (gatstack_rollout_kernel): `ticks` x [forward -> argmax -> world step -> reward], state in registers
-  TileParams step;           // physics constants of the world step (cfg, contact thresholds, drag)
+  WorldConsts step;          // constants of the world step
   float4* state_rw;          // [B*N] advanced in place
   float* returns;            // [B*N] += (optional)
   int32_t* hits;             // [B] += (optional)
@@ -293,17 +293,16 @@ __global__ void __launch_bounds__(kTileThreads) gatstack_kernel(const __grid_con
     // ---- world step + reward: the tick of tile_kernels.cu ------------------------------------------------------------
     float reward = 0.0f;
     if (t.active) {
+      const bool oa = c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE;
       uint8_t flags = 0;
       uint32_t cmask = 0;
-      tile_world_step(p.step, t, pos, action, s, flags, cmask);
-      const float dgoal = goal_distance(s.x, s.y, c);
-      if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-        const float dobs = obstacle_distance(s.x, s.y, c);
-        reward = oa_reward(dgoal, dobs, c, flags);
-        myhits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
-      } else if (!p.use_flock) {
-        sred[tid] = dgoal;     // GoTo's collective reward needs every agent's distance: finished below
-      }
+      float2 u;
+      decode_action(action, u.x, u.y);
+      agent_step(s, u, pos + t.envbase, N, t.i, oa, c, p.step, flags, cmask);
+      float dgoal, dobs;
+      reward = post_step_reward(s, oa, c, dgoal, dobs, flags);
+      if (oa) myhits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
+      else if (!p.use_flock) sred[tid] = dgoal;     // GoTo's collective reward needs every agent's distance: finished below
     }
     if (p.use_flock == 2) {
       // Cohesion (cohesion:66-85): smallest / largest surface distance to the other agents at their POST-step positions;
@@ -422,9 +421,9 @@ static void stack_fill(StackParams& p, const SwarmConfig& c, const SwarmStackSpe
   p.qmax_r = c.graph_mode == SWARM_GRAPH_RADIUS ? sq_threshold(c.graph_radius) : 0.0f;
 }
 
-// the fused evaluation loop; `step` carries the physics constants (api.cu fill_params), flock == nullptr: world reward
+// the fused evaluation loop; flock == nullptr: world reward
 cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
-                                    int ticks, const TileParams& step, const SwarmRewardSpec* flock, float* shaping,
+                                    int ticks, const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
                                     float* returns, int32_t* hits, cudaStream_t stream) {
   if (ticks <= 0) return cudaSuccess;
   StackParams p;

@@ -5,11 +5,12 @@
 // 256 threads per CTA, thread = agent, floor(256/N) whole envs per CTA (N = 12: 252 of 256 lanes busy).  Partner
 // positions are staged once in shared memory as float2; the pair loop is branch-light (the self pair is tested
 // too: it yields a zero force and its mask bit is cleared afterwards) and unrolled for memory-level parallelism.
-// Same arithmetic, in the same order, as the env-tile kernels (swarm_device.cuh), so results are bit-identical to
-// MODE_STEP of tile_kernels.cu.
+// The agent's step is agent_step of swarm_device.cuh, the world step of every other kernel, so results are
+// bit-identical to the fused rollouts' world step.
 //
 // Two kernels with identical arithmetic:
-//   sim_step_kernel         one tile per CTA, plain loads / stores (small batches, ragged tail, unaligned buffers)
+//   sim_step_kernel         one tile per CTA, plain loads / stores (small batches, ragged tail, unaligned buffers,
+//                           swarms of more than 64 agents)
 //   sim_step_stream_kernel  persistent CTAs; every tile of floor(256/N) envs is one contiguous block of the state /
 //                           action arrays, so it is pulled into a 4-deep shared-memory ring by the TMA engine
 //                           (cp.async.bulk + mbarrier complete_tx) and the new state / rewards leave through bulk
@@ -22,21 +23,7 @@ namespace swarm {
 
 constexpr int kStepThreads = 256;
 
-struct StepParams {
-  SwarmConfig cfg;
-  const float4* state_in;
-  const int32_t* actions;
-  float4* state_out;
-  float* rewards;
-  uint8_t* flags;
-  uint32_t* contact;
-  float* obs;
-  float2* dist;
-  int32_t epb;
-  float one_minus_drag, dmin_aa, dmin_ao, qmax_aa, qmax_ao;
-};
-
-__global__ void __launch_bounds__(kStepThreads) sim_step_kernel(const __grid_constant__ StepParams p) {
+__global__ void __launch_bounds__(kStepThreads) sim_step_kernel(const __grid_constant__ SimStepArgs p) {
   __shared__ float2 spos[kStepThreads];
   __shared__ float sdg[kStepThreads];
   const SwarmConfig& c = p.cfg;
@@ -60,41 +47,17 @@ __global__ void __launch_bounds__(kStepThreads) sim_step_kernel(const __grid_con
 
   float reward = 0.0f;
   if (active) {
-    float fx, fy, gx, gy;
-    decode_action(action, fx, fy);
+    const bool oa = c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE;
+    float2 u;
+    decode_action(action, u.x, u.y);
     uint8_t flags = 0;
     uint32_t cmask = 0;
-    if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-      const float dx = __fsub_rn(s.x, c.obstacle_x), dy = __fsub_rn(s.y, c.obstacle_y);
-      if (__fmaf_rn(dy, dy, __fmul_rn(dx, dx)) <= p.qmax_ao) {
-        if (contact_force(s.x, s.y, c.obstacle_x, c.obstacle_y, p.dmin_ao, c.collision_force, c.contact_margin, gx, gy)) {
-          fx = __fadd_rn(fx, gx);
-          fy = __fadd_rn(fy, gy);
-          flags |= SWARM_FLAG_OBSTACLE_CONTACT;
-        }
-      }
-    }
-    agent_contacts(spos + envbase, N, i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin, fx, fy, cmask);
-    integrate(s, fx, fy, c.dt, p.one_minus_drag);
-
-    const float dgoal = goal_distance(s.x, s.y, c);
-    float dobs = 0.0f;
-    if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-      dobs = obstacle_distance(s.x, s.y, c);
-      reward = oa_reward(dgoal, dobs, c, flags);
-    } else {
-      sdg[tid] = dgoal;
-    }
+    agent_step(s, u, spos + envbase, N, i, oa, c, p.world, flags, cmask);
+    float dgoal, dobs;
+    reward = post_step_reward(s, oa, c, dgoal, dobs, flags);
+    if (!oa) sdg[tid] = dgoal;
     p.state_out[gidx] = s;
-    if (p.flags) p.flags[gidx] = flags;
-    if (p.contact) p.contact[gidx] = cmask;
-    if (p.obs) {
-      float2* o = reinterpret_cast<float2*>(p.obs + gidx * 6);
-      o[0] = make_float2(s.x, s.y);
-      o[1] = make_float2(s.z, s.w);
-      o[2] = make_float2(c.goal_x, c.goal_y);
-    }
-    if (p.dist) p.dist[gidx] = make_float2(dgoal, dobs);
+    store_step_outputs(p, gidx, s, dgoal, dobs, flags, cmask);
   }
   if (c.scenario == SWARM_SCENARIO_GOTO) {
     // collective reward (go_to:108-115): 0 + (-d_0) + (-d_1) + ... in agent order, same value for every agent
@@ -142,7 +105,7 @@ struct StepStreamSmem {
 // NT: swarm size known at compile time (0 = run-time value): the index arithmetic and the partner sweep of the
 // benchmark shape (12 agents) unroll completely.
 template <bool EXTRAS, bool OA, int NT>
-__global__ void __launch_bounds__(kStepThreads, 4) sim_step_stream_kernel(const __grid_constant__ StepParams p,
+__global__ void __launch_bounds__(kStepThreads, 4) sim_step_stream_kernel(const __grid_constant__ SimStepArgs p,
                                                                           const long long ntiles) {
   __shared__ __align__(128) StepStreamSmem sm;
   const SwarmConfig& c = p.cfg;
@@ -179,48 +142,17 @@ __global__ void __launch_bounds__(kStepThreads, 4) sim_step_stream_kernel(const 
   // bookkeeping are paid once per PAIR of tiles (the kernel is issue bound at ~290 instructions per agent, ~25 of them
   // this per-tile overhead), and the two agents of a thread are independent instruction streams.
   auto step_agent = [&](int stage, int ob, long long gidx, int which) -> float {
-    float reward = 0.0f;
     float4 s = sm.sin[stage][tid];
     const int action = sm.ain[stage][tid];
-    float gx, gy;
     const float2 u = sm.force_of_action[min((unsigned)action, 9u)];      // vmas _set_action (a // 3, a % 3) -> (0, -1, +1)
-    float fx = u.x, fy = u.y;
     uint8_t flags = 0;
     uint32_t cmask = 0;
-    if (OA) {
-      const float dx = __fsub_rn(s.x, c.obstacle_x), dy = __fsub_rn(s.y, c.obstacle_y);
-      if (__fmaf_rn(dy, dy, __fmul_rn(dx, dx)) <= p.qmax_ao) {
-        if (contact_force(s.x, s.y, c.obstacle_x, c.obstacle_y, p.dmin_ao, c.collision_force, c.contact_margin, gx, gy)) {
-          fx = __fadd_rn(fx, gx);
-          fy = __fadd_rn(fy, gy);
-          flags |= SWARM_FLAG_OBSTACLE_CONTACT;
-        }
-      }
-    }
-    agent_contacts(&sm.sin[stage][envbase], N, i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin, fx,
-                   fy, cmask);
-    integrate(s, fx, fy, c.dt, p.one_minus_drag);
-
-    const float dgoal = goal_distance(s.x, s.y, c);
-    float dobs = 0.0f;
-    if (OA) {
-      dobs = obstacle_distance(s.x, s.y, c);
-      reward = oa_reward(dgoal, dobs, c, flags);
-    } else {
-      sm.sdg[which][tid] = dgoal;
-    }
+    agent_step(s, u, &sm.sin[stage][envbase], N, i, OA, c, p.world, flags, cmask);
+    float dgoal, dobs;
+    const float reward = post_step_reward(s, OA, c, dgoal, dobs, flags);
+    if (!OA) sm.sdg[which][tid] = dgoal;
     sm.sout[ob][tid] = s;
-    if (EXTRAS) {
-      if (p.flags) p.flags[gidx] = flags;
-      if (p.contact) p.contact[gidx] = cmask;
-      if (p.obs) {
-        float2* o = reinterpret_cast<float2*>(p.obs + gidx * 6);
-        o[0] = make_float2(s.x, s.y);
-        o[1] = make_float2(s.z, s.w);
-        o[2] = make_float2(c.goal_x, c.goal_y);
-      }
-      if (p.dist) p.dist[gidx] = make_float2(dgoal, dobs);
-    }
+    if (EXTRAS) store_step_outputs(p, gidx, s, dgoal, dobs, flags, cmask);
     return reward;
   };
 
@@ -282,30 +214,18 @@ __global__ void __launch_bounds__(kStepThreads, 4) sim_step_stream_kernel(const 
 
 static bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15u) == 0; }
 
-cudaError_t launch_sim_step(const TileParams& tp, cudaStream_t stream) {
-  StepParams p;
-  p.cfg = tp.cfg;
-  p.state_in = reinterpret_cast<const float4*>(tp.state_in);
-  p.actions = tp.actions_in;
-  p.state_out = reinterpret_cast<float4*>(tp.state_out);
-  p.rewards = tp.rewards_out;
-  p.flags = tp.flags_out;
-  p.contact = tp.contact_out;
-  p.obs = tp.obs_out;
-  p.dist = reinterpret_cast<float2*>(tp.dist_out);
-  p.one_minus_drag = tp.one_minus_drag;
-  p.dmin_aa = tp.dmin_aa;
-  p.dmin_ao = tp.dmin_ao;
-  p.qmax_aa = tp.qmax_aa;
-  p.qmax_ao = tp.qmax_ao;
-  const int N = tp.cfg.n_agents;
+cudaError_t launch_sim_step(SimStepArgs p, cudaStream_t stream) {
+  const int N = p.cfg.n_agents;
+  const long long num_envs = p.cfg.num_envs;
   long long env0 = 0;
 
-  // streaming path: full tiles whose agent count is a multiple of 4 (16-byte bulk copies), all buffers 16-byte aligned,
-  // and at least one tile per SM -- everything else (and the ragged tail) runs through the one-tile-per-CTA kernel
-  int epb_s = kStepThreads / N;
+  // streaming path: at most 64 agents, full tiles whose agent count is a multiple of 4 (16-byte bulk copies), all
+  // buffers 16-byte aligned, and at least one tile per SM -- everything else (and the ragged tail) runs through the
+  // one-tile-per-CTA kernel.  Larger swarms are bound by the O(N) contact sweep, not by HBM: at 96 and 128 agents
+  // (16 384 envs, B200) the persistent pipelined kernel took 2-11 % longer than one tile per CTA.
+  int epb_s = N <= 64 ? kStepThreads / N : 0;
   while (epb_s > 0 && ((epb_s * N) & 3)) --epb_s;
-  const long long ntiles = epb_s > 0 ? tp.cfg.num_envs / epb_s : 0;
+  const long long ntiles = epb_s > 0 ? num_envs / epb_s : 0;
   if (ntiles >= 148 && aligned16(p.state_in) && aligned16(p.actions) && aligned16(p.state_out) &&
       (!p.rewards || aligned16(p.rewards))) {
     p.epb = epb_s;
@@ -336,7 +256,7 @@ cudaError_t launch_sim_step(const TileParams& tp, cudaStream_t stream) {
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return err;
     env0 = ntiles * epb_s;
-    if (env0 == tp.cfg.num_envs) return cudaSuccess;
+    if (env0 == num_envs) return cudaSuccess;
     const long long a0 = env0 * N;
     p.state_in += a0;
     p.actions += a0;
@@ -346,7 +266,7 @@ cudaError_t launch_sim_step(const TileParams& tp, cudaStream_t stream) {
     if (p.contact) p.contact += a0;
     if (p.obs) p.obs += a0 * 6;
     if (p.dist) p.dist += a0;
-    p.cfg.num_envs = (int)(tp.cfg.num_envs - env0);
+    p.cfg.num_envs = (int)(num_envs - env0);
   }
   p.epb = kStepThreads / N;
   const long long grid = ((long long)p.cfg.num_envs + p.epb - 1) / p.epb;

@@ -10,11 +10,56 @@
 #define SWARM_DEVICE_CUH
 
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 
 #include "../../include/swarm_b200.h"
 
 namespace swarm {
+
+// largest float q with sqrtf(q) <= dmin: makes a squared-distance test exactly equivalent to the reference's
+// `vector_norm(delta) <= dmin` test on the rounded norm (host side)
+inline float sq_threshold(float dmin) {
+  if (!(dmin < 1e18f)) return INFINITY;
+  float q = dmin * dmin;
+  while (sqrtf(q) > dmin) q = nextafterf(q, 0.0f);
+  while (sqrtf(nextafterf(q, INFINITY)) <= dmin) q = nextafterf(q, INFINITY);
+  return q;
+}
+
+// the world step's constants, computed once on the host (world_consts)
+struct WorldConsts {
+  float one_minus_drag;
+  float dmin_aa, dmin_ao;        // contact distances agent-agent / agent-obstacle (sum of radii, f32 add)
+  float qmax_aa, qmax_ao;        // largest squared distance whose rounded sqrt is <= dmin (exact pre-filter)
+};
+
+inline WorldConsts world_consts(const SwarmConfig& c) {
+  WorldConsts w;
+  w.one_minus_drag = (float)(1.0 - (double)c.drag);
+  w.dmin_aa = c.agent_radius + c.agent_radius;
+  w.dmin_ao = c.landmark_radius + c.agent_radius;
+  w.qmax_aa = sq_threshold(w.dmin_aa);
+  w.qmax_ao = sq_threshold(w.dmin_ao);
+  return w;
+}
+
+// parameter block of the stand-alone world-step kernels (step_kernels.cu, large_kernels.cu, grid_kernels.cu)
+struct SimStepArgs {
+  SwarmConfig cfg;
+  const float4* state_in;
+  const int32_t* actions;
+  float4* state_out;
+  float* rewards;                // optional outputs from here on
+  uint8_t* flags;
+  uint32_t* contact;
+  float* obs;
+  float2* dist;
+  int32_t epb;                   // envs per block (step_kernels.cu)
+  WorldConsts world;
+  float* returns;                // += reward (large swarms)
+  int32_t* hits;                 // += agents inside hit_distance (large swarms)
+};
 
 // ---- 2-norm exactly like torch.linalg.vector_norm over two floats -------------------------------
 __device__ __forceinline__ float norm2(float x, float y) {
@@ -218,6 +263,60 @@ __device__ __forceinline__ float oa_reward(float d_goal, float d_obs, const Swar
   }
   if (d_obs <= c.hit_distance) flags |= SWARM_FLAG_HIT;
   return __fadd_rn(-d_goal, __fmul_rn(c.obstacle_weight, avoid));
+}
+
+// ---- vmas World.step of one agent -----------------------------------------------------------------
+// The ObstacleAvoidance landmark's contact force on the agent at s, behind the exact squared-distance pre-filter: added
+// to (fx, fy), with the contact flag.
+__device__ __forceinline__ void obstacle_contact(const float4& s, const SwarmConfig& c, const WorldConsts& w, float& fx,
+                                                 float& fy, uint8_t& flags) {
+  const float dx = __fsub_rn(s.x, c.obstacle_x), dy = __fsub_rn(s.y, c.obstacle_y);
+  if (__fmaf_rn(dy, dy, __fmul_rn(dx, dx)) <= w.qmax_ao) {
+    float gx, gy;
+    if (contact_force(s.x, s.y, c.obstacle_x, c.obstacle_y, w.dmin_ao, c.collision_force, c.contact_margin, gx, gy)) {
+      fx = __fadd_rn(fx, gx);
+      fy = __fadd_rn(fy, gy);
+      flags |= SWARM_FLAG_OBSTACLE_CONTACT;
+    }
+  }
+}
+
+// Force = decoded action u, + the obstacle's (oa: ObstacleAvoidance; pass a constant where there is one, so the branch
+// folds), + the agents' in ascending partner order (`partners` = the env's positions, `self` = own index); then
+// integration of s.
+template <typename P>
+__device__ __forceinline__ void agent_step(float4& s, float2 u, const P* __restrict__ partners, int N, int self, bool oa,
+                                           const SwarmConfig& c, const WorldConsts& w, uint8_t& flags, uint32_t& cmask) {
+  float fx = u.x, fy = u.y;
+  if (oa) obstacle_contact(s, c, w, fx, fy, flags);
+  agent_contacts(partners, N, self, s.x, s.y, w.qmax_aa, w.dmin_aa, c.collision_force, c.contact_margin, fx, fy, cmask);
+  integrate(s, fx, fy, c.dt, w.one_minus_drag);
+}
+
+// scenario.reward(agent) on the post-step state s: d_goal, d_obs (0 for GoTo) and the ObstacleAvoidance reward with its
+// flags (0 for GoTo, whose collective sum over the env's d_goal each caller adds from its own shared-memory layout)
+__device__ __forceinline__ float post_step_reward(const float4& s, bool oa, const SwarmConfig& c, float& dgoal,
+                                                  float& dobs, uint8_t& flags) {
+  dgoal = goal_distance(s.x, s.y, c);
+  dobs = 0.0f;
+  if (!oa) return 0.0f;
+  dobs = obstacle_distance(s.x, s.y, c);
+  return oa_reward(dgoal, dobs, c, flags);
+}
+
+// the optional per-agent outputs of a stand-alone world step: observation [pos, vel, goal], (d_goal, d_obs), flags and
+// agent-contact mask
+__device__ __forceinline__ void store_step_outputs(const SimStepArgs& p, long long gidx, const float4& s, float dgoal,
+                                                   float dobs, uint8_t flags, uint32_t cmask) {
+  if (p.flags) p.flags[gidx] = flags;
+  if (p.contact) p.contact[gidx] = cmask;
+  if (p.obs) {
+    float2* o = reinterpret_cast<float2*>(p.obs + gidx * 6);
+    o[0] = make_float2(s.x, s.y);
+    o[1] = make_float2(s.z, s.w);
+    o[2] = make_float2(p.cfg.goal_x, p.cfg.goal_y);
+  }
+  if (p.dist) p.dist[gidx] = make_float2(dgoal, dobs);
 }
 
 // ---- generate_grid (go_to:52-80): offsets are Python doubles, cast to f32, added to the f32 centre ----

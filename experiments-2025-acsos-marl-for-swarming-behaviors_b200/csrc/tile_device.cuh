@@ -1,5 +1,5 @@
 // tile_device.cuh -- device functions of the env-tile scheme (thread = agent, CTA = floor(128/N) envs),
-// shared by the rollout / forward / step / graph kernels (tile_kernels.cu) and the DQN gradient kernel
+// shared by the rollout / forward / graph kernels (tile_kernels.cu) and the DQN gradient kernel
 // (dqn_kernels.cu).
 #ifndef SWARM_TILE_DEVICE_CUH
 #define SWARM_TILE_DEVICE_CUH
@@ -49,31 +49,6 @@ __device__ __forceinline__ TileThread tile_thread(int n_agents, int epb, long lo
   t.envbase = t.el * n_agents;
   t.gidx = t.env * n_agents + t.i;
   return t;
-}
-
-// One world step for the agent of this thread: action decode, contact forces (obstacle first, then
-// agents in entity order), integration.  `pos` = pre-step states of the tile.  NT: swarm size at compile time (0 = the
-// run-time value), so that the partner sweep unrolls.
-template <int NT = 0>
-__device__ __forceinline__ void tile_world_step(const TileParams& p, const TileThread& t, const float4* pos, int action,
-                                                float4& s, uint8_t& flags, uint32_t& cmask) {
-  const SwarmConfig& c = p.cfg;
-  const int N = NT > 0 ? NT : c.n_agents;
-  float fx, fy, gx, gy;
-  decode_action(action, fx, fy);          // F = 0 + u
-  if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-    const float dx = __fsub_rn(s.x, c.obstacle_x), dy = __fsub_rn(s.y, c.obstacle_y);
-    if (__fmaf_rn(dy, dy, __fmul_rn(dx, dx)) <= p.qmax_ao) {
-      if (contact_force(s.x, s.y, c.obstacle_x, c.obstacle_y, p.dmin_ao, c.collision_force, c.contact_margin, gx, gy)) {
-        fx = __fadd_rn(fx, gx);
-        fy = __fadd_rn(fy, gy);
-        flags |= SWARM_FLAG_OBSTACLE_CONTACT;
-      }
-    }
-  }
-  agent_contacts(pos + t.envbase, N, t.i, s.x, s.y, p.qmax_aa, p.dmin_aa, c.collision_force, c.contact_margin,
-                 fx, fy, cmask);
-  integrate(s, fx, fy, c.dt, p.one_minus_drag);
 }
 
 // Shared-memory views used by the graph + GAT forward

@@ -3,13 +3,13 @@
 // One thread owns one agent; a CTA of 128 threads owns floor(128 / N) whole envs, so everything an
 // agent needs from its swarm (partner positions, projected features, attention terms, kNN rows) is
 // exchanged through shared memory and no env ever straddles a CTA.  The same device code is
-// instantiated in four modes:
+// instantiated in three modes:
 //   MODE_ROLLOUT  T x [graph -> GAT-Q -> (eps-)greedy -> world step (-> replay push)], state resident in
 //                 registers (simulator.py:59-93 / train_gcn_dqn.py:153-178 inner loops)
 //   MODE_FORWARD  graph -> GAT-Q (-> argmax) once                         (train_gcn_dqn.py:59-70)
-//   MODE_STEP     one world step with given actions                       (vmas Environment.step)
 //   MODE_GRAPH    edge list / neighbour table export                      (train:94-110, simulator:9-26)
-// so the stand-alone kernels and the fused rollout are consistent by construction.
+// so the stand-alone kernels and the fused rollout are consistent by construction.  The rollout's world step is the
+// agent_step of swarm_device.cuh, which the stand-alone world-step kernels (step_kernels.cu) run as well.
 #include <cstdlib>
 
 #include "tile_tc_device.cuh"
@@ -31,11 +31,10 @@ namespace swarm {
 // other attention heads and every per-tick test of an optional pointer are compiled out, which leaves the tick a
 // straight line of about a quarter of the generic kernel's code.  Same arithmetic, same bits.
 template <int MODE, bool TC, bool DENSE, bool FLOCK = false, int NT = 0, bool PLAIN = false>
-__global__ void __launch_bounds__(kTileThreads, (MODE == MODE_GRAPH || MODE == MODE_STEP) ? 8 : ((TC && !DENSE) ? 3 : 4))
+__global__ void __launch_bounds__(kTileThreads, MODE == MODE_GRAPH ? 8 : ((TC && !DENSE) ? 3 : 4))
 tile_kernel(const __grid_constant__ TileParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
   constexpr bool kQ = (MODE == MODE_ROLLOUT || MODE == MODE_FORWARD);
-  constexpr bool kStep = (MODE == MODE_ROLLOUT || MODE == MODE_STEP);
   constexpr bool kGraphOut = (MODE == MODE_GRAPH || MODE == MODE_ROLLOUT);
 
   const SwarmConfig& c = p.cfg;
@@ -207,12 +206,10 @@ tile_kernel(const __grid_constant__ TileParams p) {
     }
 
     // ------------------------------------------------------------------ world step ------------
-    if (kStep) {
+    if (MODE == MODE_ROLLOUT) {
       float reward = 0.0f;
       if (t.active) {
-        if (MODE == MODE_STEP) {
-          action = p.actions_in[t.gidx];
-        } else if (!PLAIN) {
+        if (!PLAIN) {
           if (epsilon > 0.0f) {
             // train:164-165: one coin per tick for the whole swarm, then one uniform action per agent
             const unsigned long long genv = (unsigned long long)(p.env_offset + t.env);
@@ -226,30 +223,18 @@ tile_kernel(const __grid_constant__ TileParams p) {
           }
         }
         const float4 s_prev = s;
+        const bool oa = c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE;
         uint8_t flags = 0;
         uint32_t cmask = 0;
-        tile_world_step<NT>(p, t, pos, action, s, flags, cmask);
+        float2 u;
+        decode_action(action, u.x, u.y);
+        agent_step(s, u, pos + t.envbase, N, t.i, oa, c, p.world, flags, cmask);
 
-        // scenario.reward(agent) on the post-step state
-        const float dgoal = goal_distance(s.x, s.y, c);
-        float dobs = 0.0f;
-        if (c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE) {
-          dobs = obstacle_distance(s.x, s.y, c);
-          reward = oa_reward(dgoal, dobs, c, flags);
-          myhits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
-        } else if (!FLOCK) {
-          sred[tid] = dgoal;     // GoTo's collective reward needs every agent's distance: finished below
-        }
-        if (MODE == MODE_STEP) {
-          reinterpret_cast<float4*>(p.state_out)[t.gidx] = s;
-          if (p.flags_out) p.flags_out[t.gidx] = flags;
-          if (p.contact_out) p.contact_out[t.gidx] = cmask;
-          if (p.obs_out) {
-            float* o = p.obs_out + t.gidx * 6;
-            o[0] = s.x; o[1] = s.y; o[2] = s.z; o[3] = s.w; o[4] = c.goal_x; o[5] = c.goal_y;
-          }
-          if (p.dist_out) reinterpret_cast<float2*>(p.dist_out)[t.gidx] = make_float2(dgoal, dobs);
-        } else if (!PLAIN) {
+        float dgoal, dobs;
+        reward = post_step_reward(s, oa, c, dgoal, dobs, flags);
+        if (oa) myhits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
+        else if (!FLOCK) sred[tid] = dgoal;     // GoTo's collective reward needs every agent's distance: finished below
+        if (!PLAIN) {
           const long long tb = (long long)tick * BN + t.gidx;
           if (p.trace.state) reinterpret_cast<float4*>(p.trace.state)[tb] = s;
           if (p.trace.actions) p.trace.actions[tb] = action;
@@ -303,9 +288,7 @@ tile_kernel(const __grid_constant__ TileParams p) {
       }
       if (t.active) {
         ret = __fadd_rn(ret, reward);
-        if (MODE == MODE_STEP) {
-          if (p.rewards_out) p.rewards_out[t.gidx] = reward;
-        } else if (!PLAIN) {
+        if (!PLAIN) {
           if (p.trace.rewards) p.trace.rewards[(long long)tick * BN + t.gidx] = reward;
           if (p.replay.state) {
             const long long slot = (replay_cursor + (long long)tick * c.num_envs + t.env) % p.replay.capacity;
@@ -480,7 +463,6 @@ cudaError_t launch_tile(int mode, const TileParams& p, cudaStream_t stream) {
   switch (mode) {
     case MODE_ROLLOUT: return p.use_flock ? launch_tile_flock(p, stream) : launch_tile_q<MODE_ROLLOUT>(p, stream);
     case MODE_FORWARD: return launch_tile_q<MODE_FORWARD>(p, stream);
-    case MODE_STEP: return launch_tile_impl<MODE_STEP, false, true>(p, stream);
     case MODE_GRAPH: return launch_tile_impl<MODE_GRAPH, false, true>(p, stream);
     default: return cudaErrorInvalidValue;
   }

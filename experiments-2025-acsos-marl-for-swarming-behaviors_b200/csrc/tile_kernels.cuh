@@ -3,8 +3,6 @@
 #ifndef SWARM_TILE_KERNELS_CUH
 #define SWARM_TILE_KERNELS_CUH
 
-#include <math.h>
-
 #include "swarm_device.cuh"
 
 namespace swarm {
@@ -81,24 +79,19 @@ __device__ __forceinline__ void stage_weights(const float* __restrict__ g, float
   }
 }
 
-enum TileMode { MODE_ROLLOUT = 0, MODE_FORWARD = 1, MODE_STEP = 2, MODE_GRAPH = 3 };
+enum TileMode { MODE_ROLLOUT = 0, MODE_FORWARD = 1, MODE_GRAPH = 3 };
 
 struct TileParams {
   SwarmConfig cfg;
   const float* weights;          // packed state-dict order (SWARM_W_*)
   const float* state_in;
   float* state_out;
-  const int32_t* actions_in;     // MODE_STEP: [B*N]; MODE_ROLLOUT: optional forced actions [ticks][B*N]
+  const int32_t* actions_in;     // MODE_ROLLOUT: optional forced actions [ticks][B*N]
   float* returns;                // MODE_ROLLOUT: [B*N] +=
   int32_t* hits;                 // MODE_ROLLOUT: [B] +=
   SwarmTrace trace;              // MODE_ROLLOUT, optional
   float* q_out;                  // MODE_FORWARD
   int32_t* act_out;              // MODE_FORWARD
-  float* rewards_out;            // MODE_STEP
-  uint8_t* flags_out;            // MODE_STEP
-  uint32_t* contact_out;         // MODE_STEP
-  float* obs_out;                // MODE_STEP
-  float* dist_out;               // MODE_STEP
   int32_t* edges_out;            // MODE_GRAPH
   int32_t* nbr_out;              // MODE_GRAPH
   SwarmReplay replay;            // MODE_ROLLOUT, optional (state == nullptr: no push)
@@ -115,10 +108,8 @@ struct TileParams {
                                  // b * bal_q + min(b, bal_r) on -- a single-wave grid spread evenly over every CTA slot
   int32_t maxdeg;                // max in-degree of the graph (rows of the per-thread edge scratch)
   int32_t edges_per_env;
-  float one_minus_drag;
-  float dmin_aa, dmin_ao;        // contact distances agent-agent / agent-obstacle (sum of radii, f32 add)
-  float qmax_aa, qmax_ao;        // largest squared distance whose rounded sqrt is <= dmin (exact pre-filter)
-  float qmax_r;                  // same for the radius graph: sqrt(q) <= graph_radius  <=>  q <= qmax_r
+  WorldConsts world;
+  float qmax_r;                  // largest q with sqrt(q) <= graph_radius (radius graph)
   int32_t* counts_out;           // MODE_GRAPH, radius graph: edges per env
   // MODE_ROLLOUT, FLOCK variant: the Flocking reward (flocking_scenario.py:124-171) instead of GoTo's on the GoTo world
   SwarmRewardSpec flock;         // its constants
@@ -129,16 +120,6 @@ struct TileParams {
   uint32_t knn_memo_mask;        // entries - 1
   int32_t knn_ordered;           // 1: always run the ordered (torch.topk output order) row code (SWARM_KNN_ORDERED=1)
 };
-
-// largest float q with sqrtf(q) <= dmin: makes a squared-distance test exactly equivalent to the reference's
-// `vector_norm(delta) <= dmin` test on the rounded norm (host side)
-inline float sq_threshold(float dmin) {
-  if (!(dmin < 1e18f)) return INFINITY;
-  float q = dmin * dmin;
-  while (sqrtf(q) > dmin) q = nextafterf(q, 0.0f);
-  while (sqrtf(nextafterf(q, INFINITY)) <= dmin) q = nextafterf(q, INFINITY);
-  return q;
-}
 
 // byte offsets of the dynamic shared memory regions
 struct TileLayout {

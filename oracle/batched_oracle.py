@@ -30,6 +30,7 @@ def step(scenario: str, pos: torch.Tensor, vel: torch.Tensor, actions: torch.Ten
     obstacle = torch.tensor(list(so.OBSTACLE_POS)).expand(B, 2)
     dist_min = torch.tensor(so.SPHERE_RADIUS) + torch.tensor(so.SPHERE_RADIUS)
     contact = torch.zeros(B, N, dtype=torch.int64)
+    agent_contact = torch.zeros(B, N, dtype=torch.bool)              # any partner, also where the mask has no bit
     obstacle_contact = torch.zeros(B, N, dtype=torch.bool)
 
     if scenario == so.OBSTACLE_AVOIDANCE:
@@ -43,6 +44,8 @@ def step(scenario: str, pos: torch.Tensor, vel: torch.Tensor, actions: torch.Ten
             forces[i] = forces[i] + f
             forces[j] = forces[j] + (-f)
             hit = torch.linalg.vector_norm(pos[:, i] - pos[:, j], dim=-1) <= dist_min
+            agent_contact[:, i] |= hit
+            agent_contact[:, j] |= hit
             if i < 63 and j < 63:
                 contact[:, i] |= hit.to(torch.int64) << j
                 contact[:, j] |= hit.to(torch.int64) << i
@@ -73,7 +76,7 @@ def step(scenario: str, pos: torch.Tensor, vel: torch.Tensor, actions: torch.Ten
         flags |= (d_obs <= so.HIT_DISTANCE).to(torch.uint8) * 2
         flags |= (d_obs <= so.PENALTY_DISTANCE).to(torch.uint8) * 4
     return {"pos": new_pos, "vel": new_vel, "rewards": rewards, "flags": flags, "contact": contact,
-            "d_goal": d_goal, "d_obs": d_obs}
+            "agent_contact": agent_contact, "d_goal": d_goal, "d_obs": d_obs}
 
 
 def node_features(pos: torch.Tensor, vel: torch.Tensor) -> torch.Tensor:
