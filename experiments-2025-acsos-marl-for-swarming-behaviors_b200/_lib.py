@@ -22,7 +22,7 @@ FLAG_OBSTACLE_CONTACT = 1
 FLAG_HIT = 2
 FLAG_PENALTY = 4
 W_COUNT = 1673
-ABI_VERSION = 4
+ABI_VERSION = 5
 XCHG_STRIDE = 1680
 
 # state-dict tensors in packed order (include/swarm_b200.h SWARM_W_*)
@@ -124,6 +124,13 @@ _SIGNATURES = {
     "swarm_rollout_stack_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig)]),
     "swarm_rollout_stack": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p, C.c_int32,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "swarm_dqn_stack_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_int32]),
+    "swarm_dqn_stack_grad": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p,
+                                       C.POINTER(SwarmReplay), C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "swarm_adam_clip_stack_step": (C.c_int, [C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
+                                             C.c_void_p, C.c_void_p, C.c_void_p]),
     "swarm_graph_build_radius_csr": (C.c_int, [C.POINTER(SwarmConfig)] + [C.c_void_p] * 5),
     "swarm_gatq_forward_large": (C.c_int, [C.POINTER(SwarmConfig)] + [C.c_void_p] * 5),
     "swarm_gatq_forward": (C.c_int, [C.POINTER(SwarmConfig)] + [C.c_void_p] * 5),

@@ -37,6 +37,14 @@ cudaError_t launch_gatstack_forward(const SwarmConfig& c, const SwarmStackSpec& 
 cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
                                     int ticks, const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
                                     float* returns, int32_t* hits, cudaStream_t stream);
+int stack_grad_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
+long long stack_grad_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s, int n_graphs);
+cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, const float* w_online, const float* w_target,
+                              const SwarmReplay& batch, const int64_t* indices, int n_graphs, float gamma, float loss_scale,
+                              float* grad, float* loss, float* td, void* workspace, cudaStream_t stream);
+cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const float* grad, float* m, float* v,
+                                   long long step, double lr, double beta1, double beta2, double eps, double max_norm,
+                                   float* target, float* grad_norm, cudaStream_t stream);
 cudaError_t launch_stack_accumulate(long long total, int N, const float* rewards, int per_env, const uint8_t* flags,
                                     float* returns, int32_t* hits, cudaStream_t stream);
 bool gatq_knn_large_fits(int N, int K);
@@ -826,6 +834,62 @@ int swarm_gatstack_forward(const SwarmConfig* cfg, const SwarmStackSpec* spec, c
   if (!q && !actions) return fail(SWARM_ERR_INVALID_ARG, "no output requested");
   return check_cuda(launch_gatstack_forward(*cfg, *spec, weights, state, q, actions, (cudaStream_t)stream),
                     "swarm_gatstack_forward");
+}
+
+namespace {
+int validate_spec(const SwarmStackSpec* spec) {
+  if (!spec) return fail(SWARM_ERR_INVALID_ARG, "spec is NULL");
+  if (spec->n_layers < 1 || spec->n_layers > 4) return fail(SWARM_ERR_INVALID_ARG, "n_layers must be 1 .. 4");
+  if (spec->hidden < 1 || spec->hidden > 32) return fail(SWARM_ERR_UNSUPPORTED, "hidden must be 1 .. 32");
+  if (spec->in_features != 7 && spec->in_features != 5) return fail(SWARM_ERR_INVALID_ARG, "in_features must be 7 or 5");
+  return SWARM_OK;
+}
+
+// the checks of swarm_gatstack_forward on a batch of n_graphs transitions, then the gradient tile's shared memory
+int validate_dqn_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, int32_t n_graphs) {
+  if (!cfg) return fail(SWARM_ERR_INVALID_ARG, "cfg is NULL");
+  if (n_graphs <= 0) return fail(SWARM_ERR_INVALID_ARG, "n_graphs must be positive");
+  SwarmConfig c = *cfg;
+  c.num_envs = n_graphs;
+  if (int rc = validate_stack(&c, spec)) return rc;
+  if (c.n_agents < 2) return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN update needs n_agents >= 2");
+  if (stack_grad_smem_bytes(c, *spec) > 227 * 1024)
+    return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN gradient tile exceeds 227 KB of shared memory for this (N, k, spec)");
+  return SWARM_OK;
+}
+}  // namespace
+
+int64_t swarm_dqn_stack_workspace_bytes(const SwarmConfig* cfg, const SwarmStackSpec* spec, int32_t n_graphs) {
+  if (validate_dqn_stack(cfg, spec, n_graphs) != SWARM_OK) return 0;
+  return stack_grad_workspace_bytes(*cfg, *spec, n_graphs);
+}
+
+int swarm_dqn_stack_grad(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* online_weights,
+                         const float* target_weights, const SwarmReplay* batch, const int64_t* indices, int32_t n_graphs,
+                         float gamma, float loss_scale, float* grad, float* loss, float* td, void* workspace,
+                         int64_t workspace_bytes, void* stream) {
+  if (int rc = validate_dqn_stack(cfg, spec, n_graphs)) return rc;
+  if (!online_weights || !target_weights || !grad || !loss || !workspace) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
+  if (!batch || !batch->state || !batch->next_state || !batch->actions || !batch->rewards)
+    return fail(SWARM_ERR_INVALID_ARG, "batch has NULL arrays");
+  if (workspace_bytes < stack_grad_workspace_bytes(*cfg, *spec, n_graphs))
+    return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  return check_cuda(launch_stack_grad(*cfg, *spec, online_weights, target_weights, *batch, indices, n_graphs, gamma,
+                                      loss_scale, grad, loss, td, workspace, (cudaStream_t)stream),
+                    "swarm_dqn_stack_grad");
+}
+
+int swarm_adam_clip_stack_step(const SwarmStackSpec* spec, float* weights, const float* grad, float* exp_avg,
+                               float* exp_avg_sq, int64_t step, double lr, double beta1, double beta2, double eps,
+                               double max_norm, float* target_weights, float* grad_norm, void* stream) {
+  if (int rc = validate_spec(spec)) return rc;
+  if (!weights || !grad || !exp_avg || !exp_avg_sq) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
+  if (step < 1) return fail(SWARM_ERR_INVALID_ARG, "step is 1-based");
+  if (!(lr >= 0.0) || !(beta1 >= 0.0 && beta1 < 1.0) || !(beta2 >= 0.0 && beta2 < 1.0) || !(eps >= 0.0))
+    return fail(SWARM_ERR_INVALID_ARG, "invalid Adam hyper-parameter");     // torch.optim.Adam's ValueError checks
+  return check_cuda(launch_stack_adam_clip(*spec, weights, grad, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_norm,
+                                           target_weights, grad_norm, (cudaStream_t)stream),
+                    "swarm_adam_clip_stack_step");
 }
 
 int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg) {

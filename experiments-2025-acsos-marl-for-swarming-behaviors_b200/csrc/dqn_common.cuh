@@ -1,5 +1,5 @@
 // dqn_common.cuh -- parameter block shared by the two DQN gradient kernels (dqn_kernels.cu: CUDA-core parity path,
-// dqn_tc_kernels.cu: tensor-core path).
+// dqn_tc_kernels.cu: tensor-core path) and the Adam element update of the clip + Adam kernels.
 #ifndef SWARM_DQN_COMMON_CUH
 #define SWARM_DQN_COMMON_CUH
 
@@ -35,6 +35,25 @@ struct DqnParams {
 __device__ __forceinline__ long long train_ring_size(const SwarmTrainCtl* ctl, int pushed, long long capacity) {
   const long long size = ctl->ring_size + pushed;
   return size < capacity ? size : capacity;
+}
+
+// one Adam step of one element, op for op as torch.optim.Adam (single-tensor path); shared by the clip + Adam kernels
+// of the one-layer network (dqn_kernels.cu) and of stacked networks (stack_grad_kernels.cu)
+struct AdamScalars {
+  float lerp_w, beta2, one_minus_beta2, neg_step_size, bc2_sqrt, eps;
+};
+__device__ __forceinline__ void adam_element(const AdamScalars& a, float g, float coef, float& m_io, float& v_io, float& w_io) {
+  const float gval = __fmul_rn(g, coef);
+  // exp_avg.lerp_(grad, 1 - beta1)
+  const float m = __fadd_rn(m_io, __fmul_rn(a.lerp_w, __fsub_rn(gval, m_io)));
+  // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, value = 1 - beta2)
+  float v = __fmul_rn(v_io, a.beta2);
+  v = __fadd_rn(v, __fmul_rn(__fmul_rn(a.one_minus_beta2, gval), gval));
+  // denom = sqrt(v) / sqrt(bias_correction2) + eps ; param.addcdiv_(exp_avg, denom, value = -step_size)
+  const float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), a.bc2_sqrt), a.eps);
+  w_io = __fadd_rn(w_io, __fdiv_rn(__fmul_rn(a.neg_step_size, m), denom));
+  m_io = m;
+  v_io = v;
 }
 
 }  // namespace swarm

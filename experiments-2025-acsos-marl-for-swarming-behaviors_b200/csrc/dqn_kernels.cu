@@ -573,24 +573,6 @@ __device__ __forceinline__ float clip_coefficient(const float (&g_)[kAdamPer], d
   return s_coef;
 }
 
-// one Adam step of one element, op for op as torch.optim.Adam (single-tensor path)
-struct AdamScalars {
-  float lerp_w, beta2, one_minus_beta2, neg_step_size, bc2_sqrt, eps;
-};
-__device__ __forceinline__ void adam_element(const AdamScalars& a, float g, float coef, float& m_io, float& v_io, float& w_io) {
-  const float gval = __fmul_rn(g, coef);
-  // exp_avg.lerp_(grad, 1 - beta1)
-  const float m = __fadd_rn(m_io, __fmul_rn(a.lerp_w, __fsub_rn(gval, m_io)));
-  // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, value = 1 - beta2)
-  float v = __fmul_rn(v_io, a.beta2);
-  v = __fadd_rn(v, __fmul_rn(__fmul_rn(a.one_minus_beta2, gval), gval));
-  // denom = sqrt(v) / sqrt(bias_correction2) + eps ; param.addcdiv_(exp_avg, denom, value = -step_size)
-  const float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), a.bc2_sqrt), a.eps);
-  w_io = __fadd_rn(w_io, __fdiv_rn(__fmul_rn(a.neg_step_size, m), denom));
-  m_io = m;
-  v_io = v;
-}
-
 __device__ __forceinline__ void train_ctl_advance(SwarmTrainCtl* ctl, int num_envs, long long capacity, bool stepped) {
   ctl->tick += 1;
   ctl->ring_cursor = (ctl->ring_cursor + num_envs) % capacity;

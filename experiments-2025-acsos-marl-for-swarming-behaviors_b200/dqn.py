@@ -11,9 +11,14 @@ Two drivers:
     rollout-tick + replay push, G graphs per update (throughput mode); an episode's ticks replay from a CUDA graph.
   * ``DQNTrainer.train_model_device(config)`` -- as above with reset, epsilon schedule and episode statistics on
     the device too: one graph launch per episode, no host synchronisation until the run ends.
+
+``DQNTrainer(..., model=StackedGCN(...))`` trains a stacked network (the conv1 .. convL form the reference ships as
+data/models/experiment_Flocking-seed_*.pth) instead of the one-layer GCN: ``train_model`` and ``train_model_stepwise``
+then run the stack's gradient kernel (``swarm_dqn_stack_grad``) and clip + Adam (``swarm_adam_clip_stack_step``).
 """
 from __future__ import annotations
 
+import copy
 import csv
 import os
 import random
@@ -23,9 +28,9 @@ import numpy as np
 import torch
 
 from . import _lib, ops, parallel
-from .gcn import GCN
+from .gcn import GCN, StackedGCN
 from .graph import Batch, Data, node_features, stack_observations
-from .scenarios import FlockingScenario, _KernelScenario
+from .scenarios import CohesionScenario, FlockingScenario, _KernelScenario
 
 
 class GraphReplayBuffer:
@@ -87,10 +92,12 @@ class GraphReplayBuffer:
 
 
 class DQNTrainer:
-    """train:72-231.  ``env`` is a swarm_b200 Environment (``make_env``)."""
+    """train:72-231.  ``env`` is a swarm_b200 Environment (``make_env``).  ``model``: a ``StackedGCN`` to train instead
+    of the reference's ``GCN(n_input, 32, 9)``; its ``conv1`` must take ``observation dim + 1`` input features, and the
+    target network starts as an exact copy of it."""
 
     def __init__(self, env, seed, models_path, stats_path, experiment, graph_mode: str = "complete", knn_k: int = 10,
-                 replay_capacity: int = 1000000):
+                 replay_capacity: int = 1000000, model: Optional[StackedGCN] = None):
         self.env = env
         self.seed = seed
         self.models_path = models_path
@@ -99,14 +106,25 @@ class DQNTrainer:
         self.n_input = self.env.observation_space["agent0"].shape[0] + 1
         self.n_output = env.action_space["agent0"].n
         dev = env.device
-        # constructors run on the CPU generator exactly like the reference (2 x 1 865 uniform draws)
-        self.model = GCN(input_dim=self.n_input, hidden_dim=32, output_dim=self.n_output)
-        self.target_model = GCN(input_dim=self.n_input, hidden_dim=32, output_dim=self.n_output)
-        self.target_model.load_state_dict(self.model.state_dict())
+        self.stack_spec = None
+        if model is None:
+            # constructors run on the CPU generator exactly like the reference (2 x 1 865 uniform draws)
+            self.model = GCN(input_dim=self.n_input, hidden_dim=32, output_dim=self.n_output)
+            self.target_model = GCN(input_dim=self.n_input, hidden_dim=32, output_dim=self.n_output)
+            self.target_model.load_state_dict(self.model.state_dict())
+        else:
+            if not isinstance(model, StackedGCN):
+                raise TypeError("model must be a StackedGCN")
+            if model.conv1.in_channels != self.n_input:
+                raise ValueError(f"model.conv1 takes {model.conv1.in_channels} input features, the environment's "
+                                 f"observation gives {self.n_input} (observation dim + 1)")
+            self.model = model
+            self.target_model = copy.deepcopy(model)
+            self.stack_spec = model.stack_spec()
         self.model.to(dev)
         self.target_model.to(dev)
         # packed device weights are the training state; the nn.Modules are refreshed from them on demand
-        self.w = _lib.pack_weights(self.model.state_dict(), dev)
+        self.w = _lib.pack_weights(self.model.state_dict(), dev) if model is None else self.model.packed_stack_weights(dev)
         self.w_target = self.w.clone()
         self.exp_avg = torch.zeros_like(self.w)
         self.exp_avg_sq = torch.zeros_like(self.w)
@@ -136,8 +154,41 @@ class DQNTrainer:
 
     def sync_modules(self) -> None:
         """Copy the packed training weights back into the nn.Modules (for state_dict / torch.save)."""
+        if self.stack_spec is not None:
+            self.model.load_state_dict(ops.unpack_stack_weights(self.w, self.stack_spec))
+            self.target_model.load_state_dict(ops.unpack_stack_weights(self.w_target, self.stack_spec))
+            return
         self.model.load_state_dict(_lib.unpack_weights(self.w))
         self.target_model.load_state_dict(_lib.unpack_weights(self.w_target))
+
+    def _dqn_grad(self, cfg, ring, indices, n_graphs, gamma) -> None:
+        """Gradient + loss of one update into self._grad / self._loss, for the trained network's form."""
+        if self.stack_spec is not None:
+            ops.dqn_grad_stack(cfg, self.stack_spec, self.w, self.w_target, ring, indices, n_graphs, gamma=gamma,
+                               grad=self._grad, loss=self._loss)
+        else:
+            ops.dqn_grad(cfg, self.w, self.w_target, ring, indices, n_graphs, gamma=gamma, grad=self._grad, loss=self._loss)
+
+    def _adam_clip(self, target) -> None:
+        """clip_grad_norm_ + Adam step self.opt_step on self._grad (train:125-126), optional target sync."""
+        if self.stack_spec is not None:
+            ops.adam_clip_step_stack(self.stack_spec, self.w, self._grad, self.exp_avg, self.exp_avg_sq, self.opt_step,
+                                     self.lr, self.betas, self.eps, self.max_norm, target=target)
+        else:
+            ops.adam_clip_step(self.w, self._grad, self.exp_avg, self.exp_avg_sq, self.opt_step, self.lr, self.betas,
+                               self.eps, self.max_norm, target=target)
+
+    def _greedy_actions(self, cfg) -> torch.Tensor:
+        """argmax_a Q_online for the world's current state, int32[B, N]."""
+        if self.stack_spec is not None:
+            return ops.gatstack_forward(cfg, self.stack_spec, self.w, self.env.world.state, want_q=False, want_actions=True)
+        _, act = ops.gatq_forward(cfg, self.w, self.env.world.state, want_q=False)
+        return act
+
+    def _require_one_layer(self, what: str) -> None:
+        if self.stack_spec is not None:
+            raise NotImplementedError(f"{what} runs the fused train tick of the one-layer GCN; train a StackedGCN with "
+                                      "train_model_stepwise (or train_model for one env)")
 
     def train_step_dqn(self, batch_size, model=None, target_model=None, ticks=0, gamma=0.99, update_target_every=10,
                        indices: Optional[torch.Tensor] = None):
@@ -150,20 +201,18 @@ class DQNTrainer:
         if indices is None:
             indices = torch.tensor(self.replay_buffer.sample_indices(batch_size), dtype=torch.int64, device=self.w.device)
         cfg = ops.clone_config(self.graph_cfg, num_envs=batch_size)
-        ops.dqn_grad(cfg, self.w, self.w_target, ring, indices, batch_size, gamma=gamma, grad=self._grad, loss=self._loss)
+        self._dqn_grad(cfg, ring, indices, batch_size, gamma)
         self.opt_step += 1
         sync = (ticks % update_target_every == 0)
         if sync:
             print("Updating target model")
-        ops.adam_clip_step(self.w, self._grad, self.exp_avg, self.exp_avg_sq, self.opt_step, self.lr, self.betas, self.eps,
-                           self.max_norm, target=self.w_target if sync else None)
+        self._adam_clip(self.w_target if sync else None)
         return self._loss.item()
 
     def _policy_actions(self) -> torch.Tensor:
         """argmax_a Q(s) for the env's current state with the online weights (train:161-162,167)."""
         cfg = ops.clone_config(self.graph_cfg, num_envs=self.env.num_envs)
-        _, act = ops.gatq_forward(cfg, self.w, self.env.world.state, want_q=False)
-        return act
+        return self._greedy_actions(cfg)
 
     def _rewards_tensor(self, rewards) -> torch.Tensor:
         """The rewards of the tick just stepped as f32[B, n]: what the world-step kernel wrote for the two fused
@@ -231,6 +280,7 @@ class DQNTrainer:
         ``config["cuda_graph"]`` (default on) the ticks of one episode are captured once in a CUDA graph and each
         episode is a single graph launch.  A ``FlockingScenario`` env trains on its collective reward: the tick kernel
         then evaluates the Flocking reward on the GoTo world and keeps the scenario's shaping memory up to date."""
+        self._require_one_layer("train_model_batched")
         flock = isinstance(self.env.scenario, FlockingScenario)
         if not flock and not isinstance(self.env.scenario, _KernelScenario):
             raise NotImplementedError("the fused train tick computes the GoTo / ObstacleAvoidance / Flocking rewards in the "
@@ -343,7 +393,7 @@ class DQNTrainer:
             for _ in range(env.max_steps):
                 ticks += 1
                 state = world.state.clone()
-                _, greedy = ops.gatq_forward(cfg, self.w, world.state, want_q=False)
+                greedy = self._greedy_actions(cfg)
                 explore = torch.rand(B, 1, device=dev, generator=gen) < epsilon
                 rnd = torch.randint(0, 9, (B, n), device=dev, generator=gen, dtype=torch.int32)
                 actions = torch.where(explore, rnd, greedy.view(B, n).to(torch.int32)).contiguous()
@@ -353,11 +403,9 @@ class DQNTrainer:
                 returns += rewards_dev
                 if len(ring) >= G:
                     idx = torch.randint(0, len(ring), (G,), device=dev, generator=gen, dtype=torch.int64)
-                    ops.dqn_grad(gcfg, self.w, self.w_target, ring, idx, G, gamma=gamma, grad=self._grad, loss=self._loss)
+                    self._dqn_grad(gcfg, ring, idx, G, gamma)
                     self.opt_step += 1
-                    ops.adam_clip_step(self.w, self._grad, self.exp_avg, self.exp_avg_sq, self.opt_step, self.lr,
-                                       self.betas, self.eps, self.max_norm,
-                                       target=self.w_target if ticks % every == 0 else None)
+                    self._adam_clip(self.w_target if ticks % every == 0 else None)
                     loss_sum += self._loss
                     updates += 1
             epsilon = max(config["min_epsilon"], config["epsilon"] * np.exp(-config["epsilon_decay"] * episode))
@@ -380,6 +428,7 @@ class DQNTrainer:
         statistics (train:179-199) all live on the device and the host only reads the statistics at the end.
         Per-env start centres come from the counter RNG (``shared_center`` reproduces the reference's one draw per
         reset).  Returns stats f32[episodes, 4] = (mean agent-0 return / N, hits per env, last loss, epsilon)."""
+        self._require_one_layer("train_model_device")
         flock = isinstance(self.env.scenario, FlockingScenario)
         if not (flock or isinstance(self.env.scenario, _KernelScenario)):
             raise NotImplementedError("the whole-run device loop resets GoTo / ObstacleAvoidance / Flocking worlds on the "
@@ -458,6 +507,8 @@ class DQNTrainer:
         total = 0
         n = self.env.n_agents
         cfg = ops.clone_config(self.graph_cfg, num_envs=self.env.num_envs)
+        if self.stack_spec is not None:
+            return self._evaluate_stack(cfg, eval_episodes)
         for _ in range(eval_episodes):
             self.env.reset()
             flock = isinstance(self.env.scenario, FlockingScenario)
@@ -467,6 +518,30 @@ class DQNTrainer:
                               shaping=self.env.scenario.shaping if flock else None)
             self.env.steps += self.env.max_steps
             self.env.world.adopt_rollout(out)
+            total += out["returns"][0, 0].item()
+        return total / eval_episodes
+
+    def _evaluate_stack(self, cfg, eval_episodes):
+        """evaluate_policy for a stacked network: ``swarm_rollout_stack`` with the scenario's reward (the world's own,
+        Flocking with its shaping memory, or Cohesion's per-agent reward)."""
+        total = 0
+        env = self.env
+        for _ in range(eval_episodes):
+            env.reset()
+            reward = shaping = None
+            if isinstance(env.scenario, FlockingScenario):
+                reward, shaping = env.scenario._spec(), env.scenario.shaping
+            elif isinstance(env.scenario, CohesionScenario):
+                reward = ops.reward_spec(_lib.REWARD_COHESION, env.num_envs, env.n_agents,
+                                         agent_radius=env.world.cfg.agent_radius, sigma=env.scenario.sigma)
+            elif not isinstance(env.scenario, _KernelScenario):
+                raise NotImplementedError("evaluate_policy of a StackedGCN covers the GoTo, ObstacleAvoidance, Flocking and "
+                                          "Cohesion rewards")
+            out = ops.rollout_stack(cfg, self.stack_spec, self.w, env.world.state, env.max_steps, reward=reward,
+                                    shaping=shaping)
+            env.steps += env.max_steps
+            env.world.version += 1                 # the state moved under the world: version-keyed caches drop
+            env.world._download()
             total += out["returns"][0, 0].item()
         return total / eval_episodes
 

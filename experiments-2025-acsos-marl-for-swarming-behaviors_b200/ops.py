@@ -582,6 +582,79 @@ def pack_stack_weights(state_dict, spec, device) -> torch.Tensor:
     return packed.to(device)
 
 
+def unpack_stack_weights(packed: torch.Tensor, spec) -> Dict[str, torch.Tensor]:
+    """The inverse of ``pack_stack_weights``: packed float32 vector -> state dict with the reference's key names and
+    shapes (``conv{l}.att_src`` / ``att_dst`` [1,1,H], ``conv{l}.bias`` [H], ``conv{l}.lin.weight`` [H,Cin], ``lin1.*``,
+    ``lin2.*``), as views of ``packed``."""
+    H, out, off = spec.hidden, {}, 0
+
+    def take(key, shape):
+        nonlocal off
+        n = 1
+        for s_ in shape:
+            n *= s_
+        out[key] = packed[off:off + n].reshape(shape)
+        off += n
+
+    for l in range(1, spec.n_layers + 1):
+        take(f"conv{l}.att_src", (1, 1, H))
+        take(f"conv{l}.att_dst", (1, 1, H))
+        take(f"conv{l}.bias", (H,))
+        take(f"conv{l}.lin.weight", (H, spec.in_features if l == 1 else H))
+    take("lin1.weight", (H, H))
+    take("lin1.bias", (H,))
+    take("lin2.weight", (9, H))
+    take("lin2.bias", (9,))
+    if off != packed.numel():
+        raise ValueError(f"packed weights have {packed.numel()} floats, the stack spec needs {off}")
+    return out
+
+
+def dqn_grad_stack(cfg: SwarmConfig, spec, online: torch.Tensor, target: torch.Tensor, batch: ReplayRing,
+                   indices: Optional[torch.Tensor], n_graphs: int, gamma: float = 0.99, loss_scale: Optional[float] = None,
+                   want_td: bool = False, grad: Optional[torch.Tensor] = None, loss: Optional[torch.Tensor] = None
+                   ) -> Tuple[torch.Tensor, torch.Tensor, Optional[torch.Tensor]]:
+    """train_step_dqn's loss + gradient (train:116-124) for a stacked network over n_graphs transitions of ``batch``
+    (slots ``indices`` if given), in one gradient launch + one reduce launch.  Returns (grad f32[count] in packed stack
+    order, loss f32[1], td f32[G,N] or None)."""
+    N, dev = cfg.n_agents, online.device
+    count = int(lib().swarm_stack_weight_count(C.byref(spec)))
+    _expect(online, torch.float32, count, "online weights")
+    _expect(target, torch.float32, count, "target weights")
+    if indices is not None:
+        if indices.dtype != torch.int64 or indices.numel() != n_graphs:
+            raise TypeError("indices must be int64[n_graphs]")
+    if loss_scale is None:
+        loss_scale = 1.0 / (n_graphs * N)
+    grad = grad if grad is not None else torch.empty(count, dtype=torch.float32, device=dev)
+    loss = loss if loss is not None else torch.empty(1, dtype=torch.float32, device=dev)
+    _expect(grad, torch.float32, count, "grad")
+    td = torch.empty(n_graphs, N, dtype=torch.float32, device=dev) if want_td else None
+    wb = int(lib().swarm_dqn_stack_workspace_bytes(C.byref(cfg), C.byref(spec), n_graphs))
+    ws = torch.empty(max(wb, 1), dtype=torch.uint8, device=dev)
+    rs = batch.struct()
+    check(lib().swarm_dqn_stack_grad(C.byref(cfg), C.byref(spec), ptr(online), ptr(target), C.byref(rs), ptr(indices),
+                                     n_graphs, float(gamma), float(loss_scale), ptr(grad), ptr(loss), ptr(td), ptr(ws), wb,
+                                     stream_ptr(dev)))
+    return grad, loss, td
+
+
+def adam_clip_step_stack(spec, weights: torch.Tensor, grad: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor,
+                         step: int, lr: float = 1e-3, betas: Tuple[float, float] = (0.9, 0.999), eps: float = 1e-8,
+                         max_norm: float = 1.0, target: Optional[torch.Tensor] = None,
+                         grad_norm: Optional[torch.Tensor] = None) -> None:
+    """clip_grad_norm_(max_norm) + torch.optim.Adam step on a stack's packed weights, in place (train:125-126);
+    optionally copies the new weights into ``target`` (train:131-133) and the pre-clip norm into ``grad_norm``."""
+    count = int(lib().swarm_stack_weight_count(C.byref(spec)))
+    for name, t in (("weights", weights), ("grad", grad), ("exp_avg", exp_avg), ("exp_avg_sq", exp_avg_sq)):
+        _expect(t, torch.float32, count, name)
+    if target is not None:
+        _expect(target, torch.float32, count, "target")
+    check(lib().swarm_adam_clip_stack_step(C.byref(spec), ptr(weights), ptr(grad), ptr(exp_avg), ptr(exp_avg_sq), int(step),
+                                           float(lr), float(betas[0]), float(betas[1]), float(eps), float(max_norm),
+                                           ptr(target), ptr(grad_norm), stream_ptr(weights.device)))
+
+
 def gatstack_forward(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Tensor, want_q: bool = True,
                      want_actions: bool = False):
     """A whole multi-layer GAT Q-network forward on the per-env graph in one launch: q f32[B,N,9], actions int32[B,N]."""

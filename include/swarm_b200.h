@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SWARM_ABI_VERSION 4
+#define SWARM_ABI_VERSION 5
 
 enum { SWARM_SCENARIO_GOTO = 0, SWARM_SCENARIO_OBSTACLE_AVOIDANCE = 1 };
 /* SWARM_GRAPH_RADIUS is an EXTENSION (the reference has no radius graph, SURVEY.md Appendix C): the complete-graph
@@ -519,6 +519,33 @@ int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg);
 int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
                         int32_t ticks, const SwarmRewardSpec* reward, float* shaping, float* returns, int32_t* hits,
                         void* workspace, int64_t workspace_bytes, void* stream);
+
+/* One DQN loss + gradient of a stacked network (train_step_dqn, train_gcn_dqn.py:116-124, for the conv1 .. convL form):
+ * the contract of swarm_dqn_grad for the network described by `spec`.  Transitions come from `batch` (slot g, or slot
+ * indices[g] when indices != NULL); values = Q_online(s)[a], targets = r + gamma * max_a Q_target(s') (no terminal
+ * mask), loss = loss_scale * sum over the n_graphs*N nodes of (values - targets)^2 (loss_scale = 1 / (n_graphs*N) gives
+ * nn.MSELoss).  Each graph is built per env from cfg->graph_mode, on s for the online network and on s' for the target;
+ * node features as swarm_gatstack_forward, whose Q values the kernel reproduces bit for bit.  Hand-written backward
+ * pass through the layer stack; per-CTA partial sums reduced in a fixed order, no atomics (bit-reproducible).
+ * cfg->num_envs is ignored; 2 <= n_agents <= 128, graphs and spec as for swarm_gatstack_forward.  Outputs:
+ * grad float[swarm_stack_weight_count(spec)] (packed stack order), loss float[1] (both overwritten); td (optional)
+ * float[n_graphs*N] = values - targets, formed with separately rounded ops (gamma * next, + r, values -).
+ * workspace: swarm_dqn_stack_workspace_bytes(cfg, spec, n_graphs) bytes (0 for arguments the call would reject). */
+int64_t swarm_dqn_stack_workspace_bytes(const SwarmConfig* cfg, const SwarmStackSpec* spec, int32_t n_graphs);
+int swarm_dqn_stack_grad(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* online_weights,
+                         const float* target_weights, const SwarmReplay* batch, const int64_t* indices, int32_t n_graphs,
+                         float gamma, float loss_scale, float* grad, float* loss, float* td, void* workspace,
+                         int64_t workspace_bytes, void* stream);
+
+/* clip_grad_norm_(model.parameters(), max_norm) + one torch.optim.Adam step (train:125-126) on the packed weights of a
+ * stack, in place: swarm_adam_clip_step for swarm_stack_weight_count(spec) floats.  The per-tensor 2-norms are taken over
+ * the state-dict tensors in packed order (per layer att_src, att_dst, bias, lin.weight; then lin1.weight, lin1.bias,
+ * lin2.weight, lin2.bias -- the order of StackedGCN.parameters()), then the 2-norm of those; clip coefficient
+ * max_norm / (norm + 1e-6), clamped to 1; max_norm <= 0 disables clipping.  `step` is the 1-based step count;
+ * target_weights (optional) receives a copy of the updated weights, grad_norm (optional) float[1] the pre-clip norm. */
+int swarm_adam_clip_stack_step(const SwarmStackSpec* spec, float* weights, const float* grad, float* exp_avg,
+                               float* exp_avg_sq, int64_t step, double lr, double beta1, double beta2, double eps,
+                               double max_norm, float* target_weights, float* grad_norm, void* stream);
 
 #ifdef __cplusplus
 }
