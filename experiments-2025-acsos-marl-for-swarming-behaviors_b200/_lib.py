@@ -22,7 +22,7 @@ FLAG_OBSTACLE_CONTACT = 1
 FLAG_HIT = 2
 FLAG_PENALTY = 4
 W_COUNT = 1673
-ABI_VERSION = 5
+ABI_VERSION = 6
 XCHG_STRIDE = 1680
 
 # state-dict tensors in packed order (include/swarm_b200.h SWARM_W_*)
@@ -121,6 +121,9 @@ _SIGNATURES = {
     "swarm_graph_build_radius": (C.c_int, [C.POINTER(SwarmConfig)] + [C.c_void_p] * 4),
     "swarm_stack_weight_count": (C.c_int64, [C.POINTER(SwarmStackSpec)]),
     "swarm_gatstack_forward": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec)] + [C.c_void_p] * 5),
+    "swarm_gatstack_large_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec)]),
+    "swarm_gatstack_forward_large": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec)] + [C.c_void_p] * 6
+                                     + [C.c_int64, C.c_void_p]),
     "swarm_rollout_stack_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig)]),
     "swarm_rollout_stack": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p, C.c_int32,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),

@@ -37,6 +37,11 @@ cudaError_t launch_gatstack_forward(const SwarmConfig& c, const SwarmStackSpec& 
 cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
                                     int ticks, const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
                                     float* returns, int32_t* hits, cudaStream_t stream);
+int stack_large_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
+long long stack_large_workspace_bytes(const SwarmConfig& c, int hp);
+long long stack_large_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
+cudaError_t launch_gatstack_large(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, const float* state,
+                                  const int32_t* nbr, float* q, int32_t* actions, void* workspace, cudaStream_t stream);
 int stack_grad_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
 long long stack_grad_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s, int n_graphs);
 cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, const float* w_online, const float* w_target,
@@ -807,8 +812,10 @@ int swarm_scenario_reward(const SwarmRewardSpec* spec, const float* state, float
 }
 
 namespace {
-int validate_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec) {
-  if (int rc = validate(cfg, true)) return rc;
+// large = false: the env-tile kernels (n_agents <= 128, kNN n_agents <= 16); large = true: the one-CTA-per-env kernel
+// (any n_agents <= 4096; above 128 agents the kNN table comes from the partial_sort branch of swarm_graph_build)
+int validate_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, bool large = false) {
+  if (int rc = validate(cfg, true, large)) return rc;
   if (!spec) return fail(SWARM_ERR_INVALID_ARG, "spec is NULL");
   if (spec->n_layers < 1 || spec->n_layers > 4) return fail(SWARM_ERR_INVALID_ARG, "n_layers must be 1 .. 4");
   if (spec->hidden < 1 || spec->hidden > 32) return fail(SWARM_ERR_UNSUPPORTED, "hidden must be 1 .. 32");
@@ -816,8 +823,13 @@ int validate_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec) {
   for (int l = 0; l < spec->n_layers; ++l)
     if (spec->activation[l] != SWARM_ACT_TANH && spec->activation[l] != SWARM_ACT_RELU)
       return fail(SWARM_ERR_INVALID_ARG, "unknown activation");
-  if (cfg->graph_mode == SWARM_GRAPH_KNN && cfg->n_agents > 16)
+  if (!large && cfg->graph_mode == SWARM_GRAPH_KNN && cfg->n_agents > 16)
     return fail(SWARM_ERR_UNSUPPORTED, "stacked networks on the kNN graph are implemented for n_agents <= 16");
+  if (large && cfg->graph_mode == SWARM_GRAPH_KNN && cfg->n_agents > kTileThreads &&
+      (int64_t)cfg->knn_k * 64 > cfg->n_agents)
+    return fail(SWARM_ERR_UNSUPPORTED, "large-swarm kNN implements torch.topk's partial_sort branch (64 k <= n_agents)");
+  if (large && stack_large_smem_bytes(*cfg, *spec) > 227 * 1024)
+    return fail(SWARM_ERR_UNSUPPORTED, "the large stacked forward needs more than 227 KB of shared memory for this (N, spec)");
   return SWARM_OK;
 }
 }  // namespace
@@ -836,6 +848,25 @@ int swarm_gatstack_forward(const SwarmConfig* cfg, const SwarmStackSpec* spec, c
                     "swarm_gatstack_forward");
 }
 
+int64_t swarm_gatstack_large_workspace_bytes(const SwarmConfig* cfg, const SwarmStackSpec* spec) {
+  if (validate_stack(cfg, spec, true) != SWARM_OK) return 0;
+  return stack_large_workspace_bytes(*cfg, *spec);
+}
+
+int swarm_gatstack_forward_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights,
+                                 const float* state, const int32_t* neighbours, float* q, int32_t* actions,
+                                 void* workspace, int64_t workspace_bytes, void* stream) {
+  if (int rc = validate_stack(cfg, spec, true)) return rc;
+  if (!weights || !state || !workspace) return fail(SWARM_ERR_INVALID_ARG, "weights/state/workspace is NULL");
+  if (cfg->graph_mode == SWARM_GRAPH_KNN && !neighbours)
+    return fail(SWARM_ERR_INVALID_ARG, "the kNN graph needs the topk table (neighbours, swarm_graph_build)");
+  if (!q && !actions) return fail(SWARM_ERR_INVALID_ARG, "no output requested");
+  if (workspace_bytes < stack_large_workspace_bytes(*cfg, *spec)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  return check_cuda(launch_gatstack_large(*cfg, *spec, weights, state, neighbours, q, actions, workspace,
+                                          (cudaStream_t)stream),
+                    "swarm_gatstack_forward_large");
+}
+
 namespace {
 int validate_spec(const SwarmStackSpec* spec) {
   if (!spec) return fail(SWARM_ERR_INVALID_ARG, "spec is NULL");
@@ -849,6 +880,8 @@ int validate_spec(const SwarmStackSpec* spec) {
 int validate_dqn_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, int32_t n_graphs) {
   if (!cfg) return fail(SWARM_ERR_INVALID_ARG, "cfg is NULL");
   if (n_graphs <= 0) return fail(SWARM_ERR_INVALID_ARG, "n_graphs must be positive");
+  if (cfg->n_agents > kTileThreads)
+    return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN update is implemented for n_agents <= 128");
   SwarmConfig c = *cfg;
   c.num_envs = n_graphs;
   if (int rc = validate_stack(&c, spec)) return rc;
@@ -895,16 +928,51 @@ int swarm_adam_clip_stack_step(const SwarmStackSpec* spec, float* weights, const
 int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg) {
   if (!cfg || cfg->num_envs <= 0 || cfg->n_agents <= 0) return 0;
   const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
+  if (cfg->n_agents > kTileThreads) {
+    // actions, topk table (kNN), then the large forward's workspace at the widest layer (hidden 32)
+    const int64_t k = cfg->graph_mode == SWARM_GRAPH_KNN ? (cfg->knn_k > 0 ? cfg->knn_k : 0) : 0;
+    return 256 + ((bn * 4 + bn * k * 4 + 255) & ~(int64_t)255) + stack_large_workspace_bytes(*cfg, 32);
+  }
   return bn * 4 + bn * 4 + bn + 1024;             // actions, rewards, flags
+}
+
+// n_agents > 128: per tick [topk table ->] the large stacked forward (argmax) -> the large world step with returns / hits
+static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
+                               int32_t ticks, float* returns, int32_t* hits, void* workspace, cudaStream_t st) {
+  const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
+  const bool knn = cfg->graph_mode == SWARM_GRAPH_KNN;
+  uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
+  int32_t* actions = reinterpret_cast<int32_t*>(base);
+  int32_t* nbr = actions + bn;
+  void* fwd_ws = reinterpret_cast<void*>(base + ((bn * 4 + (knn ? bn * cfg->knn_k * 4 : 0) + 255) & ~(int64_t)255));
+  // in place: one CTA owns a whole env and stages its positions first
+  SimStepArgs p = step_args(*cfg, state, actions, state);
+  p.returns = returns;
+  p.hits = hits;
+  for (int t = 0; t < ticks; ++t) {
+    if (knn)
+      if (cudaError_t e = launch_graph_large(*cfg, state, nullptr, nbr, (int)swarm_edges_per_env(cfg), st); e != cudaSuccess)
+        return check_cuda(e, "swarm_rollout_stack (graph)");
+    if (cudaError_t e = launch_gatstack_large(*cfg, *spec, weights, state, knn ? nbr : nullptr, nullptr, actions, fwd_ws, st);
+        e != cudaSuccess)
+      return check_cuda(e, "swarm_rollout_stack (forward)");
+    if (cudaError_t e = launch_sim_step_large(p, st); e != cudaSuccess) return check_cuda(e, "swarm_rollout_stack (step)");
+  }
+  return SWARM_OK;
 }
 
 int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
                         int32_t ticks, const SwarmRewardSpec* reward, float* shaping, float* returns, int32_t* hits,
                         void* workspace, int64_t workspace_bytes, void* stream) {
-  if (int rc = validate_stack(cfg, spec)) return rc;
+  if (int rc = validate_stack(cfg, spec, cfg && cfg->n_agents > kTileThreads)) return rc;
+  const bool large = cfg->n_agents > kTileThreads;
+  if (large && reward)
+    return fail(SWARM_ERR_UNSUPPORTED, "the Flocking / Cohesion rewards are implemented for n_agents <= 128 "
+                                       "(larger swarms: reward = NULL, the world's own reward)");
   if (!weights || !state || !workspace) return fail(SWARM_ERR_INVALID_ARG, "weights/state/workspace is NULL");
   if (ticks < 0) return fail(SWARM_ERR_INVALID_ARG, "ticks must be >= 0");
   if (workspace_bytes < swarm_rollout_stack_workspace_bytes(cfg)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  if (large) return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, workspace, (cudaStream_t)stream);
   SwarmRewardSpec rs;
   if (reward) {
     rs = *reward;

@@ -657,17 +657,49 @@ def adam_clip_step_stack(spec, weights: torch.Tensor, grad: torch.Tensor, exp_av
 
 def gatstack_forward(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Tensor, want_q: bool = True,
                      want_actions: bool = False):
-    """A whole multi-layer GAT Q-network forward on the per-env graph in one launch: q f32[B,N,9], actions int32[B,N]."""
+    """A whole multi-layer GAT Q-network forward on the per-env graph in one launch: q f32[B,N,9], actions int32[B,N].
+    Above 128 agents it runs ``gatstack_forward_large`` (kNN: after the topk table of ``graph_build``)."""
     B, N = cfg.num_envs, cfg.n_agents
     _expect(state, torch.float32, B * N * 4, "state")
     _expect(weights, torch.float32, int(lib().swarm_stack_weight_count(C.byref(spec))), "weights")
     dev = state.device
     q = torch.empty(B, N, 9, dtype=torch.float32, device=dev) if want_q else None
     act = torch.empty(B, N, dtype=torch.int32, device=dev) if want_actions else None
-    check(lib().swarm_gatstack_forward(C.byref(cfg), C.byref(spec), ptr(weights), ptr(state), ptr(q), ptr(act), stream_ptr(dev)))
+    if N > 128:
+        gatstack_forward_large(cfg, spec, weights, state, q=q, actions=act)
+    else:
+        check(lib().swarm_gatstack_forward(C.byref(cfg), C.byref(spec), ptr(weights), ptr(state), ptr(q), ptr(act),
+                                           stream_ptr(dev)))
     if want_q and want_actions:
         return q, act
     return q if want_q else act
+
+
+def gatstack_forward_large(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Tensor,
+                           neighbours: Optional[torch.Tensor] = None, q: Optional[torch.Tensor] = None,
+                           actions: Optional[torch.Tensor] = None) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """The stacked forward of ``swarm_gatstack_forward_large`` (one CTA per env, any N <= 4096) into the given ``q``
+    f32[B,N,9] / ``actions`` int32[B,N]; on the kNN graph ``neighbours`` is the topk table int32[B,N,k] of
+    ``swarm_graph_build`` (as ``graph_build(..., want_neighbours=True)`` returns it), built here when not given."""
+    B, N = cfg.num_envs, cfg.n_agents
+    _expect(state, torch.float32, B * N * 4, "state")
+    _expect(weights, torch.float32, int(lib().swarm_stack_weight_count(C.byref(spec))), "weights")
+    if q is not None:
+        _expect(q, torch.float32, B * N * 9, "q")
+    if actions is not None:
+        _expect(actions, torch.int32, B * N, "actions")
+    dev = state.device
+    if cfg.graph_mode == _lib.GRAPH_KNN:
+        if neighbours is None:
+            # the topk table alone (swarm_graph_build without the edge list)
+            neighbours = torch.empty(B, N, cfg.knn_k, dtype=torch.int32, device=dev)
+            check(lib().swarm_graph_build(C.byref(cfg), ptr(state), None, ptr(neighbours), stream_ptr(dev)))
+        _expect(neighbours, torch.int32, B * N * cfg.knn_k, "neighbours")
+    wb = int(lib().swarm_gatstack_large_workspace_bytes(C.byref(cfg), C.byref(spec)))
+    ws = torch.empty(max(wb, 1), dtype=torch.uint8, device=dev)
+    check(lib().swarm_gatstack_forward_large(C.byref(cfg), C.byref(spec), ptr(weights), ptr(state), ptr(neighbours), ptr(q),
+                                             ptr(actions), ptr(ws), wb, stream_ptr(dev)))
+    return q, actions
 
 
 def rollout_stack(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Tensor, ticks: int,

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SWARM_ABI_VERSION 5
+#define SWARM_ABI_VERSION 6
 
 enum { SWARM_SCENARIO_GOTO = 0, SWARM_SCENARIO_OBSTACLE_AVOIDANCE = 1 };
 /* SWARM_GRAPH_RADIUS is an EXTENSION (the reference has no radius graph, SURVEY.md Appendix C): the complete-graph
@@ -501,10 +501,24 @@ typedef struct SwarmStackSpec {
 int64_t swarm_stack_weight_count(const SwarmStackSpec* spec);
 
 /* The whole forward of a stack on the per-env graph named by cfg->graph_mode (complete; radius; kNN for n_agents <= 16)
- * in ONE launch: in-edge lists built once in shared memory, layer outputs never leave the chip.  n_agents <= 128.
- * q float[B*N][9] and actions int32[B*N] (argmax, first maximum wins) are optional. */
+ * in ONE launch: in-edge lists built once in shared memory, layer outputs never leave the chip.  n_agents <= 128
+ * (larger swarms: swarm_gatstack_forward_large).  q float[B*N][9] and actions int32[B*N] (argmax, first maximum wins)
+ * are optional. */
 int swarm_gatstack_forward(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, const float* state,
                            float* q, int32_t* actions, void* stream);
+
+/* The same forward for large swarms, ONE launch with one CTA per env: any spec, 1 <= n_agents <= 4096, on the radius
+ * and complete graphs and on the kNN graph from the caller's topk table (neighbours int32[B][N][k] of swarm_graph_build;
+ * above 128 agents 64 k <= n_agents, its partial_sort branch).  The attention runs in input space per layer
+ * (sum alpha h_src = W sum alpha x_src, <h, att> = <x, W^T att>): float32-level different rounding from
+ * swarm_gatstack_forward.  The complete graph costs O(N log N) per layer (sources sorted by alpha_src, prefix / suffix
+ * scans).  The layer rows live in the workspace (double-buffered, [2][B][N][8 | 16 | 32] floats).  q / actions as
+ * swarm_gatstack_forward.  workspace: swarm_gatstack_large_workspace_bytes(cfg, spec) bytes (0 for rejected
+ * arguments). */
+int64_t swarm_gatstack_large_workspace_bytes(const SwarmConfig* cfg, const SwarmStackSpec* spec);
+int swarm_gatstack_forward_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights,
+                                 const float* state, const int32_t* neighbours, float* q, int32_t* actions,
+                                 void* workspace, int64_t workspace_bytes, void* stream);
 
 /* `ticks` greedy evaluation ticks (simulator.py:59-93) of a stacked network, launched back to back from the library:
  * per tick swarm_gatstack_forward (argmax) -> swarm_sim_step in place -> the tick's reward -> returns float[B*N] (+=),
@@ -513,8 +527,10 @@ int swarm_gatstack_forward(const SwarmConfig* cfg, const SwarmStackSpec* spec, c
  * of swarm_scenario_reward) or Cohesion's per-agent reward on the GoTo world, evaluated by the swarm_scenario_reward
  * arithmetic after every step.  The whole loop is ONE launch (state, running return and Flocking memory in registers
  * across the ticks, same tick as swarm_rollout); SWARM_STACK_FUSED=0 launches forward, world step, reward kernel and
- * totals per tick instead (same results, bit for bit).  No host work or allocation inside (graph capturable).
- * workspace: swarm_rollout_stack_workspace_bytes(cfg). */
+ * totals per tick instead (same results, bit for bit).  n_agents > 128 (up to 4096): per tick [kNN: the topk table of
+ * swarm_graph_build ->] swarm_gatstack_forward_large (argmax) -> swarm_sim_step in place, returns / hits accumulated by
+ * the world step; reward must be NULL there (the Flocking / Cohesion rewards are implemented for n_agents <= 128).
+ * No host work or allocation inside (graph capturable).  workspace: swarm_rollout_stack_workspace_bytes(cfg). */
 int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg);
 int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
                         int32_t ticks, const SwarmRewardSpec* reward, float* shaping, float* returns, int32_t* hits,
