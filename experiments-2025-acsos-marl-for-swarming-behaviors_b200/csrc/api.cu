@@ -50,8 +50,6 @@ cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, 
 cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const float* grad, float* m, float* v,
                                    long long step, double lr, double beta1, double beta2, double eps, double max_norm,
                                    float* target, float* grad_norm, cudaStream_t stream);
-cudaError_t launch_stack_accumulate(long long total, int N, const float* rewards, int per_env, const uint8_t* flags,
-                                    float* returns, int32_t* hits, cudaStream_t stream);
 bool gatq_knn_large_fits(int N, int K);
 bool gatq_large_x_fits(int N, bool radius);
 cudaError_t launch_gatq_large_x(const SwarmConfig& c, const float* weights, const float* state, float* q, int32_t* actions,
@@ -933,7 +931,8 @@ int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg) {
     const int64_t k = cfg->graph_mode == SWARM_GRAPH_KNN ? (cfg->knn_k > 0 ? cfg->knn_k : 0) : 0;
     return 256 + ((bn * 4 + bn * k * 4 + 255) & ~(int64_t)255) + stack_large_workspace_bytes(*cfg, 32);
   }
-  return bn * 4 + bn * 4 + bn + 1024;             // actions, rewards, flags
+  // the n_agents <= 128 rollout is one launch that does not touch the workspace; this size is kept as the ABI states it
+  return bn * 4 + bn * 4 + bn + 1024;
 }
 
 // n_agents > 128: per tick [topk table ->] the large stacked forward (argmax) -> the large world step with returns / hits
@@ -988,38 +987,10 @@ int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, cons
     rs.reset = 0;
     rs.env_index = -1;
   }
-  const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
-  uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
-  int32_t* actions = reinterpret_cast<int32_t*>(base);
-  float* rewards = reinterpret_cast<float*>(actions + bn);
-  uint8_t* flags = reinterpret_cast<uint8_t*>(rewards + bn);
-  cudaStream_t st = (cudaStream_t)stream;
-  // the whole loop is ONE launch with the state in registers (stack_kernels.cu gatstack_kernel<HP, true>);
-  // SWARM_STACK_FUSED=0 takes the launch sequence below (forward, step, reward kernel, totals per tick)
-  const char* fused_env = std::getenv("SWARM_STACK_FUSED");
-  if (!(fused_env && fused_env[0] == '0'))
-    return check_cuda(launch_gatstack_rollout(*cfg, *spec, weights, state, ticks, world_consts(*cfg), reward ? &rs : nullptr,
-                                              shaping, returns, hits, st),
-                      "swarm_rollout_stack");
-  SimStepArgs p = step_args(*cfg, state, actions, state);
-  p.rewards = rewards;
-  p.flags = flags;
-  for (int t = 0; t < ticks; ++t) {
-    if (cudaError_t e = launch_gatstack_forward(*cfg, *spec, weights, state, nullptr, actions, st); e != cudaSuccess)
-      return check_cuda(e, "swarm_rollout_stack (forward)");
-    if (cudaError_t e = launch_sim_step(p, st); e != cudaSuccess) return check_cuda(e, "swarm_rollout_stack (step)");
-    int per_env = 0;
-    if (reward) {
-      per_env = rs.kind == SWARM_REWARD_FLOCKING ? 1 : 0;
-      if (cudaError_t e2 = launch_scenario_reward(rs, state, shaping, rewards, nullptr, st); e2 != cudaSuccess)
-        return check_cuda(e2, "swarm_rollout_stack (reward)");
-    }
-    if (returns || hits)
-      if (cudaError_t e3 = launch_stack_accumulate(bn, cfg->n_agents, rewards, per_env, flags, returns, hits, st);
-          e3 != cudaSuccess)
-        return check_cuda(e3, "swarm_rollout_stack (accumulate)");
-  }
-  return SWARM_OK;
+  // the whole loop is ONE launch with the state in registers (stack_kernels.cu gatstack_kernel<HP, true>)
+  return check_cuda(launch_gatstack_rollout(*cfg, *spec, weights, state, ticks, world_consts(*cfg), reward ? &rs : nullptr,
+                                            shaping, returns, hits, (cudaStream_t)stream),
+                    "swarm_rollout_stack");
 }
 
 int swarm_episode_end(const SwarmConfig* cfg, SwarmTrainCtl* ctl, float* returns, int32_t* hits, const float* loss,

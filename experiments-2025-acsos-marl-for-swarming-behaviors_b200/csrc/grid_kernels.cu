@@ -11,9 +11,10 @@
 //                         filtered by distance) as a compact CSR grouped by target -- in-degrees, then sources in
 //                         ascending order through a 9-way merge of the cell lists, which is exactly the order the edge
 //                         list -> stable sort by target gives; feeds swarm_gatq_forward_csr (bit-faithful forward)
-//   gatq_large_x_kernel   GCN.forward (train_gcn_dqn.py:59-70) + argmax for a large env on the radius or the complete
-//                         graph with the attention in input space (see large_kernels.cu gatq_knn_large_x_kernel): no
-//                         edge list at all -- the complete graph of 1 024 agents would be 1.07e9 edges per tick at C4.
+//   gatq_large_x_kernel   GCN.forward (train_gcn_dqn.py:59-70) + argmax for a large env on the radius graph with the
+//                         attention in input space (see large_kernels.cu gatq_knn_large_x_kernel): no edge list at all
+//   gatq_large_sorted_kernel  the same on the complete graph in O(N log N) -- the complete graph of 1 024 agents would
+//                         be 1.07e9 edges per tick at C4.
 #include <cstdlib>
 
 #include "gatq_device.cuh"
@@ -250,20 +251,19 @@ struct LargeXParams {
   float qmax_r;
 };
 
-__host__ __device__ inline size_t large_x_smem_bytes(int N, bool radius) {
+__host__ __device__ inline size_t large_x_smem_bytes(int N) {
   size_t b = (size_t)((TW_COUNT + 3) & ~3) * 4 + 64;        // weights, v_s / v_d
   b += (size_t)N * 16 + (size_t)N * 4;                       // states, alpha_src
   b += 64 * 4;                                               // reduction scratch
-  if (radius) b += (size_t)grid_pow2(N) * 4 + (size_t)kGridCells * 4;
+  b += (size_t)grid_pow2(N) * 4 + (size_t)kGridCells * 4;    // grid keys, cell ranges
   return b + 64;
 }
 
-template <bool RADIUS>
 __global__ void __launch_bounds__(kGridThreads, 2) gatq_large_x_kernel(const __grid_constant__ LargeXParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const SwarmConfig& c = p.cfg;
   const int N = c.n_agents, P = grid_pow2(N);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   const long long env = blockIdx.x;
   float* sw = reinterpret_cast<float*>(smem_raw);
   float* sv = sw + ((TW_COUNT + 3) & ~3);                 // v_s[8], v_d[8]
@@ -286,53 +286,37 @@ __global__ void __launch_bounds__(kGridThreads, 2) gatq_large_x_kernel(const __g
       for (int cc = 0; cc < 32; ++cc) v = fmaf(att[cc], sw[TW_W0T + k * 32 + cc], v);
     sv[tid] = v;
   }
-  CellGrid g;
-  if (RADIUS)
-    g = grid_build([&](int j) { const float4 s = sst[j]; return make_float2(s.x, s.y); }, N, P, c.graph_radius, keys, cbeg,
-                   cend, sred);
+  const CellGrid g = grid_build([&](int j) { const float4 s = sst[j]; return make_float2(s.x, s.y); }, N, P,
+                                c.graph_radius, keys, cbeg, cend, sred);
   __syncthreads();
-  // alpha_src of every node; for the complete graph also the two largest of the env (the softmax shift of node i is the
-  // largest alpha_src among its sources: everybody but itself)
-  float t1 = -INFINITY, t2 = -INFINITY;
-  int t1i = -1;
   for (int i = tid; i < N; i += kGridThreads) {
     const float4 st = sst[i];
-    const float a = fmaf(st.x, sv[0], fmaf(st.y, sv[1], fmaf(st.z, sv[2], fmaf(st.w, sv[3],
-                    fmaf(c.goal_x, sv[4], fmaf(c.goal_y, sv[5], (float)i * sv[6]))))));
-    sas[i] = a;
-    if (a > t1) { t2 = t1; t1 = a; t1i = i; }
-    else if (a > t2) t2 = a;
+    sas[i] = fmaf(st.x, sv[0], fmaf(st.y, sv[1], fmaf(st.z, sv[2], fmaf(st.w, sv[3],
+             fmaf(c.goal_x, sv[4], fmaf(c.goal_y, sv[5], (float)i * sv[6]))))));
   }
-  if (!RADIUS) {
-    auto merge = [&](float o1, int oi, float o2) {
-      if (o1 > t1) { t2 = fmaxf(t1, o2); t1 = o1; t1i = oi; }
-      else t2 = fmaxf(t2, o1);
-    };
-#pragma unroll
-    for (int sh = 16; sh > 0; sh >>= 1) {
-      const float o1 = __shfl_xor_sync(0xffffffffu, t1, sh), o2 = __shfl_xor_sync(0xffffffffu, t2, sh);
-      const int oi = __shfl_xor_sync(0xffffffffu, t1i, sh);
-      merge(o1, oi, o2);
-    }
-    if (lane == 0) {
-      sred[warp * 3 + 0] = t1;
-      sred[warp * 3 + 1] = __int_as_float(t1i);
-      sred[warp * 3 + 2] = t2;
-    }
-    __syncthreads();
-    t1 = -INFINITY; t2 = -INFINITY; t1i = -1;
-    for (int w = 0; w < kGridThreads / 32; ++w) merge(sred[w * 3 + 0], __float_as_int(sred[w * 3 + 1]), sred[w * 3 + 2]);
-  } else {
-    __syncthreads();
-  }
+  __syncthreads();
 
   for (int i = tid; i < N; i += kGridThreads) {
     const float4 st = sst[i];
     const float adst = fmaf(st.x, sv[8], fmaf(st.y, sv[9], fmaf(st.z, sv[10], fmaf(st.w, sv[11],
                        fmaf(c.goal_x, sv[12], fmaf(c.goal_y, sv[13], (float)i * sv[14]))))));
+    // in-edges: agents j != i within the radius (train:94-110 filtered by distance) + the trailing (0,0) of node 0
+    const float2 neg = make_float2(-st.x, -st.y);
+    const int cx = g.cx(st.x), cy = g.cy(st.y);
+    const int y0 = max(cy - 1, 0), y1 = min(cy + 1, g.ny - 1), x0 = max(cx - 1, 0), x1 = min(cx + 1, g.nx - 1);
+    float amax = (i == 0) ? sas[0] : -INFINITY;
+    for (int yy = y0; yy <= y1; ++yy)
+      for (int xx = x0; xx <= x1; ++xx) {
+        const int cc = yy * g.nx + xx;
+        for (int q = cbeg[cc], e = cend[cc]; q < e; ++q) {
+          const int j = (int)(keys[q] & kIdxMask);
+          const float4 sj = sst[j];
+          if (j != i && grid_hit(make_float2(sj.x, sj.y), neg, p.qmax_r)) amax = fmaxf(amax, sas[j]);
+        }
+      }
+    const float m = gat_logit(amax, adst);                // LeakyReLU and the rounded add are monotone
     float den = 0.0f, acc_id = 0.0f;
     float2 acc_p = make_float2(0.f, 0.f), acc_v = make_float2(0.f, 0.f);
-    float m;
     auto add = [&](int j) {
       const float4 sj = sst[j];
       const float w = __expf(gat_logit(sas[j], adst) - m);
@@ -341,42 +325,16 @@ __global__ void __launch_bounds__(kGridThreads, 2) gatq_large_x_kernel(const __g
       acc_v = __ffma2_rn(make_float2(w, w), make_float2(sj.z, sj.w), acc_v);
       acc_id = fmaf(w, (float)j, acc_id);
     };
-    if (RADIUS) {
-      // in-edges: agents j != i within the radius (train:94-110 filtered by distance) + the trailing (0,0) of node 0
-      const float2 neg = make_float2(-st.x, -st.y);
-      const int cx = g.cx(st.x), cy = g.cy(st.y);
-      const int y0 = max(cy - 1, 0), y1 = min(cy + 1, g.ny - 1), x0 = max(cx - 1, 0), x1 = min(cx + 1, g.nx - 1);
-      float amax = (i == 0) ? sas[0] : -INFINITY;
-      for (int yy = y0; yy <= y1; ++yy)
-        for (int xx = x0; xx <= x1; ++xx) {
-          const int cc = yy * g.nx + xx;
-          for (int q = cbeg[cc], e = cend[cc]; q < e; ++q) {
-            const int j = (int)(keys[q] & kIdxMask);
-            const float4 sj = sst[j];
-            if (j != i && grid_hit(make_float2(sj.x, sj.y), neg, p.qmax_r)) amax = fmaxf(amax, sas[j]);
-          }
+    for (int yy = y0; yy <= y1; ++yy)
+      for (int xx = x0; xx <= x1; ++xx) {
+        const int cc = yy * g.nx + xx;
+        for (int q = cbeg[cc], e = cend[cc]; q < e; ++q) {
+          const int j = (int)(keys[q] & kIdxMask);
+          const float4 sj = sst[j];
+          if (j != i && grid_hit(make_float2(sj.x, sj.y), neg, p.qmax_r)) add(j);
         }
-      m = gat_logit(amax, adst);                          // LeakyReLU and the rounded add are monotone
-      for (int yy = y0; yy <= y1; ++yy)
-        for (int xx = x0; xx <= x1; ++xx) {
-          const int cc = yy * g.nx + xx;
-          for (int q = cbeg[cc], e = cend[cc]; q < e; ++q) {
-            const int j = (int)(keys[q] & kIdxMask);
-            const float4 sj = sst[j];
-            if (j != i && grid_hit(make_float2(sj.x, sj.y), neg, p.qmax_r)) add(j);
-          }
-        }
-      if (i == 0) add(0);
-    } else {
-      // complete graph (train:94-110): every j != i, node 0 additionally its (0,0)
-      const float amax = (i == 0 || t1i != i) ? t1 : t2;
-      m = gat_logit(amax, adst);
-#pragma unroll 4
-      for (int j = 0; j < i; ++j) add(j);
-#pragma unroll 4
-      for (int j = i + 1; j < N; ++j) add(j);
-      if (i == 0) add(0);
-    }
+      }
+    if (i == 0) add(0);
     const float inv = 1.0f / __fadd_rn(den, 1e-16f);
     const float wsum = den * inv;
     const float xm[7] = {acc_p.x * inv, acc_p.y * inv, acc_v.x * inv, acc_v.y * inv, c.goal_x * wsum, c.goal_y * wsum,
@@ -416,7 +374,8 @@ __global__ void __launch_bounds__(kGridThreads, 2) gatq_large_x_kernel(const __g
 // added is positive and the two factors are <= 1 (m_i = LeakyReLU(A + d_i) is the row's largest logit), so there is no
 // overflow and no cancellation -- except for the ONE node that holds A itself (its row's largest logit comes from the
 // second largest a): that node sums its row directly.  1 M pair evaluations per env at N = 1 024 become ~20 k operations.
-// Same mathematics as gatq_large_x_kernel<false>, float32-level different rounding (tests: Q within 1e-5).
+// Same mathematics as the bit-faithful CSR forward (swarm_gatq_forward_csr), float32-level different rounding (tests: Q
+// within 1e-5).
 struct SortedScan {
   float v[6];
 };
@@ -736,13 +695,9 @@ __global__ void __launch_bounds__(kGridThreads, 2) gatq_large_sorted_kernel(cons
   }
 }
 
-bool gatq_large_sorted_enabled(int N) {
-  const char* e = std::getenv("SWARM_COMPLETE_SORTED");
-  if (e && e[0] == '0') return false;
-  return large_sorted_smem_bytes(N) <= 227 * 1024;
+bool gatq_large_x_fits(int N, bool radius) {
+  return N <= (1 << kIdxBits) && (radius ? large_x_smem_bytes(N) : large_sorted_smem_bytes(N)) <= 227 * 1024;
 }
-
-bool gatq_large_x_fits(int N, bool radius) { return N <= (1 << kIdxBits) && large_x_smem_bytes(N, radius) <= 227 * 1024; }
 
 cudaError_t launch_gatq_large_x(const SwarmConfig& c, const float* weights, const float* state, float* q, int32_t* actions,
                                 cudaStream_t stream) {
@@ -754,21 +709,17 @@ cudaError_t launch_gatq_large_x(const SwarmConfig& c, const float* weights, cons
   p.act_out = actions;
   const bool radius = c.graph_mode == SWARM_GRAPH_RADIUS;
   p.qmax_r = radius ? sq_threshold(c.graph_radius) : 0.0f;
-  const size_t smem = large_x_smem_bytes(c.n_agents, radius);
   if (radius) {
-    cudaError_t err = cudaFuncSetAttribute(gatq_large_x_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = large_x_smem_bytes(c.n_agents);
+    cudaError_t err = cudaFuncSetAttribute(gatq_large_x_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (err != cudaSuccess) return err;
-    gatq_large_x_kernel<true><<<c.num_envs, kGridThreads, smem, stream>>>(p);
-  } else if (gatq_large_sorted_enabled(c.n_agents)) {
-    // complete graph in O(N log N): sorted sources, prefix / suffix scans (SWARM_COMPLETE_SORTED=0: the pairwise kernel)
-    const size_t ssm = large_sorted_smem_bytes(c.n_agents);
-    cudaError_t err = cudaFuncSetAttribute(gatq_large_sorted_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm);
-    if (err != cudaSuccess) return err;
-    gatq_large_sorted_kernel<<<c.num_envs, kGridThreads, ssm, stream>>>(p);
+    gatq_large_x_kernel<<<c.num_envs, kGridThreads, smem, stream>>>(p);
   } else {
-    cudaError_t err = cudaFuncSetAttribute(gatq_large_x_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    // complete graph in O(N log N): sorted sources, prefix / suffix scans
+    const size_t smem = large_sorted_smem_bytes(c.n_agents);
+    cudaError_t err = cudaFuncSetAttribute(gatq_large_sorted_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (err != cudaSuccess) return err;
-    gatq_large_x_kernel<false><<<c.num_envs, kGridThreads, smem, stream>>>(p);
+    gatq_large_sorted_kernel<<<c.num_envs, kGridThreads, smem, stream>>>(p);
   }
   return cudaGetLastError();
 }

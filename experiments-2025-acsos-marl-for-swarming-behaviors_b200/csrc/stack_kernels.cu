@@ -304,23 +304,4 @@ cudaError_t launch_gatstack_forward(const SwarmConfig& c, const SwarmStackSpec& 
   return launch_stack_hp<32>(p, stream);
 }
 
-// returns[b][i] += reward (per agent, or the env's collective reward); hits[b] += agents inside hit_distance this tick
-__global__ void __launch_bounds__(256) stack_accumulate_kernel(long long total, int N, const float* __restrict__ rewards,
-                                                               int per_env, const uint8_t* __restrict__ flags,
-                                                               float* __restrict__ returns, int32_t* __restrict__ hits) {
-  for (long long gI = (long long)blockIdx.x * blockDim.x + threadIdx.x; gI < total; gI += (long long)gridDim.x * blockDim.x) {
-    const long long b = gI / N;
-    if (returns) returns[gI] = __fadd_rn(returns[gI], per_env ? rewards[b] : rewards[gI]);
-    if (hits && flags && (flags[gI] & SWARM_FLAG_HIT)) atomicAdd(&hits[b], 1);        // integer: order-independent
-  }
-}
-
-cudaError_t launch_stack_accumulate(long long total, int N, const float* rewards, int per_env, const uint8_t* flags,
-                                    float* returns, int32_t* hits, cudaStream_t stream) {
-  long long blocks = (total + 255) / 256;
-  if (blocks > 148 * 8) blocks = 148 * 8;
-  stack_accumulate_kernel<<<(int)(blocks < 1 ? 1 : blocks), 256, 0, stream>>>(total, N, rewards, per_env, flags, returns, hits);
-  return cudaGetLastError();
-}
-
 }  // namespace swarm

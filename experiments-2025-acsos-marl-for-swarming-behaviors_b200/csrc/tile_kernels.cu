@@ -10,8 +10,6 @@
 //   MODE_GRAPH    edge list / neighbour table export                      (train:94-110, simulator:9-26)
 // so the stand-alone kernels and the fused rollout are consistent by construction.  The rollout's world step is the
 // agent_step of swarm_device.cuh, which the stand-alone world-step kernels (step_kernels.cu) run as well.
-#include <cstdlib>
-
 #include "tile_tc_device.cuh"
 
 namespace swarm {
@@ -400,21 +398,15 @@ static cudaError_t launch_tile_impl(const TileParams& p, cudaStream_t stream) {
 
 // Grid shape of the Q modes.  A batch that fits one wave of CTA slots is spread EVENLY over all of them (a tick of a
 // CTA costs about the same for 7 envs as for 10 -- it is latency bound -- so what counts is that every SM carries the
-// same number of resident CTAs: C2's 4 096 envs are 410 full CTAs on 444 slots, 34 SMs with one CTA less);
-// SWARM_TILE_DENSE = 0 / 1 forces the 3- / 4-CTAs-per-SM register budget, SWARM_TILE_GRID the number of CTAs.
+// same number of resident CTAs: C2's 4 096 envs are 410 full CTAs on 444 slots, 34 SMs with one CTA less).
 static bool tile_grid_plan(TileParams& p) {
-  static const char* dense_env = std::getenv("SWARM_TILE_DENSE");
-  static const char* grid_env = std::getenv("SWARM_TILE_GRID");
   const long long B = p.cfg.num_envs;
   const long long uniform = (B + p.epb - 1) / p.epb;
-  bool dense = uniform > 3 * 148;
-  if (dense_env) dense = dense_env[0] == '1';
+  const bool dense = uniform > 3 * 148;
   const long long slots = (dense ? 4 : 3) * 148;
-  long long G = 0;
-  if (grid_env) G = std::atoll(grid_env);
-  else if (uniform <= slots) G = B < slots ? B : slots;
   p.bal_q = p.bal_r = 0;
-  if (G >= uniform && G <= B && G > 0) {
+  if (uniform <= slots && B > 0) {
+    const long long G = B < slots ? B : slots;       // uniform <= G <= B
     p.bal_q = (int)(B / G);
     p.bal_r = (int)(B - (long long)p.bal_q * G);
   }

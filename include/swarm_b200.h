@@ -520,14 +520,13 @@ int swarm_gatstack_forward_large(const SwarmConfig* cfg, const SwarmStackSpec* s
                                  const float* state, const int32_t* neighbours, float* q, int32_t* actions,
                                  void* workspace, int64_t workspace_bytes, void* stream);
 
-/* `ticks` greedy evaluation ticks (simulator.py:59-93) of a stacked network, launched back to back from the library:
- * per tick swarm_gatstack_forward (argmax) -> swarm_sim_step in place -> the tick's reward -> returns float[B*N] (+=),
- * hits int32[B] (+=, obstacles_hits()).  reward == NULL: the world's own reward (GoTo / ObstacleAvoidance); a
- * SwarmRewardSpec selects the Flocking collective reward (shaping float[B][N][2] required, initialised by a reset call
- * of swarm_scenario_reward) or Cohesion's per-agent reward on the GoTo world, evaluated by the swarm_scenario_reward
- * arithmetic after every step.  The whole loop is ONE launch (state, running return and Flocking memory in registers
- * across the ticks, same tick as swarm_rollout); SWARM_STACK_FUSED=0 launches forward, world step, reward kernel and
- * totals per tick instead (same results, bit for bit).  n_agents > 128 (up to 4096): per tick [kNN: the topk table of
+/* `ticks` greedy evaluation ticks (simulator.py:59-93) of a stacked network: per tick swarm_gatstack_forward (argmax)
+ * -> swarm_sim_step in place -> the tick's reward -> returns float[B*N] (+=), hits int32[B] (+=, obstacles_hits()).
+ * reward == NULL: the world's own reward (GoTo / ObstacleAvoidance); a SwarmRewardSpec selects the Flocking collective
+ * reward (shaping float[B][N][2] required, initialised by a reset call of swarm_scenario_reward) or Cohesion's per-agent
+ * reward on the GoTo world, evaluated by the swarm_scenario_reward arithmetic after every step.  n_agents <= 128: the
+ * whole loop is ONE launch (state, running return and Flocking memory in registers across the ticks, same tick as
+ * swarm_rollout) that leaves the workspace untouched.  n_agents > 128 (up to 4096): per tick [kNN: the topk table of
  * swarm_graph_build ->] swarm_gatstack_forward_large (argmax) -> swarm_sim_step in place, returns / hits accumulated by
  * the world step; reward must be NULL there (the Flocking / Cohesion rewards are implemented for n_agents <= 128).
  * No host work or allocation inside (graph capturable).  workspace: swarm_rollout_stack_workspace_bytes(cfg). */

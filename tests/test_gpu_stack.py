@@ -136,9 +136,9 @@ def test_five_feature_input_matches_oracle(hidden, layers):
 
 @pytest.mark.parametrize("graph", ["knn", "complete", "radius"])
 @pytest.mark.parametrize("reward", ["world_oa", "world_goto", "flocking", "cohesion"])
-def test_rollout_stack_equals_composed_calls(reward, graph, monkeypatch):
-    """swarm_rollout_stack (forward -> step -> reward -> totals, launched from the library) == the same calls composed by
-    hand, bit for bit; Flocking carries its shaping memory, Cohesion uses the 5-feature input."""
+def test_rollout_stack_equals_composed_calls(reward, graph):
+    """swarm_rollout_stack (forward -> step -> reward -> totals in one launch) == the same calls composed by hand, bit
+    for bit; Flocking carries its shaping memory, Cohesion uses the 5-feature input."""
     import swarm_b200 as sb
     ops, L = sb.ops, sb._lib
     dev = _dev()
@@ -178,17 +178,13 @@ def test_rollout_stack_equals_composed_calls(reward, graph, monkeypatch):
         else:
             ret += out["rewards"]
         hits += ((out["flags"] & L.FLAG_HIT) != 0).sum(dim=1, dtype=torch.int32)
-    # default: ONE launch for the whole loop (world reward / Flocking); SWARM_STACK_FUSED=0: the launch sequence
-    for fused in ("1", "0"):
-        monkeypatch.setenv("SWARM_STACK_FUSED", fused)
-        res = ops.rollout_stack(cfg, spec, w, state0.clone(), T, reward=rs,
-                                shaping=shaping0.clone() if shaping0 is not None else None)
-        assert torch.equal(res["state"], st), f"fused={fused}: state"
-        assert torch.equal(res["returns"], ret), f"fused={fused}: returns"
-        assert torch.equal(res["hits"], hits), f"fused={fused}: hits"
-        if reward == "flocking":
-            assert torch.equal(res["shaping"], sh), f"fused={fused}: shaping"
-    monkeypatch.delenv("SWARM_STACK_FUSED")
+    res = ops.rollout_stack(cfg, spec, w, state0.clone(), T, reward=rs,
+                            shaping=shaping0.clone() if shaping0 is not None else None)
+    assert torch.equal(res["state"], st), "state"
+    assert torch.equal(res["returns"], ret), "returns"
+    assert torch.equal(res["hits"], hits), "hits"
+    if reward == "flocking":
+        assert torch.equal(res["shaping"], sh), "shaping"
     assert (st != state0).any() and torch.isfinite(ret).all()
     # running totals continue
     res2 = ops.rollout_stack(cfg, spec, w, res["state"].clone(), 3, reward=rs, shaping=res.get("shaping"),
