@@ -22,7 +22,7 @@ FLAG_OBSTACLE_CONTACT = 1
 FLAG_HIT = 2
 FLAG_PENALTY = 4
 W_COUNT = 1673
-ABI_VERSION = 6
+ABI_VERSION = 7
 XCHG_STRIDE = 1680
 
 # state-dict tensors in packed order (include/swarm_b200.h SWARM_W_*)
@@ -179,6 +179,9 @@ _SIGNATURES = {
     "swarm_train_tick": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmTrainHyper)] + [C.c_void_p] * 8
                          + [C.POINTER(SwarmReplay)] + [C.c_void_p] * 3 + [C.c_int64, C.POINTER(SwarmPeerExchange),
                                                                           C.c_void_p]),
+    "swarm_train_tick_stack": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.POINTER(SwarmTrainHyper)]
+                               + [C.c_void_p] * 10 + [C.POINTER(SwarmReplay)] + [C.c_void_p] * 3
+                               + [C.c_int64, C.c_void_p]),
 }
 
 

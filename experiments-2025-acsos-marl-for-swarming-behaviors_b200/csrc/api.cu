@@ -37,6 +37,10 @@ cudaError_t launch_gatstack_forward(const SwarmConfig& c, const SwarmStackSpec& 
 cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
                                     int ticks, const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
                                     float* returns, int32_t* hits, cudaStream_t stream);
+cudaError_t launch_gatstack_train_tick(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
+                                       const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
+                                       float* returns, int32_t* hits, const SwarmReplay& ring, const SwarmTrainCtl* ctl,
+                                       unsigned long long rng_seed, long long env_offset, cudaStream_t stream);
 int stack_large_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
 long long stack_large_workspace_bytes(const SwarmConfig& c, int hp);
 long long stack_large_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
@@ -46,10 +50,13 @@ int stack_grad_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
 long long stack_grad_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s, int n_graphs);
 cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, const float* w_online, const float* w_target,
                               const SwarmReplay& batch, const int64_t* indices, int n_graphs, float gamma, float loss_scale,
-                              float* grad, float* loss, float* td, void* workspace, cudaStream_t stream);
+                              float* grad, float* loss, float* td, void* workspace, cudaStream_t stream,
+                              SwarmTrainCtl* ctl = nullptr, int64_t* indices_out = nullptr,
+                              unsigned long long sample_seed = 0, int pushed_envs = 0);
 cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const float* grad, float* m, float* v,
                                    long long step, double lr, double beta1, double beta2, double eps, double max_norm,
-                                   float* target, float* grad_norm, cudaStream_t stream);
+                                   float* target, float* grad_norm, cudaStream_t stream, SwarmTrainCtl* ctl = nullptr,
+                                   int num_envs = 0, long long ring_capacity = 1, int update_target_every = 1);
 bool gatq_knn_large_fits(int N, int K);
 bool gatq_large_x_fits(int N, bool radius);
 cudaError_t launch_gatq_large_x(const SwarmConfig& c, const float* weights, const float* state, float* q, int32_t* actions,
@@ -935,6 +942,25 @@ int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg) {
   return bn * 4 + bn * 4 + bn + 1024;
 }
 
+// the Flocking / Cohesion reward of the n_agents <= 128 stacked tick (reward == NULL: the world's own): checked, and
+// copied into rs as one tick over every env reads it
+static int stack_reward(const SwarmConfig* cfg, const SwarmRewardSpec* reward, const float* shaping, SwarmRewardSpec& rs) {
+  if (!reward) return SWARM_OK;
+  rs = *reward;
+  if (rs.kind != SWARM_REWARD_FLOCKING && rs.kind != SWARM_REWARD_COHESION)
+    return fail(SWARM_ERR_INVALID_ARG, "unknown reward kind");
+  if (cfg->scenario != SWARM_SCENARIO_GOTO)
+    return fail(SWARM_ERR_INVALID_ARG, "the Flocking / Cohesion rewards run on the GoTo world (cfg->scenario)");
+  if (rs.num_envs != cfg->num_envs || rs.n_agents != cfg->n_agents)
+    return fail(SWARM_ERR_INVALID_ARG, "reward spec and cfg disagree on num_envs / n_agents");
+  if (rs.n_agents < 2) return fail(SWARM_ERR_INVALID_ARG, "the scenario rewards need at least two agents");
+  if (rs.kind == SWARM_REWARD_FLOCKING && !shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
+  if (rs.kind == SWARM_REWARD_COHESION && !(rs.sigma > 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "sigma must be > 0");
+  rs.reset = 0;
+  rs.env_index = -1;
+  return SWARM_OK;
+}
+
 // n_agents > 128: per tick [topk table ->] the large stacked forward (argmax) -> the large world step with returns / hits
 static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
                                int32_t ticks, float* returns, int32_t* hits, void* workspace, cudaStream_t st) {
@@ -973,24 +999,48 @@ int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, cons
   if (workspace_bytes < swarm_rollout_stack_workspace_bytes(cfg)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
   if (large) return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, workspace, (cudaStream_t)stream);
   SwarmRewardSpec rs;
-  if (reward) {
-    rs = *reward;
-    if (rs.kind != SWARM_REWARD_FLOCKING && rs.kind != SWARM_REWARD_COHESION)
-      return fail(SWARM_ERR_INVALID_ARG, "unknown reward kind");
-    if (cfg->scenario != SWARM_SCENARIO_GOTO)
-      return fail(SWARM_ERR_INVALID_ARG, "the Flocking / Cohesion rewards run on the GoTo world (cfg->scenario)");
-    if (rs.num_envs != cfg->num_envs || rs.n_agents != cfg->n_agents)
-      return fail(SWARM_ERR_INVALID_ARG, "reward spec and cfg disagree on num_envs / n_agents");
-    if (rs.n_agents < 2) return fail(SWARM_ERR_INVALID_ARG, "the scenario rewards need at least two agents");
-    if (rs.kind == SWARM_REWARD_FLOCKING && !shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
-    if (rs.kind == SWARM_REWARD_COHESION && !(rs.sigma > 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "sigma must be > 0");
-    rs.reset = 0;
-    rs.env_index = -1;
-  }
+  if (int rc = stack_reward(cfg, reward, shaping, rs)) return rc;
   // the whole loop is ONE launch with the state in registers (stack_kernels.cu gatstack_kernel<HP, true>)
   return check_cuda(launch_gatstack_rollout(*cfg, *spec, weights, state, ticks, world_consts(*cfg), reward ? &rs : nullptr,
                                             shaping, returns, hits, (cudaStream_t)stream),
                     "swarm_rollout_stack");
+}
+
+int swarm_train_tick_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                           const SwarmRewardSpec* reward, float* shaping, SwarmTrainCtl* ctl, float* weights,
+                           float* target_weights, float* exp_avg, float* exp_avg_sq, float* state, float* returns,
+                           int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
+                           int64_t workspace_bytes, void* stream) {
+  if (int rc = validate_hyper(hyper)) return rc;
+  if (int rc = validate_stack(cfg, spec)) return rc;
+  const int G = hyper->graphs_per_update;
+  if (int rc = validate_dqn_stack(cfg, spec, G)) return rc;
+  if (hyper->flocking)
+    return fail(SWARM_ERR_INVALID_ARG, "hyper->flocking must be NULL: the stacked tick takes its reward as `reward`");
+  if (!ctl || !weights || !target_weights || !exp_avg || !exp_avg_sq || !state || !grad || !workspace)
+    return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
+  if (!ring || !ring->state || !ring->next_state || !ring->actions || !ring->rewards || ring->capacity <= 0)
+    return fail(SWARM_ERR_INVALID_ARG, "replay ring has NULL arrays or no capacity");
+  if (cfg->num_envs > ring->capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
+  if (workspace_bytes < stack_grad_workspace_bytes(*cfg, *spec, G)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  SwarmRewardSpec rs;
+  if (int rc = stack_reward(cfg, reward, shaping, rs)) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  float* loss = grad + stack_weight_count_host(*spec);
+  if (int rc = check_cuda(launch_gatstack_train_tick(*cfg, *spec, weights, state, world_consts(*cfg), reward ? &rs : nullptr,
+                                                     shaping, returns, hits, *ring, ctl, hyper->rng_seed, hyper->env_offset,
+                                                     st),
+                          "swarm_train_tick_stack(rollout)"))
+    return rc;
+  if (int rc = check_cuda(launch_stack_grad(*cfg, *spec, weights, target_weights, *ring, nullptr, G, hyper->gamma,
+                                            hyper->loss_scale, grad, loss, nullptr, workspace, st, ctl, indices,
+                                            hyper->sample_seed, cfg->num_envs),
+                          "swarm_train_tick_stack(grad)"))
+    return rc;
+  return check_cuda(launch_stack_adam_clip(*spec, weights, grad, exp_avg, exp_avg_sq, 1, hyper->lr, hyper->beta1,
+                                           hyper->beta2, hyper->eps, hyper->max_norm, target_weights, nullptr, st, ctl,
+                                           cfg->num_envs, ring->capacity, hyper->update_target_every),
+                    "swarm_train_tick_stack(apply)");
 }
 
 int swarm_episode_end(const SwarmConfig* cfg, SwarmTrainCtl* ctl, float* returns, int32_t* hits, const float* loss,

@@ -37,6 +37,16 @@ __device__ __forceinline__ long long train_ring_size(const SwarmTrainCtl* ctl, i
   return size < capacity ? size : capacity;
 }
 
+// end of a device-driven tick: tick, ring cursor / fill and (after an update) the optimiser step advance; shared by the
+// clip + Adam kernels of the one-layer network and of stacked networks
+__device__ __forceinline__ void train_ctl_advance(SwarmTrainCtl* ctl, int num_envs, long long capacity, bool stepped) {
+  ctl->tick += 1;
+  ctl->ring_cursor = (ctl->ring_cursor + num_envs) % capacity;
+  const long long sz = ctl->ring_size + num_envs;
+  ctl->ring_size = sz < capacity ? sz : capacity;
+  if (stepped) ctl->opt_step += 1;
+}
+
 // one Adam step of one element, op for op as torch.optim.Adam (single-tensor path); shared by the clip + Adam kernels
 // of the one-layer network (dqn_kernels.cu) and of stacked networks (stack_grad_kernels.cu)
 struct AdamScalars {

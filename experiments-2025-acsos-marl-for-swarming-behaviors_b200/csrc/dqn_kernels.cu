@@ -573,14 +573,6 @@ __device__ __forceinline__ float clip_coefficient(const float (&g_)[kAdamPer], d
   return s_coef;
 }
 
-__device__ __forceinline__ void train_ctl_advance(SwarmTrainCtl* ctl, int num_envs, long long capacity, bool stepped) {
-  ctl->tick += 1;
-  ctl->ring_cursor = (ctl->ring_cursor + num_envs) % capacity;
-  const long long sz = ctl->ring_size + num_envs;
-  ctl->ring_size = sz < capacity ? sz : capacity;
-  if (stepped) ctl->opt_step += 1;
-}
-
 // one naturally aligned 64-bit word = (epoch << 32 | float bits): single-copy atomic, so the word itself is the flag
 __device__ __forceinline__ void st_relaxed_sys_u64(uint64_t* p, uint64_t v) {
   asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");

@@ -32,6 +32,11 @@ struct StackGradParams {
   float* td;
   int32_t epb, maxdeg, stride, count;
   float qmax_r;
+  // device-driven tick (stack_grad_ctl_kernel): slots are drawn here from the ring fill after this tick's push
+  const SwarmTrainCtl* ctl;
+  int64_t* indices_out;       // [n_graphs] the drawn slots (exported for tests / logging)
+  unsigned long long sample_seed;
+  int32_t pushed_envs;        // transitions pushed by this tick's rollout
 };
 
 struct StackGradSmem {
@@ -98,8 +103,12 @@ __device__ __forceinline__ float dot_row(const float (&v)[HP], const float* row)
   return acc;
 }
 
-template <int HP>
-__global__ void __launch_bounds__(kTileThreads) stack_grad_kernel(const __grid_constant__ StackGradParams p) {
+// CTL: the gradient phase of swarm_train_tick_stack -- every CTA exits while the ring holds fewer than n_graphs slots,
+// otherwise graph g takes a slot drawn from the ring fill (the draw of dqn_grad_tc_kernel).  A separate template value
+// so that the stand-alone gradient kernel keeps its code instruction for instruction (the parameter block is taken by
+// value for the same reason: through a reference the inlined body compiled to different code).
+template <int HP, bool CTL>
+__device__ __forceinline__ void stack_grad_body(const StackGradParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
   using SL = StackLayout<HP>;
   constexpr int T = kTileThreads;
@@ -109,6 +118,7 @@ __global__ void __launch_bounds__(kTileThreads) stack_grad_kernel(const __grid_c
   const int N = c.n_agents, K = c.knn_k, L = sp.n_layers, H = sp.hidden;
   const TileThread t = tile_thread(N, p.epb, p.n_graphs);
   const int tid = t.tid;
+  if (CTL && train_ring_size(p.ctl, p.pushed_envs, p.batch.capacity) < p.n_graphs) return;   // not filled yet (train:113-115)
   const StackGradSmem S = stack_grad_smem<HP>(L, p.maxdeg, c.graph_mode);
   float* sw = reinterpret_cast<float*>(smem + S.w);
   float4* sst = reinterpret_cast<float4*>(smem + S.st);
@@ -139,7 +149,11 @@ __global__ void __launch_bounds__(kTileThreads) stack_grad_kernel(const __grid_c
   float rew = 0.0f;
   if (t.active) {
     long long slot = t.env;
-    if (p.indices) {
+    if (CTL) {
+      const uint64_t rnd = rng_draw(p.sample_seed, (uint64_t)t.env, (uint64_t)(p.ctl->tick + 1), 0x5A17u);
+      slot = (long long)__umul64hi(rnd, (uint64_t)train_ring_size(p.ctl, p.pushed_envs, p.batch.capacity));
+      if (p.indices_out && t.i == 0) p.indices_out[t.env] = slot;
+    } else if (p.indices) {
       slot = p.indices[t.env];                            // caller-supplied: clamped into the ring, never out of bounds
       slot = slot < 0 ? 0 : (slot >= p.batch.capacity ? p.batch.capacity - 1 : slot);
     }
@@ -377,16 +391,46 @@ __global__ void __launch_bounds__(kTileThreads) stack_grad_kernel(const __grid_c
   }
 }
 
+template <int HP>
+__global__ void __launch_bounds__(kTileThreads) stack_grad_kernel(const __grid_constant__ StackGradParams p) {
+  stack_grad_body<HP, false>(p);
+}
+
+// width 8: a 96-register budget (five CTAs per SM, more than the Flocking shape's shared memory allows) -- with ptxas's
+// own choice of 72 the sampling prologue spilled 24 bytes
+template <int HP>
+__global__ void __launch_bounds__(kTileThreads, HP == 8 ? 5 : 0) stack_grad_ctl_kernel(const __grid_constant__ StackGradParams p) {
+  stack_grad_body<HP, true>(p);
+}
+
 // grad[o] = sum over CTAs (in CTA order) of partials[cta][o]; loss = loss_scale * sum of squared TD errors
-__global__ void __launch_bounds__(256) stack_reduce_kernel(const float* __restrict__ partials, int n_ctas, int stride,
-                                                           int count, float loss_scale, float* __restrict__ grad,
-                                                           float* __restrict__ loss) {
-  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+__device__ __forceinline__ void stack_reduce_element(const float* __restrict__ partials, int n_ctas, int stride, int count,
+                                                     float loss_scale, float* __restrict__ grad, float* __restrict__ loss,
+                                                     int o) {
   if (o > count) return;
   float acc = 0.0f;
   for (int b = 0; b < n_ctas; ++b) acc = __fadd_rn(acc, partials[(long long)b * stride + o]);
   if (o < count) grad[o] = acc;
   else loss[0] = __fmul_rn(acc, loss_scale);
+}
+
+__global__ void __launch_bounds__(256) stack_reduce_kernel(const float* __restrict__ partials, int n_ctas, int stride,
+                                                           int count, float loss_scale, float* __restrict__ grad,
+                                                           float* __restrict__ loss) {
+  stack_reduce_element(partials, n_ctas, stride, count, loss_scale, grad, loss, blockIdx.x * blockDim.x + threadIdx.x);
+}
+
+// device-driven tick: publishes whether this tick updates (read by the clip + Adam kernel) and leaves grad / loss
+// untouched when it does not (as dqn_reduce_kernel)
+__global__ void __launch_bounds__(256) stack_reduce_ctl_kernel(const float* __restrict__ partials, int n_ctas, int stride,
+                                                               int count, float loss_scale, float* __restrict__ grad,
+                                                               float* __restrict__ loss, SwarmTrainCtl* __restrict__ ctl,
+                                                               int pushed_envs, long long capacity, int n_graphs) {
+  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool upd = train_ring_size(ctl, pushed_envs, capacity) >= n_graphs;
+  if (o == 0) ctl->updating = upd ? 1 : 0;
+  if (!upd) return;
+  stack_reduce_element(partials, n_ctas, stride, count, loss_scale, grad, loss, o);
 }
 
 // ---- launchers -------------------------------------------------------------------------------------------------------
@@ -424,17 +468,23 @@ long long stack_grad_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec&
 template <int HP>
 static cudaError_t launch_stack_grad_hp(const StackGradParams& p, int ctas, cudaStream_t stream) {
   const int smem = stack_grad_smem<HP>(p.spec.n_layers, p.maxdeg, p.cfg.graph_mode).total;
-  cudaError_t err = cudaFuncSetAttribute(stack_grad_kernel<HP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  auto* kernel = p.ctl ? stack_grad_ctl_kernel<HP> : stack_grad_kernel<HP>;
+  cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (err != cudaSuccess) return err;
-  stack_grad_kernel<HP><<<ctas, kTileThreads, smem, stream>>>(p);
+  kernel<<<ctas, kTileThreads, smem, stream>>>(p);
   return cudaGetLastError();
 }
 
 cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, const float* w_online, const float* w_target,
                               const SwarmReplay& batch, const int64_t* indices, int n_graphs, float gamma, float loss_scale,
-                              float* grad, float* loss, float* td, void* workspace, cudaStream_t stream) {
+                              float* grad, float* loss, float* td, void* workspace, cudaStream_t stream,
+                              SwarmTrainCtl* ctl, int64_t* indices_out, unsigned long long sample_seed, int pushed_envs) {
   StackGradParams p;
   std::memset(&p, 0, sizeof(p));
+  p.ctl = ctl;
+  p.indices_out = indices_out;
+  p.sample_seed = sample_seed;
+  p.pushed_envs = pushed_envs;
   p.cfg = c;
   p.spec = spec;
   p.w_online = w_online;
@@ -459,8 +509,12 @@ cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, 
     default: err = launch_stack_grad_hp<32>(p, ctas, stream); break;
   }
   if (err != cudaSuccess) return err;
-  stack_reduce_kernel<<<(p.count + 1 + 255) / 256, 256, 0, stream>>>(p.partials, ctas, p.stride, p.count, loss_scale, grad,
-                                                                      loss);
+  const int blocks = (p.count + 1 + 255) / 256;
+  if (ctl)
+    stack_reduce_ctl_kernel<<<blocks, 256, 0, stream>>>(p.partials, ctas, p.stride, p.count, loss_scale, grad, loss, ctl,
+                                                        pushed_envs, batch.capacity, n_graphs);
+  else
+    stack_reduce_kernel<<<blocks, 256, 0, stream>>>(p.partials, ctas, p.stride, p.count, loss_scale, grad, loss);
   return cudaGetLastError();
 }
 
@@ -482,17 +536,42 @@ struct StackAdamParams {
   int32_t seg[kStackMaxTensors + 1];
   AdamScalars sc;
   float max_norm;
+  // device-driven tick (stack_adam_clip_ctl_kernel): the step-dependent scalars come from *ctl on the device and the
+  // cursor is advanced at the end
+  SwarmTrainCtl* ctl;
+  double lr, beta1, beta2;
+  long long ring_capacity;
+  int32_t num_envs;
+  int32_t update_target_every;
 };
 
-__global__ void __launch_bounds__(256) stack_adam_clip_kernel(const __grid_constant__ StackAdamParams p) {
+// CTL: the last launch of swarm_train_tick_stack, as adam_clip_kernel<false> with a cursor (dqn_kernels.cu): bias
+// corrections from ctl->opt_step + 1, target sync when (ctl->tick + 1) % update_target_every == 0, no update while
+// ctl->updating == 0, then the cursor advances.  A separate template value so that the stand-alone kernel keeps its code
+// instruction for instruction (tid is read in the kernel, where the compiler knows it is below 256).
+template <bool CTL>
+__device__ __forceinline__ void stack_adam_clip_body(const StackAdamParams p, const int tid) {
   __shared__ double swarp[kStackMaxTensors][8];
   __shared__ float s_coef;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  __shared__ float s_neg_step, s_bc2_sqrt;
+  __shared__ int s_update, s_sync;
+  const int lane = tid & 31, warp = tid >> 5;
   float g_[kStackAdamPer];
 #pragma unroll
   for (int i = 0; i < kStackAdamPer; ++i) {
     const int o = tid + 256 * i;
     g_[i] = o < p.count ? p.grad[o] : 0.0f;
+  }
+  if (CTL && tid == 255) {
+    // step-dependent scalars from the device cursor (after this warp's loads went out: the two pow chains run under
+    // their latency)
+    const long long step = p.ctl->opt_step + 1;
+    const double bc1 = 1.0 - pow(p.beta1, (double)step);
+    const double bc2 = 1.0 - pow(p.beta2, (double)step);
+    s_neg_step = (float)(-(p.lr / bc1));
+    s_bc2_sqrt = (float)sqrt(bc2);
+    s_update = p.ctl->updating;
+    s_sync = ((p.ctl->tick + 1) % p.update_target_every) == 0;
   }
   for (int sgi = 0; sgi < p.n_tensors; ++sgi) {
     double acc = 0.0;
@@ -506,6 +585,17 @@ __global__ void __launch_bounds__(256) stack_adam_clip_kernel(const __grid_const
     if (lane == 0) swarp[sgi][warp] = acc;
   }
   __syncthreads();
+  AdamScalars sc = p.sc;
+  float* target = p.target;
+  if (CTL) {
+    if (!s_update) {
+      if (tid == 0) train_ctl_advance(p.ctl, p.num_envs, p.ring_capacity, false);
+      return;
+    }
+    sc.neg_step_size = s_neg_step;
+    sc.bc2_sqrt = s_bc2_sqrt;
+    if (!s_sync) target = nullptr;
+  }
   if (tid == 0) {
     double tot = 0.0;
     for (int sgi = 0; sgi < p.n_tensors; ++sgi) {
@@ -531,19 +621,36 @@ __global__ void __launch_bounds__(256) stack_adam_clip_kernel(const __grid_const
     const int o = tid + 256 * i;
     if (o >= p.count) break;
     float m = p.m[o], v = p.v[o], w = p.w[o];
-    adam_element(p.sc, g_[i], coef, m, v, w);
+    adam_element(sc, g_[i], coef, m, v, w);
     p.m[o] = m;
     p.v[o] = v;
     p.w[o] = w;
-    if (p.target) p.target[o] = w;
+    if (target) target[o] = w;
   }
+  if (CTL && tid == 0) train_ctl_advance(p.ctl, p.num_envs, p.ring_capacity, true);
+}
+
+__global__ void __launch_bounds__(256) stack_adam_clip_kernel(const __grid_constant__ StackAdamParams p) {
+  stack_adam_clip_body<false>(p, threadIdx.x);
+}
+
+__global__ void __launch_bounds__(256) stack_adam_clip_ctl_kernel(const __grid_constant__ StackAdamParams p) {
+  stack_adam_clip_body<true>(p, threadIdx.x);
 }
 
 cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const float* grad, float* m, float* v,
                                    long long step, double lr, double beta1, double beta2, double eps, double max_norm,
-                                   float* target, float* grad_norm, cudaStream_t stream) {
+                                   float* target, float* grad_norm, cudaStream_t stream, SwarmTrainCtl* ctl,
+                                   int num_envs, long long ring_capacity, int update_target_every) {
   StackAdamParams p;
   std::memset(&p, 0, sizeof(p));
+  p.ctl = ctl;
+  p.lr = lr;
+  p.beta1 = beta1;
+  p.beta2 = beta2;
+  p.ring_capacity = ring_capacity;
+  p.num_envs = num_envs;
+  p.update_target_every = update_target_every > 0 ? update_target_every : 1;
   p.w = w;
   p.grad = grad;
   p.m = m;
@@ -571,7 +678,8 @@ cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const f
   p.sc.bc2_sqrt = (float)sqrt(bc2);
   p.sc.eps = (float)eps;
   p.max_norm = (float)max_norm;
-  stack_adam_clip_kernel<<<1, 256, 0, stream>>>(p);
+  if (ctl) stack_adam_clip_ctl_kernel<<<1, 256, 0, stream>>>(p);
+  else stack_adam_clip_kernel<<<1, 256, 0, stream>>>(p);
   return cudaGetLastError();
 }
 

@@ -36,6 +36,12 @@ struct StackParams {
   float2* shaping;           // [B*N] Flocking memory, read at launch, written back
   int32_t use_flock;
   int32_t ticks;
+  // device-driven train tick (gatstack_train_kernel): one tick with epsilon-greedy exploration and the replay push;
+  // epsilon, the RNG tick and the ring cursor come from *ctl
+  const SwarmTrainCtl* ctl;
+  SwarmReplay replay;
+  unsigned long long rng_seed;
+  long long env_offset;
 };
 
 struct StackSmem {
@@ -61,8 +67,13 @@ __host__ __device__ inline StackSmem stack_smem(int L, int n, int k, int maxdeg,
 // stacked network -- p.ticks x [forward -> argmax -> world step -> reward] with the agent's state, running return and
 // Flocking memory in registers, exactly the tick of tile_kernels.cu's rollout (same world-step and reward device code,
 // so it equals forward + swarm_sim_step + swarm_scenario_reward composed by hand bit for bit).
-template <int HP, bool ROLLOUT>
-__global__ void __launch_bounds__(kTileThreads) gatstack_kernel(const __grid_constant__ StackParams p) {
+// TRAIN (with ROLLOUT, p.ticks = 1): the rollout tick of the device-driven train tick (train:160-172) -- the greedy
+// action is replaced by the exploration draws of tile_kernels.cu's MODE_ROLLOUT with p.ctl, and the transition
+// (s, a, r, s') is pushed at slot (ctl->ring_cursor + env) % capacity.  A separate template value so that the forward
+// and the evaluation rollout keep their code instruction for instruction.
+template <int HP, bool ROLLOUT, bool TRAIN>
+__device__ __forceinline__ void gatstack_body(const StackParams& p) {
+  static_assert(!TRAIN || ROLLOUT, "the train tick is a rollout tick");
   extern __shared__ __align__(16) unsigned char smem[];
   using SL = StackLayout<HP>;
   const SwarmConfig& c = p.cfg;
@@ -141,9 +152,27 @@ __global__ void __launch_bounds__(kTileThreads) gatstack_kernel(const __grid_con
       const bool oa = c.scenario == SWARM_SCENARIO_OBSTACLE_AVOIDANCE;
       uint8_t flags = 0;
       uint32_t cmask = 0;
+      // the cursor is read here, not in the prologue: live across the layers it would cost spills
+      const float epsilon = TRAIN ? p.ctl->epsilon : 0.0f;
+      if (TRAIN && epsilon > 0.0f) {
+        // train:164-165: one coin per tick for the whole swarm, then one uniform action per agent (the stream of the
+        // one-layer tick)
+        const unsigned long long genv = (unsigned long long)(p.env_offset + t.env);
+        const unsigned long long gt = (unsigned long long)(p.ctl->tick + 1);
+        const float coin = (float)(rng_draw(p.rng_seed, genv, gt, 0xFFFFu) >> 40) * (1.0f / 16777216.0f);
+        if (coin < epsilon) action = (int)(((rng_draw(p.rng_seed, genv, gt, (uint32_t)t.i) >> 32) * 9ull) >> 32);
+      }
+      const float4 s_prev = s;
       float2 u;
       decode_action(action, u.x, u.y);
       agent_step(s, u, pos + t.envbase, N, t.i, oa, c, p.step, flags, cmask);
+      if (TRAIN) {
+        // GraphReplayBuffer.push (train:171-172), state-only transition; the reward follows below
+        const long long ri = ((p.ctl->ring_cursor + t.env) % p.replay.capacity) * N + t.i;
+        reinterpret_cast<float4*>(p.replay.state)[ri] = s_prev;
+        reinterpret_cast<float4*>(p.replay.next_state)[ri] = s;
+        p.replay.actions[ri] = (uint8_t)sanitize_action(action);
+      }
       float dgoal, dobs;
       reward = post_step_reward(s, oa, c, dgoal, dobs, flags);
       if (oa) myhits += (flags & SWARM_FLAG_HIT) ? 1 : 0;
@@ -209,6 +238,7 @@ __global__ void __launch_bounds__(kTileThreads) gatstack_kernel(const __grid_con
         for (int a = 0; a < N; ++a) reward = __fadd_rn(reward, -sred[t.envbase + a]);
     }
     ret = __fadd_rn(ret, reward);
+    if (TRAIN && t.active) p.replay.rewards[((p.ctl->ring_cursor + t.env) % p.replay.capacity) * N + t.i] = reward;
   }
   }   // tick loop
 
@@ -231,20 +261,28 @@ __global__ void __launch_bounds__(kTileThreads) gatstack_kernel(const __grid_con
   }
 }
 
+template <int HP, bool ROLLOUT>
+__global__ void __launch_bounds__(kTileThreads) gatstack_kernel(const __grid_constant__ StackParams p) {
+  gatstack_body<HP, ROLLOUT, false>(p);
+}
+
+template <int HP>
+__global__ void __launch_bounds__(kTileThreads) gatstack_train_kernel(const __grid_constant__ StackParams p) {
+  gatstack_body<HP, true, true>(p);
+}
+
 template <int HP>
 static cudaError_t launch_stack_hp(const StackParams& p, cudaStream_t stream) {
   const SwarmConfig& c = p.cfg;
   const StackSmem S = stack_smem<HP>(p.spec.n_layers, c.n_agents, c.knn_k, p.maxdeg, c.graph_mode);
   if (S.total > 227 * 1024) return cudaErrorInvalidConfiguration;
+  auto* kernel = p.ctl ? gatstack_train_kernel<HP> : (p.ticks > 0 ? gatstack_kernel<HP, true> : gatstack_kernel<HP, false>);
   if (S.total > 48 * 1024) {
-    cudaError_t err = p.ticks > 0
-        ? cudaFuncSetAttribute(gatstack_kernel<HP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, S.total)
-        : cudaFuncSetAttribute(gatstack_kernel<HP, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, S.total);
+    cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, S.total);
     if (err != cudaSuccess) return err;
   }
   const int grid = (c.num_envs + p.epb - 1) / p.epb;
-  if (p.ticks > 0) gatstack_kernel<HP, true><<<grid, kTileThreads, S.total, stream>>>(p);
-  else gatstack_kernel<HP, false><<<grid, kTileThreads, S.total, stream>>>(p);
+  kernel<<<grid, kTileThreads, S.total, stream>>>(p);
   return cudaGetLastError();
 }
 
@@ -283,6 +321,30 @@ cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& 
     p.shaping = reinterpret_cast<float2*>(shaping);
     p.use_flock = flock->kind == SWARM_REWARD_COHESION ? 2 : 1;
   }
+  return launch_stack(p, stream);
+}
+
+// the rollout tick of swarm_train_tick_stack: one tick of the loop above with exploration and the replay push
+cudaError_t launch_gatstack_train_tick(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
+                                       const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
+                                       float* returns, int32_t* hits, const SwarmReplay& ring, const SwarmTrainCtl* ctl,
+                                       unsigned long long rng_seed, long long env_offset, cudaStream_t stream) {
+  StackParams p;
+  stack_fill(p, c, spec, weights);
+  p.step = step;
+  p.state_rw = reinterpret_cast<float4*>(state);
+  p.returns = returns;
+  p.hits = hits;
+  p.ticks = 1;
+  if (flock) {
+    p.flock = *flock;
+    p.shaping = reinterpret_cast<float2*>(shaping);
+    p.use_flock = flock->kind == SWARM_REWARD_COHESION ? 2 : 1;
+  }
+  p.ctl = ctl;
+  p.replay = ring;
+  p.rng_seed = rng_seed;
+  p.env_offset = env_offset;
   return launch_stack(p, stream);
 }
 

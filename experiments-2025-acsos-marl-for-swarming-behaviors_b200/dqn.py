@@ -14,7 +14,9 @@ Two drivers:
 
 ``DQNTrainer(..., model=StackedGCN(...))`` trains a stacked network (the conv1 .. convL form the reference ships as
 data/models/experiment_Flocking-seed_*.pth) instead of the one-layer GCN: ``train_model`` and ``train_model_stepwise``
-then run the stack's gradient kernel (``swarm_dqn_stack_grad``) and clip + Adam (``swarm_adam_clip_stack_step``).
+then run the stack's gradient kernel (``swarm_dqn_stack_grad``) and clip + Adam (``swarm_adam_clip_stack_step``), and
+``train_model_stack_device`` is the stack's whole-run device loop -- one ``swarm_train_tick_stack`` call (four launches)
+per tick, one CUDA-graph replay per episode -- for the GoTo, ObstacleAvoidance, Flocking and Cohesion rewards on one GPU.
 """
 from __future__ import annotations
 
@@ -188,7 +190,7 @@ class DQNTrainer:
     def _require_one_layer(self, what: str) -> None:
         if self.stack_spec is not None:
             raise NotImplementedError(f"{what} runs the fused train tick of the one-layer GCN; train a StackedGCN with "
-                                      "train_model_stepwise (or train_model for one env)")
+                                      "train_model_stack_device or train_model_stepwise (or train_model for one env)")
 
     def train_step_dqn(self, batch_size, model=None, target_model=None, ticks=0, gamma=0.99, update_target_every=10,
                        indices: Optional[torch.Tensor] = None):
@@ -478,23 +480,81 @@ class DQNTrainer:
                 tt.apply_phase(self.w, self.w_target, self.exp_avg, self.exp_avg_sq)
             tt.episode_end(returns, hits, stats, config["epsilon"], config["epsilon_decay"], config["min_epsilon"])
 
-        done = 0
-        if bool(config.get("cuda_graph", True)) and episodes > 1:
-            episode()                                   # eager once: kernel attributes set, NCCL communicator warm
-            done = 1
-            torch.cuda.synchronize(dev)
-            graph = torch.cuda.CUDAGraph()
-            side = torch.cuda.Stream(dev)
-            side.wait_stream(torch.cuda.current_stream(dev))
-            with torch.cuda.graph(graph, stream=side):
-                episode()
-            for _ in range(episodes - 1):            # capture records, it does not execute
-                graph.replay()
-            done = episodes
-        for _ in range(episodes - done):
-            episode()
+        _run_episodes(episode, episodes, bool(config.get("cuda_graph", True)), dev)
         cur = tt.read_cursor()
         self.opt_step = cur["opt_step"]
+        self._grad.copy_(tt.grad)
+        self._loss.copy_(tt.loss)
+        self.sync_modules()
+        out = stats.cpu()
+        self.episode_losses.extend(out[:, 2].tolist())
+        return out
+
+    def train_model_stack_device(self, config) -> torch.Tensor:
+        """``train_model_device`` for a stacked network: every episode is ONE replay of a CUDA graph holding
+        [reset -> max_steps x swarm_train_tick_stack -> swarm_episode_end] (after one eager episode; ``cuda_graph``
+        False runs every episode eagerly), four launches per tick and no host synchronisation until the run ends.  The
+        reward is the world's own (GoTo / ObstacleAvoidance), Flocking's (its shaping memory reset on the device with
+        the world) or Cohesion's.  GoTo / ObstacleAvoidance / Flocking start from ``swarm_reset_random``; Cohesion starts
+        from its fixed table, so its reset is a device copy of the state one ``env.reset()`` leaves.  One GPU.  Returns
+        stats f32[episodes, 4] = (mean agent-0 return / N, hits per env, last loss, epsilon)."""
+        if self.stack_spec is None:
+            raise NotImplementedError("train_model_stack_device trains a StackedGCN; the one-layer GCN has "
+                                      "train_model_device")
+        if parallel.world_size() > 1:
+            raise NotImplementedError("train_model_stack_device runs on one GPU (data-parallel stacked training is not "
+                                      "implemented)")
+        env, world = self.env, self.env.world
+        flock = isinstance(env.scenario, FlockingScenario)
+        cohesion = isinstance(env.scenario, CohesionScenario)
+        if not (flock or cohesion or isinstance(env.scenario, _KernelScenario)):
+            raise NotImplementedError("the stacked device loop covers the GoTo, ObstacleAvoidance, Flocking and Cohesion "
+                                      "rewards; train other scenarios with train_model_stepwise")
+        B, n, dev = env.num_envs, env.n_agents, env.device
+        episodes = int(config["episodes"])
+        cfg = ops.clone_config(self.graph_cfg, num_envs=B)
+        reward = shaping = None
+        if flock:
+            reward, shaping = env.scenario._spec(), env.scenario.shaping
+        elif cohesion:
+            reward = ops.reward_spec(_lib.REWARD_COHESION, B, n, agent_radius=world.cfg.agent_radius,
+                                     sigma=env.scenario.sigma)
+        tt = ops.StackTrainTick(cfg, self.stack_spec, self.replay_buffer.ring,
+                                graphs_per_update=int(config.get("graphs_per_update", 32)),
+                                update_target_every=int(config.get("update_target_every", 200)),
+                                gamma=float(config.get("gamma", 0.99)), lr=self.lr, betas=self.betas, eps=self.eps,
+                                max_norm=self.max_norm, rng_seed=self.seed,
+                                sample_seed=int(config.get("sample_seed", self.seed)),
+                                env_offset=int(config.get("env_offset", 0)), reward=reward, shaping=shaping)
+        if cohesion:
+            env.reset()
+            start = world.state.clone()
+
+            def reset():
+                world.state.copy_(start)
+        else:
+            spec = ops.reset_spec(cfg.scenario, random=bool(getattr(env.scenario, "random", True)),
+                                  seed=int(config.get("reset_seed", self.seed)), env_offset=tt.hyper.env_offset,
+                                  shared_center=bool(config.get("shared_center", False)), flocking=flock)
+
+            def reset():
+                ops.reset_random(cfg, spec, world.state, ctl=tt.ctl)
+                if flock:
+                    ops.scenario_reward(reward, world.state, shaping, reset=True)
+        self.w_target.copy_(self.w)
+        tt.load_cursor(int(config.get("start_tick", 0)), self.opt_step, config["epsilon"], 0)
+        returns = torch.zeros(B, n, dtype=torch.float32, device=dev)
+        hits = torch.zeros(B, dtype=torch.int32, device=dev)
+        stats = torch.zeros(episodes, 4, dtype=torch.float32, device=dev)
+
+        def episode():
+            reset()
+            for _ in range(env.max_steps):
+                tt.tick(self.w, self.w_target, self.exp_avg, self.exp_avg_sq, world.state, returns, hits)
+            tt.episode_end(returns, hits, stats, config["epsilon"], config["epsilon_decay"], config["min_epsilon"])
+
+        _run_episodes(episode, episodes, bool(config.get("cuda_graph", True)), dev)
+        self.opt_step = tt.read_cursor()["opt_step"]
         self._grad.copy_(tt.grad)
         self._loss.copy_(tt.loss)
         self.sync_modules()
@@ -554,6 +614,26 @@ class DQNTrainer:
             for i in range(len(self.episode_losses)):
                 if (i + 1) % 10 == 0:
                     writer.writerow([i, self.episode_rewards[i // 10].item(), self.episode_losses[i // 10]])
+
+
+def _run_episodes(episode, episodes: int, cuda_graph: bool, dev) -> None:
+    """Run ``episode()`` ``episodes`` times: with ``cuda_graph`` (and more than one episode) once eagerly -- kernel
+    attributes set, an NCCL communicator warm -- then captured once and replayed for the others."""
+    done = 0
+    if cuda_graph and episodes > 1:
+        episode()
+        done = 1
+        torch.cuda.synchronize(dev)
+        graph = torch.cuda.CUDAGraph()
+        side = torch.cuda.Stream(dev)
+        side.wait_stream(torch.cuda.current_stream(dev))
+        with torch.cuda.graph(graph, stream=side):
+            episode()
+        for _ in range(episodes - 1):            # capture records, it does not execute
+            graph.replay()
+        done = episodes
+    for _ in range(episodes - done):
+        episode()
 
 
 def set_seed(seed):

@@ -358,18 +358,16 @@ def reset_random(cfg: SwarmConfig, spec: _lib.SwarmResetSpec, state: torch.Tenso
     return state
 
 
-class TrainTick:
-    """Device-driven train tick (swarm_train_tick_grad / swarm_train_tick_apply): one iteration of the loop body of
-    train_gcn_dqn.py:153-178 for all B envs, with the tick number, replay cursor / fill, optimiser step and epsilon
-    held in a 48-byte device struct that the kernels advance themselves.  No launch argument changes from tick to
-    tick, so ``grad_phase`` / ``apply_phase`` can be captured in a CUDA graph and replayed (``DQNTrainer``)."""
+class _TrainCursor:
+    """The device cursor of a device-driven train tick (``TrainTick``, ``StackTrainTick``): the tick number, replay
+    cursor / fill, optimiser step and epsilon held in a 48-byte device struct that the kernels advance themselves, the
+    hyper-parameters, and the host-side bookkeeping around them.  Subclasses hold ``loss``, the last update's loss."""
 
     CTL_WORDS = 6      # int64 words: tick, ring_cursor, ring_size, opt_step, (epsilon f32 | updating i32), episode
 
-    def __init__(self, cfg: SwarmConfig, ring: ReplayRing, *, graphs_per_update: int = 32, update_target_every: int = 200,
-                 gamma: float = 0.99, loss_scale: Optional[float] = None, lr: float = 1e-3, betas=(0.9, 0.999),
-                 eps: float = 1e-8, max_norm: float = 1.0, rng_seed: int = 0, sample_seed: int = 0, env_offset: int = 0,
-                 flocking: Optional["_lib.SwarmRewardSpec"] = None, shaping: Optional[torch.Tensor] = None):
+    def __init__(self, cfg: SwarmConfig, ring: ReplayRing, graphs_per_update: int, update_target_every: int, gamma: float,
+                 loss_scale: Optional[float], lr: float, betas, eps: float, max_norm: float, rng_seed: int,
+                 sample_seed: int, env_offset: int):
         dev = ring.state.device
         self.cfg, self.ring = cfg, ring
         G = int(graphs_per_update)
@@ -381,27 +379,11 @@ class TrainTick:
         h.graphs_per_update, h.update_target_every = G, int(update_target_every)
         h.gamma = float(gamma)
         h.loss_scale = float(loss_scale) if loss_scale is not None else 1.0 / (G * cfg.n_agents)
-        if flocking is not None:
-            # the tick's reward is the Flocking collective reward; `shaping` f32[B,N,2] is its memory (in / out)
-            if shaping is None:
-                raise ValueError("Flocking needs the shaping buffer f32[B,N,2]")
-            _expect(shaping, torch.float32, cfg.num_envs * cfg.n_agents * 2, "shaping")
-            self._flocking, self._shaping = _lib.SwarmRewardSpec.from_buffer_copy(flocking), shaping   # kept alive
-            h.flocking = C.addressof(self._flocking)
-            h.flocking_shaping = ptr(shaping)
         self.hyper = h
         assert C.sizeof(_lib.SwarmTrainCtl) == 8 * self.CTL_WORDS
         self.ctl = torch.zeros(self.CTL_WORDS, dtype=torch.int64, device=dev)
         self.indices = torch.zeros(G, dtype=torch.int64, device=dev)
-        # gradient and loss share one buffer so that a data-parallel trainer all-reduces both in one collective
-        self.grad_loss = torch.zeros(_lib.W_COUNT + 1, dtype=torch.float32, device=dev)
-        self.grad = self.grad_loss[:_lib.W_COUNT]
-        self.loss = self.grad_loss[_lib.W_COUNT:]
-        gcfg = clone_config(cfg, num_envs=G)
-        self._ws_bytes = int(lib().swarm_dqn_workspace_bytes(C.byref(gcfg), G))
-        self.workspace = torch.empty(max(self._ws_bytes, 256), dtype=torch.uint8, device=dev)
         self._rstruct = ring.struct()
-        self.peers = None          # parallel.PeerExchange: fuse the gradient all-reduce into apply_phase
 
     # -- cursor <-> host bookkeeping ---------------------------------------------------------------
     def load_cursor(self, tick: int, opt_step: int, epsilon: float, episode: int = 0) -> None:
@@ -429,6 +411,39 @@ class TrainTick:
         check(lib().swarm_episode_end(C.byref(self.cfg), ptr(self.ctl), ptr(returns), ptr(hits), ptr(self.loss), ptr(stats),
                                       max_ep, float(epsilon0), float(epsilon_decay), float(min_epsilon),
                                       stream_ptr(returns.device)))
+
+
+class TrainTick(_TrainCursor):
+    """Device-driven train tick (swarm_train_tick_grad / swarm_train_tick_apply): one iteration of the loop body of
+    train_gcn_dqn.py:153-178 for all B envs, with the tick number, replay cursor / fill, optimiser step and epsilon
+    held in a 48-byte device struct that the kernels advance themselves.  No launch argument changes from tick to
+    tick, so ``grad_phase`` / ``apply_phase`` can be captured in a CUDA graph and replayed (``DQNTrainer``)."""
+
+    def __init__(self, cfg: SwarmConfig, ring: ReplayRing, *, graphs_per_update: int = 32, update_target_every: int = 200,
+                 gamma: float = 0.99, loss_scale: Optional[float] = None, lr: float = 1e-3, betas=(0.9, 0.999),
+                 eps: float = 1e-8, max_norm: float = 1.0, rng_seed: int = 0, sample_seed: int = 0, env_offset: int = 0,
+                 flocking: Optional["_lib.SwarmRewardSpec"] = None, shaping: Optional[torch.Tensor] = None):
+        super().__init__(cfg, ring, graphs_per_update, update_target_every, gamma, loss_scale, lr, betas, eps, max_norm,
+                         rng_seed, sample_seed, env_offset)
+        dev = ring.state.device
+        G = int(graphs_per_update)
+        h = self.hyper
+        if flocking is not None:
+            # the tick's reward is the Flocking collective reward; `shaping` f32[B,N,2] is its memory (in / out)
+            if shaping is None:
+                raise ValueError("Flocking needs the shaping buffer f32[B,N,2]")
+            _expect(shaping, torch.float32, cfg.num_envs * cfg.n_agents * 2, "shaping")
+            self._flocking, self._shaping = _lib.SwarmRewardSpec.from_buffer_copy(flocking), shaping   # kept alive
+            h.flocking = C.addressof(self._flocking)
+            h.flocking_shaping = ptr(shaping)
+        # gradient and loss share one buffer so that a data-parallel trainer all-reduces both in one collective
+        self.grad_loss = torch.zeros(_lib.W_COUNT + 1, dtype=torch.float32, device=dev)
+        self.grad = self.grad_loss[:_lib.W_COUNT]
+        self.loss = self.grad_loss[_lib.W_COUNT:]
+        gcfg = clone_config(cfg, num_envs=G)
+        self._ws_bytes = int(lib().swarm_dqn_workspace_bytes(C.byref(gcfg), G))
+        self.workspace = torch.empty(max(self._ws_bytes, 256), dtype=torch.uint8, device=dev)
+        self.peers = None          # parallel.PeerExchange: fuse the gradient all-reduce into apply_phase
 
     # -- the two phases -------------------------------------------------------------------------------
     def grad_phase(self, weights: torch.Tensor, target: torch.Tensor, state: torch.Tensor, returns: torch.Tensor,
@@ -458,6 +473,46 @@ class TrainTick:
                                      ptr(exp_avg), ptr(exp_avg_sq), ptr(state), ptr(returns), ptr(hits),
                                      C.byref(self._rstruct), ptr(self.indices), ptr(self.grad_loss), ptr(self.workspace),
                                      self._ws_bytes, peers, stream_ptr(state.device)))
+
+
+class StackTrainTick(_TrainCursor):
+    """``TrainTick`` for a stacked network (swarm_train_tick_stack): one call per tick runs the rollout tick, the slot
+    draw + gradient, the partial-sum reduce and clip + Adam (+ target sync) with the cursor on the device, so the ticks
+    of an episode capture into a CUDA graph.  ``reward``: None for the world's own reward (GoTo / ObstacleAvoidance), or
+    a Flocking / Cohesion ``reward_spec`` on the GoTo world (Flocking: ``shaping`` f32[B,N,2] is its memory, in / out).
+    One GPU: no phase split, no peer exchange."""
+
+    def __init__(self, cfg: SwarmConfig, spec, ring: ReplayRing, *, graphs_per_update: int = 32,
+                 update_target_every: int = 200, gamma: float = 0.99, loss_scale: Optional[float] = None, lr: float = 1e-3,
+                 betas=(0.9, 0.999), eps: float = 1e-8, max_norm: float = 1.0, rng_seed: int = 0, sample_seed: int = 0,
+                 env_offset: int = 0, reward: Optional["_lib.SwarmRewardSpec"] = None,
+                 shaping: Optional[torch.Tensor] = None):
+        super().__init__(cfg, ring, graphs_per_update, update_target_every, gamma, loss_scale, lr, betas, eps, max_norm,
+                         rng_seed, sample_seed, env_offset)
+        dev = ring.state.device
+        G = int(graphs_per_update)
+        self.spec = spec
+        self._reward = _lib.SwarmRewardSpec.from_buffer_copy(reward) if reward is not None else None    # kept alive
+        self._shaping = shaping
+        if shaping is not None:
+            _expect(shaping, torch.float32, cfg.num_envs * cfg.n_agents * 2, "shaping")
+        self.count = int(lib().swarm_stack_weight_count(C.byref(spec)))
+        self.grad_loss = torch.zeros(self.count + 1, dtype=torch.float32, device=dev)
+        self.grad = self.grad_loss[:self.count]
+        self.loss = self.grad_loss[self.count:]
+        self._ws_bytes = int(lib().swarm_dqn_stack_workspace_bytes(C.byref(cfg), C.byref(spec), G))
+        self.workspace = torch.empty(max(self._ws_bytes, 256), dtype=torch.uint8, device=dev)
+
+    def tick(self, weights: torch.Tensor, target: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor,
+             state: torch.Tensor, returns: torch.Tensor, hits: torch.Tensor) -> None:
+        for name, t in (("weights", weights), ("target", target), ("exp_avg", exp_avg), ("exp_avg_sq", exp_avg_sq)):
+            _expect(t, torch.float32, self.count, name)
+        check(lib().swarm_train_tick_stack(C.byref(self.cfg), C.byref(self.spec), C.byref(self.hyper),
+                                           C.addressof(self._reward) if self._reward is not None else None,
+                                           ptr(self._shaping), ptr(self.ctl), ptr(weights), ptr(target), ptr(exp_avg),
+                                           ptr(exp_avg_sq), ptr(state), ptr(returns), ptr(hits), C.byref(self._rstruct),
+                                           ptr(self.indices), ptr(self.grad_loss), ptr(self.workspace), self._ws_bytes,
+                                           stream_ptr(state.device)))
 
 
 def csr_from_edges(edge_index: torch.Tensor, n_nodes: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:

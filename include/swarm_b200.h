@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SWARM_ABI_VERSION 6
+#define SWARM_ABI_VERSION 7
 
 enum { SWARM_SCENARIO_GOTO = 0, SWARM_SCENARIO_OBSTACLE_AVOIDANCE = 1 };
 /* SWARM_GRAPH_RADIUS is an EXTENSION (the reference has no radius graph, SURVEY.md Appendix C): the complete-graph
@@ -415,6 +415,29 @@ int swarm_train_tick(const SwarmConfig* cfg, const SwarmTrainHyper* hyper, Swarm
                      float* target_weights, float* exp_avg, float* exp_avg_sq, float* state, float* returns,
                      int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
                      int64_t workspace_bytes, const SwarmPeerExchange* peers, void* stream);
+
+/* The same device-driven tick for a stacked network (SwarmStackSpec, below), four launches and no host work, so it
+ * captures into a CUDA graph like swarm_train_tick:
+ *   1. rollout tick of all cfg->num_envs envs with the online weights: swarm_gatstack_forward (argmax), the exploration
+ *      draws of swarm_train_tick_grad (same rng_seed / env_offset stream, epsilon and tick from ctl), the world step,
+ *      the tick's reward, returns / hits accumulated, (s, a, r, s') pushed at slot (ctl->ring_cursor + env) % capacity;
+ *   2. graphs_per_update slots drawn from the filled ring as swarm_train_tick_grad draws them (exported to indices
+ *      int64[G] when indices != NULL), gradient + loss of that batch as swarm_dqn_stack_grad;
+ *   3. the sum of the gradient kernel's per-CTA partials; sets ctl->updating;
+ *   4. swarm_adam_clip_stack_step with the bias corrections from ctl->opt_step + 1, target <- online when
+ *      (ctl->tick + 1) % update_target_every == 0, then ctl advances as in swarm_train_tick_apply.
+ * While the ring holds fewer than G slots, grad / loss are left untouched and ctl->updating = 0.
+ * reward: as for swarm_rollout_stack -- NULL gives the world's own reward (GoTo / ObstacleAvoidance), a Flocking spec
+ * (shaping float[B][N][2] required, read and written back) or a Cohesion spec selects that reward on the GoTo world;
+ * hyper->flocking must be NULL.  grad float[count + 1] = gradient (count = swarm_stack_weight_count(spec)), then the
+ * loss.  2 <= n_agents <= 128, graphs and spec as for swarm_dqn_stack_grad.  workspace:
+ * swarm_dqn_stack_workspace_bytes(cfg, spec, G).  One GPU: there is no two-phase split and no peer exchange. */
+struct SwarmStackSpec;
+int swarm_train_tick_stack(const SwarmConfig* cfg, const struct SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                           const struct SwarmRewardSpec* reward, float* shaping, SwarmTrainCtl* ctl, float* weights,
+                           float* target_weights, float* exp_avg, float* exp_avg_sq, float* state, float* returns,
+                           int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
+                           int64_t workspace_bytes, void* stream);
 
 /* ---- device-side episode boundary (SURVEY.md 8f rank 2) -------------------------------------------------------
  * The reference resets with one CPU torch.normal draw per episode (go_to:84-88, oa:100-102) and does its episode
