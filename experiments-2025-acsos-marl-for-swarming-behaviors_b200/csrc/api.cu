@@ -161,11 +161,7 @@ int fill_params(TileParams& p, const SwarmConfig* cfg, int mode) {
   p.use_tc = (mode == MODE_ROLLOUT || mode == MODE_FORWARD) && !(tc_env && tc_env[0] == '0');
   const char* ord_env = std::getenv("SWARM_KNN_ORDERED");
   p.knn_ordered = (ord_env && ord_env[0] == '1') ? 1 : 0;
-  TileLayout L = tile_layout(mode, kTileThreads, n, cfg->knn_k, p.maxdeg, cfg->graph_mode, p.use_tc != 0);
-  if (L.total > 227 * 1024 && p.use_tc) {
-    p.use_tc = 0;
-    L = tile_layout(mode, kTileThreads, n, cfg->knn_k, p.maxdeg, cfg->graph_mode, false);
-  }
+  const TileLayout L = tile_layout(mode, kTileThreads, n, cfg->knn_k, p.maxdeg, cfg->graph_mode, p.use_tc != 0);
   if (L.total > 227 * 1024) return fail(SWARM_ERR_UNSUPPORTED, "shared-memory tile exceeds 227 KB for this (N, k)");
   return SWARM_OK;
 }

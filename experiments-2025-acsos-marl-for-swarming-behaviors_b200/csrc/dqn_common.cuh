@@ -1,5 +1,5 @@
-// dqn_common.cuh -- parameter block shared by the two DQN gradient kernels (dqn_kernels.cu: CUDA-core parity path,
-// dqn_tc_kernels.cu: tensor-core path) and the Adam element update of the clip + Adam kernels.
+// dqn_common.cuh -- parameter block of the DQN gradient kernel (dqn_tc_kernels.cu, launched from dqn_kernels.cu) and
+// what the device-driven tick and the clip + Adam kernels share.
 #ifndef SWARM_DQN_COMMON_CUH
 #define SWARM_DQN_COMMON_CUH
 
@@ -23,7 +23,6 @@ struct DqnParams {
   float* td;
   int32_t epb, maxdeg;
   float qmax_r;               // radius graph threshold (see TileParams)
-  int32_t parallel;           // 1: target pass and online pass of a transition run side by side on two thread groups
   // device-driven tick (swarm_train_tick_grad): slots are drawn here from the ring fill after this tick's push
   const SwarmTrainCtl* ctl;
   int64_t* indices_out;       // [n_graphs] the drawn slots (exported for tests / logging)

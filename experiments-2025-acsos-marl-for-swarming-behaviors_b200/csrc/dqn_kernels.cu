@@ -1,55 +1,15 @@
-// dqn_kernels.cu -- DQN update on the device: TD target, loss, hand-written backward pass of the GAT
-// Q-network, deterministic gradient reduction, gradient clipping + Adam (train_gcn_dqn.py:112-137).
-//
-// dqn_grad_kernel keeps the env-tile scheme of the rollout (thread = node, CTA = floor(128/N) sampled
-// transitions).  Per transition it runs the target network on s', the online network on s (keeping the
-// activations), the TD error and the backward pass.  Everything a node contributes to another node's
-// gradient goes through shared memory as a *gather* over per-env dense matrices (sum of alpha / d-logit per
-// (target, source) pair), and all weight gradients are tile GEMMs  dW = L^T R  over the CTA's 128 node
-// rows; per-CTA partials are then summed in CTA order by dqn_reduce_kernel.  No atomics anywhere, so the
-// gradient is bit-reproducible from run to run.
+// dqn_kernels.cu -- the rest of the one-layer DQN update on the device (train_gcn_dqn.py:112-137) around the
+// gradient kernel of dqn_tc_kernels.cu:
+//   dqn_reduce_kernel        the per-CTA partial gradients summed in CTA order (no atomics: bit-reproducible)
+//   adam_clip_kernel         clip_grad_norm_ + torch.optim.Adam (+ target copy) in one CTA
+//   reduce_clip_adam_kernel  the two as one thread-block cluster (swarm_train_tick)
+//   csr_bwd_*_kernel         the GCN backward on an arbitrary CSR graph (the nn.Module seam)
+// and the launchers of the whole update.
 #include <cooperative_groups.h>
 
 #include "dqn_common.cuh"
 
 namespace swarm {
-
-struct DqnLayout {
-  int w_on, w_tg, st, h, asrc, wt, wd, inl, kv, ki, nbr, u, r, dp, dob, dh, x, dq, ds, dt, ma, mz, red, total;
-};
-
-__host__ __device__ inline DqnLayout dqn_layout(int n, int k, int maxdeg, int epb, int graph_mode) {
-  const int T = kTileThreads;
-  DqnLayout L;
-  int off = 0;
-  const bool knn = graph_mode == SWARM_GRAPH_KNN;
-  auto take = [&](int bytes) { int o = off; off = tile_align16(off + bytes); return o; };
-  L.w_on = take(TW_COUNT * 4);
-  L.w_tg = take(TW_COUNT * 4);
-  L.st = take(T * 16);
-  L.h = take(T * kHPad * 4);
-  L.asrc = take(T * 4);
-  L.wt = take(maxdeg * T * 4);
-  L.wd = take(maxdeg * T * 4);
-  L.inl = take(maxdeg * T);
-  L.kv = take(knn ? n * T * 4 : 0);
-  L.ki = take(knn ? n * T : 0);
-  L.nbr = take(knn ? k * T : 0);
-  L.u = take(T * kHPad * 4);
-  L.r = take(T * kHPad * 4);
-  L.dp = take(T * kHPad * 4);
-  L.dob = take(T * kHPad * 4);
-  L.dh = take(T * kHPad * 4);
-  L.x = take(T * kXPad * 4);
-  L.dq = take(T * kW2Pad * 4);
-  L.ds = take(T * 4);
-  L.dt = take(T * 4);
-  L.ma = take(epb * n * n * 4);
-  L.mz = take(epb * n * n * 4);
-  L.red = take(T * 4);
-  L.total = off;
-  return L;
-}
 
 __device__ __forceinline__ void store_row32(float* tile, int row, const float (&v)[32]) {
   float4* r = reinterpret_cast<float4*>(tile + row * kHPad);
@@ -151,323 +111,6 @@ __device__ __forceinline__ void dqn_head(const float (&agg)[32], float* __restri
   const float* b2 = sw + TW_B2;
 #pragma unroll
   for (int a = 0; a < 9; ++a) q[a] = __fadd_rn(qq[a], b2[a]);
-}
-
-__global__ void __launch_bounds__(kTileThreads) dqn_grad_kernel(const __grid_constant__ DqnParams p) {
-  extern __shared__ __align__(16) unsigned char smem[];
-  const SwarmConfig& c = p.cfg;
-  const int T = kTileThreads;
-  const int N = c.n_agents;
-  const int K = c.knn_k;
-  const bool knn = c.graph_mode == SWARM_GRAPH_KNN;
-  const bool radius = c.graph_mode == SWARM_GRAPH_RADIUS;
-  // Thread groups: el in [0, epb) runs the online network on s (and the backward pass); in `parallel` mode
-  // el in [epb, 2 epb) runs the target network on s' of transition el - epb at the same time, otherwise the online
-  // group runs both passes one after the other.
-  TileThread t = tile_thread(N, p.parallel ? 2 * p.epb : p.epb, p.n_graphs);
-  const int tid = t.tid;
-  const bool tgt_group = p.parallel && t.el >= p.epb;
-  {
-    const int gl = tgt_group ? t.el - p.epb : t.el;
-    t.env = (long long)blockIdx.x * p.epb + gl;
-    t.active = (t.el < (p.parallel ? 2 * p.epb : p.epb)) && (t.env < p.n_graphs);
-    t.gidx = t.env * N + t.i;
-  }
-  long long ring_size = 0;
-  if (p.ctl) {
-    ring_size = train_ring_size(p.ctl, p.pushed_envs, p.batch.capacity);
-    if (ring_size < p.n_graphs) return;        // replay ring not filled yet (train:113-115)
-  }
-
-  const DqnLayout L = dqn_layout(N, K, p.maxdeg, p.epb, c.graph_mode);
-  float* sw_on = reinterpret_cast<float*>(smem + L.w_on);
-  float* sw_tg = reinterpret_cast<float*>(smem + L.w_tg);
-  float4* sst = reinterpret_cast<float4*>(smem + L.st);
-  TileGraphSmem g;
-  g.sh = reinterpret_cast<float*>(smem + L.h);
-  g.sas = reinterpret_cast<float*>(smem + L.asrc);
-  g.swt = reinterpret_cast<float*>(smem + L.wt);
-  g.sin = smem + L.inl;
-  g.skv = reinterpret_cast<float*>(smem + L.kv);
-  g.ski = smem + L.ki;
-  g.snbr = smem + L.nbr;
-  float* swd = reinterpret_cast<float*>(smem + L.wd);
-  float* tU = reinterpret_cast<float*>(smem + L.u);
-  float* tR = reinterpret_cast<float*>(smem + L.r);
-  float* tDP = reinterpret_cast<float*>(smem + L.dp);
-  float* tDO = reinterpret_cast<float*>(smem + L.dob);
-  float* tDH = reinterpret_cast<float*>(smem + L.dh);
-  float* tX = reinterpret_cast<float*>(smem + L.x);
-  float* tDQ = reinterpret_cast<float*>(smem + L.dq);
-  float* sds = reinterpret_cast<float*>(smem + L.ds);
-  float* sdt = reinterpret_cast<float*>(smem + L.dt);
-  float* mA = reinterpret_cast<float*>(smem + L.ma);
-  float* mZ = reinterpret_cast<float*>(smem + L.mz);
-  float* sred = reinterpret_cast<float*>(smem + L.red);
-  const int rows = p.epb * N;                  // node rows of this CTA that can be non-zero (online group)
-
-  stage_weights(p.w_online, sw_on, tid, T);
-  stage_weights(p.w_target, sw_tg, tid, T);
-
-  float4 s = make_float4(0.f, 0.f, 0.f, 0.f), s2 = s;
-  int act = 0;
-  float rew = 0.0f;
-  if (t.active) {
-    long long slot = t.env;
-    if (p.ctl) {
-      // GraphReplayBuffer.sample's index draw (train:38-39) on the device: slot ~ U{0 .. ring_size - 1}, counter RNG
-      // keyed by (sample_seed, tick, graph)
-      const uint64_t rnd = rng_draw(p.sample_seed, (uint64_t)t.env, (uint64_t)(p.ctl->tick + 1), 0x5A17u);
-      slot = (long long)__umul64hi(rnd, (uint64_t)ring_size);
-      if (p.indices_out && t.i == 0 && !tgt_group) p.indices_out[t.env] = slot;
-    } else if (p.indices) {
-      slot = p.indices[t.env];                            // caller-supplied: clamped into the ring, never out of bounds
-      slot = slot < 0 ? 0 : (slot >= p.batch.capacity ? p.batch.capacity - 1 : slot);
-    }
-    const long long ri = slot * N + t.i;
-    s = reinterpret_cast<const float4*>(p.batch.state)[ri];
-    s2 = reinterpret_cast<const float4*>(p.batch.next_state)[ri];
-    act = sanitize_action(p.batch.actions[ri]);
-    rew = p.batch.rewards[ri];
-  } else if (tid < rows) {
-    // rows of idle threads inside the row range take part in the tile GEMMs below: exact zeros
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    float* tiles[6] = {g.sh, tU, tR, tDP, tDO, tDH};
-#pragma unroll 1
-    for (int b = 0; b < 6; ++b) {
-      float4* row = reinterpret_cast<float4*>(tiles[b] + tid * kHPad);
-#pragma unroll
-      for (int c4 = 0; c4 < 8; ++c4) row[c4] = z;
-    }
-    reinterpret_cast<float4*>(tX + tid * kXPad)[0] = z;
-    reinterpret_cast<float4*>(tX + tid * kXPad)[1] = z;
-#pragma unroll
-    for (int a = 0; a < kW2Pad; ++a) tDQ[tid * kW2Pad + a] = 0.0f;
-  }
-
-  int deg = 0;
-  if (!knn && !radius && t.active) deg = tile_in_edges_complete(g, t, N);
-  float agg[32], r[32];
-  float adst = 0.0f, y = 0.0f, delta = 0.0f, dq = 0.0f;
-
-  // target network on s' -> y = r + gamma * max_a Q_target(s')  (train:120-121);
-  // online network on s, activations kept                        (train:119)
-  // sequential mode: pass 0 = target, pass 1 = online on the same threads; parallel mode: one pass, the role is the
-  // thread group's
-  const int npass = p.parallel ? 1 : 2;
-#pragma unroll 1
-  for (int pass = 0; pass < npass; ++pass) {
-    const bool target_role = p.parallel ? tgt_group : (pass == 0);
-    const float4 sp = target_role ? s2 : s;
-    const float* sw = target_role ? sw_tg : sw_on;
-    __syncthreads();                              // weights staged / previous pass done with sst and the h tile
-    sst[tid] = sp;
-    __syncthreads();
-    if (knn && N <= kKnnSmallMax) {
-      uint64_t cache_rank = ~0ull, cache_nbr = 0;
-      const uint64_t nbr_word = tile_knn_small(t, sst, sp, N, K, cache_rank, cache_nbr);
-      deg = tile_in_edges_knn_small(g, t, N, K, nbr_word, reinterpret_cast<uint32_t*>(g.skv));
-    } else if (knn) {
-      tile_knn_rows(g, t, sst, sp, N, K);
-      deg = tile_in_edges_knn(g, t, N, K, reinterpret_cast<uint32_t*>(g.skv));   // distance rows are dead now
-    } else if (radius && t.active) {
-      deg = tile_in_edges_radius(g, t, sst, sp, N, p.qmax_r);
-    }
-    const float x[7] = {sp.x, sp.y, sp.z, sp.w, c.goal_x, c.goal_y, (float)t.i};
-    tile_gat_conv(g, t, sw, x, deg, agg, adst);   // alpha_e in g.swt, h rows in g.sh, alpha_src in g.sas
-    if (t.active) {
-      float q[9];
-      dqn_head(agg, tU + tid * kHPad, tR + tid * kHPad, sw, r, q);
-      if (target_role) {
-        float qmax = q[0];
-#pragma unroll
-        for (int a = 1; a < 9; ++a) qmax = fmaxf(qmax, q[a]);
-        y = __fadd_rn(rew, __fmul_rn(p.gamma, qmax));
-        if (p.parallel) sds[tid] = y;             // handed to the online thread of the same node below
-      } else {
-        float v = q[0];
-#pragma unroll
-        for (int a = 1; a < 9; ++a) v = (act == a) ? q[a] : v;        // values = Q(s).gather(1, a)  (train:119)
-        delta = v;                                                    // minus y below
-        float4* xr = reinterpret_cast<float4*>(tX + tid * kXPad);
-        xr[0] = make_float4(x[0], x[1], x[2], x[3]);
-        xr[1] = make_float4(x[4], x[5], x[6], 0.f);
-      }
-    }
-  }
-  if (p.parallel) {
-    __syncthreads();
-    if (t.active && !tgt_group) y = sds[tid + rows];
-    __syncthreads();                              // sds is reused for d alpha_src below
-  }
-  const bool learner = t.active && !tgt_group;    // threads that own a node of the online pass
-  if (learner) {
-    delta = __fsub_rn(delta, y);
-    dq = 2.0f * delta * p.loss_scale;             // d mean((v - y)^2) / dv
-    if (p.td) p.td[t.gidx] = delta;
-  } else {
-    delta = 0.0f;
-  }
-  const float* sw = sw_on;
-  sred[tid] = delta * delta;
-
-  float dvec[32];
-#pragma unroll
-  for (int k = 0; k < 32; ++k) dvec[k] = 0.0f;
-  float dt_i = 0.0f;
-  if (learner) {
-    float* dqr = tDQ + tid * kW2Pad;
-#pragma unroll
-    for (int a = 0; a < kW2Pad; ++a) dqr[a] = (a == act) ? dq : 0.0f;
-
-    // ---------------- backward: lin2 -> ReLU -> lin1 -> tanh ------------------------------------------
-    // dr = W2[a,:]^T dq ; dp = dr * [r > 0]
-#pragma unroll
-    for (int k = 0; k < 32; ++k) {
-      const float dr = sw[TW_W2T + k * kW2Pad + act] * dq;
-      dvec[k] = r[k] > 0.0f ? dr : 0.0f;
-    }
-    store_row32(tDP, tid, dvec);
-    // du[k] = sum_c W1[c][k] dp[c] ; do = du * (1 - u^2), four k per iteration through the own rows
-    {
-      const float4* w1 = reinterpret_cast<const float4*>(sw + TW_W1T);
-      const float4* u4 = reinterpret_cast<const float4*>(tU + tid * kHPad);
-      float4* do4 = reinterpret_cast<float4*>(tDO + tid * kHPad);
-#pragma unroll 1
-      for (int k4 = 0; k4 < 8; ++k4) {
-        const float4 uk = u4[k4];
-        float o[4];
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk) {
-          float acc = 0.0f;
-#pragma unroll
-          for (int c4 = 0; c4 < 8; ++c4) {
-            const float4 w = w1[(k4 * 4 + kk) * 8 + c4];
-            acc = fmaf(w.x, dvec[4 * c4 + 0], acc);
-            acc = fmaf(w.y, dvec[4 * c4 + 1], acc);
-            acc = fmaf(w.z, dvec[4 * c4 + 2], acc);
-            acc = fmaf(w.w, dvec[4 * c4 + 3], acc);
-          }
-          const float uu = f4c(uk, kk);
-          o[kk] = acc * (1.0f - uu * uu);
-        }
-        do4[k4] = make_float4(o[0], o[1], o[2], o[3]);
-      }
-      load_row32(tDO, tid, dvec);                   // dvec = d(out_i) from here on
-    }
-
-    // ---------------- backward: aggregation + edge softmax + LeakyReLU ----------------------------------
-    float* ra = mA + (t.el * N + t.i) * N;
-    float* rz = mZ + (t.el * N + t.i) * N;
-    for (int j = 0; j < N; ++j) { ra[j] = 0.0f; rz[j] = 0.0f; }
-    // d alpha_e = <d out_i, h_j> ; softmax backward: d z_e = alpha_e (d alpha_e - sum_e' alpha_e' d alpha_e')
-    float dot_sum = 0.0f;
-    for (int e = 0; e < deg; ++e) {
-      const int j = g.sin[e * T + tid];
-      const float4* hj = reinterpret_cast<const float4*>(g.sh + (t.envbase + j) * kHPad);
-      float da = 0.0f;
-#pragma unroll
-      for (int c4 = 0; c4 < 8; ++c4) {
-        const float4 hv = hj[c4];
-        da = fmaf(dvec[4 * c4 + 0], hv.x, da);
-        da = fmaf(dvec[4 * c4 + 1], hv.y, da);
-        da = fmaf(dvec[4 * c4 + 2], hv.z, da);
-        da = fmaf(dvec[4 * c4 + 3], hv.w, da);
-      }
-      swd[e * T + tid] = da;
-      dot_sum = fmaf(g.swt[e * T + tid], da, dot_sum);
-    }
-    for (int e = 0; e < deg; ++e) {
-      const int j = g.sin[e * T + tid];
-      const float alpha = g.swt[e * T + tid];
-      const float dz = alpha * (swd[e * T + tid] - dot_sum);
-      const float raw = __fadd_rn(g.sas[t.envbase + j], adst);
-      const float dzz = raw > 0.0f ? dz : 0.2f * dz;
-      ra[j] += alpha;         // parallel edges (duplicates, double self loops) accumulate
-      rz[j] += dzz;
-      dt_i += dzz;
-    }
-  }
-  sdt[tid] = dt_i;
-  __syncthreads();            // tDO, mA, mZ complete
-
-  // gather in the source role:  d h_j = sum_i A[i][j] d out_i + ds_j att_src + dt_j att_dst
-  {
-    float ds_j = 0.0f;
-    if (learner) {
-      float dh[32];
-#pragma unroll
-      for (int k = 0; k < 32; ++k) dh[k] = 0.0f;
-      for (int ii = 0; ii < N; ++ii) {
-        const float a = mA[(t.el * N + ii) * N + t.i];
-        ds_j += mZ[(t.el * N + ii) * N + t.i];
-        const float4* dr = reinterpret_cast<const float4*>(tDO + (t.envbase + ii) * kHPad);
-#pragma unroll
-        for (int c4 = 0; c4 < 8; ++c4) {
-          const float4 dv = dr[c4];
-          dh[4 * c4 + 0] = fmaf(a, dv.x, dh[4 * c4 + 0]);
-          dh[4 * c4 + 1] = fmaf(a, dv.y, dh[4 * c4 + 1]);
-          dh[4 * c4 + 2] = fmaf(a, dv.z, dh[4 * c4 + 2]);
-          dh[4 * c4 + 3] = fmaf(a, dv.w, dh[4 * c4 + 3]);
-        }
-      }
-      const float* as = sw + TW_ATT_S;
-      const float* ad = sw + TW_ATT_D;
-#pragma unroll
-      for (int k = 0; k < 32; ++k) dh[k] = fmaf(ds_j, as[k], fmaf(dt_i, ad[k], dh[k]));
-      store_row32(tDH, tid, dh);
-    }
-    sds[tid] = ds_j;
-  }
-  __syncthreads();            // every tile complete
-
-  // ---------------- weight gradients: tile GEMMs over the CTA's node rows ------------------------------
-  float* out = p.partials + (long long)blockIdx.x * kPartialStride;
-  constexpr int G_W0 = 64, G_AS = 8, G_AD = 8, G_B0 = 8, G_W1 = 256, G_B1 = 8, G_W2 = 72, G_B2 = 3;
-  constexpr int G_TOTAL = G_W0 + G_AS + G_AD + G_B0 + G_W1 + G_B1 + G_W2 + G_B2;
-#pragma unroll 1
-  for (int grp = tid; grp < G_TOTAL; grp += T) {
-    int gi = grp;
-    if (gi < G_W0) {                                   // dW0[c][k] = sum_n DH[n][c] X[n][k]
-      const int cc = gi >> 1, k4 = (gi & 1) * 4;
-      const float4 a = tile_gemm4(tDH, kHPad, cc, tX, kXPad, k4, rows);
-      float* o = out + SWARM_W_CONV_LIN + cc * 7 + k4;
-      o[0] = a.x; o[1] = a.y; o[2] = a.z;
-      if (k4 == 0) o[3] = a.w;
-      continue;
-    }
-    gi -= G_W0;
-    // the remaining groups all write four consecutive outputs of one packed tensor
-    const float* A = nullptr;
-    const float* Bm;
-    int lda = 0, ac = 0, ldb = kHPad, bc, oidx, nout = 4;
-    if (gi < G_AS) {                                   // d att_src[c] = sum_n ds[n] H[n][c]
-      A = sds; lda = 1; Bm = g.sh; bc = gi * 4; oidx = SWARM_W_ATT_SRC + gi * 4;
-    } else if ((gi -= G_AS) < G_AD) {                  // d att_dst[c] = sum_n dt[n] H[n][c]
-      A = sdt; lda = 1; Bm = g.sh; bc = gi * 4; oidx = SWARM_W_ATT_DST + gi * 4;
-    } else if ((gi -= G_AD) < G_B0) {                  // d conv1.bias[c] = sum_n DO[n][c]
-      Bm = tDO; bc = gi * 4; oidx = SWARM_W_CONV_BIAS + gi * 4;
-    } else if ((gi -= G_B0) < G_W1) {                  // dW1[c][k] = sum_n DP[n][c] U[n][k]
-      A = tDP; lda = kHPad; ac = gi >> 3; Bm = tU; bc = (gi & 7) * 4; oidx = SWARM_W_LIN1 + ac * 32 + bc;
-    } else if ((gi -= G_W1) < G_B1) {                  // d lin1.bias[c] = sum_n DP[n][c]
-      Bm = tDP; bc = gi * 4; oidx = SWARM_W_LIN1_BIAS + gi * 4;
-    } else if ((gi -= G_B1) < G_W2) {                  // dW2[a][k] = sum_n DQ[n][a] R[n][k]
-      A = tDQ; lda = kW2Pad; ac = gi >> 3; Bm = tR; bc = (gi & 7) * 4; oidx = SWARM_W_LIN2 + ac * 32 + bc;
-    } else {                                           // d lin2.bias[a] = sum_n DQ[n][a]
-      gi -= G_W2;
-      Bm = tDQ; ldb = kW2Pad; bc = gi * 4; oidx = SWARM_W_LIN2_BIAS + gi * 4;
-      nout = gi < 2 ? 4 : 1;
-    }
-    const float4 a = tile_gemm4(A, lda, ac, Bm, ldb, bc, rows);
-    float* o = out + oidx;
-    o[0] = a.x;
-    if (nout == 4) { o[1] = a.y; o[2] = a.z; o[3] = a.w; }
-  }
-  if (tid == 0) {
-    float sse = 0.0f;
-    for (int n = 0; n < rows; ++n) sse += sred[n];
-    out[SWARM_W_COUNT] = sse;
-  }
 }
 
 // grad[o] = sum over CTAs (in CTA order) of partials[cta][o]; loss = loss_scale * sum of squared TD errors
@@ -1210,7 +853,7 @@ int dqn_maxdeg(const SwarmConfig& c) {
 }
 
 // graphs per CTA: as many as fit (floor(128/N)) for big batches, fewer for small ones so that the update spreads over
-// the SMs (G = 32 -> one graph per CTA) and the tile GEMMs only walk the rows that exist
+// the SMs (G = 32 -> one graph per CTA) and the node contractions only walk the rows that exist
 int dqn_epb(const SwarmConfig& c, int n_graphs) {
   const int full = kTileThreads / c.n_agents;
   int epb = (n_graphs + 147) / 148;
@@ -1224,18 +867,7 @@ long long dqn_workspace_bytes(const SwarmConfig& c, int n_graphs) {
   return ctas * kPartialStride * 4 + 256;
 }
 
-bool dqn_tc_enabled();
-int dqn_tc_smem_bytes(const SwarmConfig& c);
 cudaError_t launch_dqn_grad_tc(DqnParams& p, cudaStream_t stream);
-
-// the tensor-core kernel (dqn_tc_kernels.cu) unless SWARM_TC=0 or its tile does not fit shared memory
-static bool dqn_use_tc(const SwarmConfig& c) { return dqn_tc_enabled() && dqn_tc_smem_bytes(c) <= 227 * 1024; }
-
-int dqn_smem_bytes(const SwarmConfig& c) {
-  if (dqn_use_tc(c)) return dqn_tc_smem_bytes(c);
-  const int epb = kTileThreads / c.n_agents;
-  return dqn_layout(c.n_agents, c.knn_k, dqn_maxdeg(c), epb, c.graph_mode).total;
-}
 
 cudaError_t launch_dqn_grad(const SwarmConfig& c, const float* w_online, const float* w_target, const SwarmReplay& batch,
                             const int64_t* indices, int n_graphs, float gamma, float loss_scale, float* grad, float* loss,
@@ -1258,19 +890,10 @@ cudaError_t launch_dqn_grad(const SwarmConfig& c, const float* w_online, const f
   p.td = td;
   p.qmax_r = sq_threshold(c.graph_radius);
   p.epb = dqn_epb(c, n_graphs);
-  p.parallel = (2 * p.epb * c.n_agents <= kTileThreads) ? 1 : 0;
   p.maxdeg = dqn_maxdeg(c);
   const int ctas = (n_graphs + p.epb - 1) / p.epb;
-  cudaError_t err;
-  if (dqn_use_tc(c)) {
-    err = launch_dqn_grad_tc(p, stream);
-    if (err != cudaSuccess) return err;
-  } else {
-    const int smem = dqn_layout(c.n_agents, c.knn_k, p.maxdeg, p.epb, c.graph_mode).total;
-    err = cudaFuncSetAttribute(dqn_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (err != cudaSuccess) return err;
-    dqn_grad_kernel<<<ctas, kTileThreads, smem, stream>>>(p);
-  }
+  cudaError_t err = launch_dqn_grad_tc(p, stream);
+  if (err != cudaSuccess) return err;
   // skip_reduce: the caller sums the partials inside launch_reduce_clip_adam
   if (!skip_reduce)
     dqn_reduce_kernel<<<(SWARM_W_COUNT + 1 + 255) / 256, 256, 0, stream>>>(p.partials, ctas, loss_scale, grad, loss, ctl,

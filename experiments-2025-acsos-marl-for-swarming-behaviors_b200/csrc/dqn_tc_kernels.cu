@@ -17,10 +17,8 @@
 //               staging tiles (__syncwarp only), column sums give the bias gradients, and the attention vectors get
 //               theirs through v = W0^T att:  d att = W0 dv,  dW0 += att (x) dv  with  dv_s = sum_j d alpha_src_j x_j.
 //               The four warp partials are added in warp order.
-// One transition set costs ~3 k instructions per warp instead of ~19 k on the CUDA-core kernel (dqn_kernels.cu, which
-// stays as the SWARM_TC=0 parity path), and the CTA needs 2 x 5 KB of staging per warp instead of six 18 KB tiles.
-#include <cstdlib>
-
+// One transition set costs ~3 k instructions per warp instead of ~19 k on a CUDA-core kernel of the same scheme, and
+// the CTA needs 2 x 5 KB of staging per warp instead of six 18 KB tiles.
 #include "dqn_common.cuh"
 #include "tile_tc_device.cuh"
 
@@ -762,20 +760,14 @@ __global__ void __launch_bounds__(kTileThreads, 2) dqn_grad_tc_kernel(const __gr
 }
 
 int dqn_maxdeg(const SwarmConfig& c);
-int dqn_epb(const SwarmConfig& c, int n_graphs);
 
-bool dqn_tc_enabled() {
-  static const char* tc_env = std::getenv("SWARM_TC");
-  return !(tc_env && tc_env[0] == '0');
-}
-
-int dqn_tc_smem_bytes(const SwarmConfig& c) {
+// the largest tile (floor(128 / N) transitions per CTA) that launch_dqn_grad_tc can ask for
+int dqn_smem_bytes(const SwarmConfig& c) {
   return dqn_tc_layout(c.n_agents, c.knn_k, dqn_maxdeg(c), kTileThreads / c.n_agents, c.graph_mode).total;
 }
 
 cudaError_t launch_dqn_grad_tc(DqnParams& p, cudaStream_t stream) {
   const SwarmConfig& c = p.cfg;
-  p.parallel = 0;
   const int smem = dqn_tc_layout(c.n_agents, c.knn_k, p.maxdeg, p.epb, c.graph_mode).total;
   const int ctas = (p.n_graphs + p.epb - 1) / p.epb;
   cudaError_t err;

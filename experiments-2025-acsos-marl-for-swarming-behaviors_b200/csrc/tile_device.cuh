@@ -1,6 +1,6 @@
 // tile_device.cuh -- device functions of the env-tile scheme (thread = agent, CTA = floor(128/N) envs),
 // shared by the rollout / forward / graph kernels (tile_kernels.cu) and the DQN gradient kernel
-// (dqn_kernels.cu).
+// (dqn_tc_kernels.cu).
 #ifndef SWARM_TILE_DEVICE_CUH
 #define SWARM_TILE_DEVICE_CUH
 
@@ -463,8 +463,8 @@ __device__ __forceinline__ void tile_gat_publish(const TileGraphSmem& g, const T
 
 // Edge softmax over the in-edge list of this node in edge-list order (torch_geometric.utils.softmax: max,
 // exp(z - max), sum + 1e-16, divide) followed by the aggregation.  On return agg = sum_e alpha_e h_j (bias not yet
-// added); the parity path (FUSED = false) also leaves the attention coefficients alpha_e in g.swt[e][tid] (read by
-// the DQN backward pass).
+// added); the parity path (FUSED = false) also leaves the attention coefficients alpha_e in g.swt[e][tid], which no
+// caller reads.
 template <bool FUSED = false>
 __device__ __forceinline__ void tile_gat_attend(const TileGraphSmem& g, const TileThread& t, int deg, float adst,
                                                 float (&agg)[32]) {

@@ -4,6 +4,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -185,6 +186,29 @@ def test_training_argument_validation_without_device(sb):
     assert lib.swarm_reset_random(C.byref(cfg), C.byref(sp), None, -1, None, 8, None) == -1
     assert lib.swarm_episode_end(C.byref(cfg), None, 8, None, None, None, 0, 0.9, 0.01, 0.05, None) == -1
     assert lib.swarm_episode_end(C.byref(cfg), 8, 8, None, None, 8, 0, 0.9, 0.01, 0.05, None) == -1     # stats without rows
+
+
+def _largest_dqn_agents():
+    """Largest n_agents that swarm_dqn_workspace_bytes(cfg, 32) accepts: complete, radius, kNN k = 5, kNN k = 10."""
+    import swarm_b200 as sb
+    lib, L = sb._lib.lib(), sb._lib
+    out = []
+    for graph, k in ((L.GRAPH_COMPLETE, 1), (L.GRAPH_RADIUS, 1), (L.GRAPH_KNN, 5), (L.GRAPH_KNN, 10)):
+        ok = [n for n in range(k, 129)
+              if lib.swarm_dqn_workspace_bytes(C.byref(sb.ops.make_config(L.SCENARIO_GOTO, 1, n, graph, k)), 32) > 0]
+        out.append(max(ok))
+    return out
+
+
+def test_dqn_accepts_the_same_swarm_sizes_with_and_without_swarm_tc(sb):
+    # the DQN gradient has one kernel: SWARM_TC=0 selects the bit-faithful forward only and leaves these limits alone
+    # (checked in a child process started with the variable set, so no cached read of the environment can hide it)
+    expected = [128, 120, 81, 79]
+    assert _largest_dqn_agents() == expected
+    code = f"import sys; sys.path[:0] = {[ROOT, os.path.dirname(__file__)]!r}; import test_abi; print(test_abi._largest_dqn_agents())"
+    child = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, SWARM_TC="0"), capture_output=True, text=True,
+                           check=True)
+    assert child.stdout.strip().splitlines()[-1] == str(expected)
 
 
 def test_reward_spec_layout_defaults_and_validation(sb, tmp_path):
