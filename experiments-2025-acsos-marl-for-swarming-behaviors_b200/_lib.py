@@ -22,7 +22,7 @@ FLAG_OBSTACLE_CONTACT = 1
 FLAG_HIT = 2
 FLAG_PENALTY = 4
 W_COUNT = 1673
-ABI_VERSION = 7
+ABI_VERSION = 8
 XCHG_STRIDE = 1680
 
 # state-dict tensors in packed order (include/swarm_b200.h SWARM_W_*)
@@ -127,6 +127,10 @@ _SIGNATURES = {
     "swarm_rollout_stack_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig)]),
     "swarm_rollout_stack": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p, C.c_int32,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "swarm_rollout_stack_large_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig), C.c_void_p]),
+    "swarm_rollout_stack_large": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p,
+                                            C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_int64, C.c_void_p]),
     "swarm_dqn_stack_workspace_bytes": (C.c_int64, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_int32]),
     "swarm_dqn_stack_grad": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.c_void_p, C.c_void_p,
                                        C.POINTER(SwarmReplay), C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_void_p,
@@ -170,6 +174,8 @@ _SIGNATURES = {
                               + [C.POINTER(SwarmReplay)] + [C.c_void_p] * 4 + [C.c_int64, C.c_void_p]),
     "swarm_default_reward_spec": (None, [C.POINTER(SwarmRewardSpec), C.c_int32, C.c_int32, C.c_int32]),
     "swarm_scenario_reward": (C.c_int, [C.POINTER(SwarmRewardSpec)] + [C.c_void_p] * 5),
+    "swarm_scenario_reward_large_workspace_bytes": (C.c_int64, [C.POINTER(SwarmRewardSpec)]),
+    "swarm_scenario_reward_large": (C.c_int, [C.POINTER(SwarmRewardSpec)] + [C.c_void_p] * 5 + [C.c_int64, C.c_void_p]),
     "swarm_reset_random": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmResetSpec), C.c_void_p, C.c_int64,
                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "swarm_episode_end": (C.c_int, [C.POINTER(SwarmConfig)] + [C.c_void_p] * 5 + [C.c_int64, C.c_double, C.c_double,

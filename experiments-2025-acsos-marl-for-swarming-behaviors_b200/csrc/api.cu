@@ -26,6 +26,9 @@ cudaError_t launch_gat_layer_backward(int n, long long E, int ci, int co, const 
                                       float* gb, float* grad_x, void* workspace, cudaStream_t stream);
 cudaError_t launch_scenario_reward(const SwarmRewardSpec& sp, const float* state, float* shaping, float* reward,
                                    float* terms, cudaStream_t stream);
+long long scenario_reward_large_workspace_bytes(const SwarmRewardSpec& sp);
+cudaError_t launch_scenario_reward_large(const SwarmRewardSpec& sp, const float* state, float* shaping, float* reward,
+                                         float* terms, float* returns, void* workspace, cudaStream_t stream);
 cudaError_t launch_reset_random(const SwarmConfig& c, const SwarmResetSpec& sp, int cols, int rows, const SwarmTrainCtl* ctl,
                                 long long episode, float* centers_out, float* state, cudaStream_t stream);
 cudaError_t launch_episode_end(const SwarmConfig& c, SwarmTrainCtl* ctl, float* returns, int32_t* hits, const float* loss,
@@ -786,19 +789,28 @@ void swarm_default_reward_spec(SwarmRewardSpec* spec, int32_t kind, int32_t num_
   spec->sigma = 0.15f;
 }
 
-int swarm_scenario_reward(const SwarmRewardSpec* spec, const float* state, float* shaping, float* reward, float* terms,
-                          void* stream) {
+namespace {
+// the argument checks of the scenario rewards up to the num_envs * n_agents bound; large = false: the env-tile kernel
+// (n_agents <= 128), true: the large-swarm kernel (n_agents <= 4096)
+int validate_reward_spec(const SwarmRewardSpec* spec, bool large) {
   if (!spec) return fail(SWARM_ERR_INVALID_ARG, "spec is NULL");
   if (spec->kind != SWARM_REWARD_FLOCKING && spec->kind != SWARM_REWARD_COHESION)
     return fail(SWARM_ERR_INVALID_ARG, "unknown reward kind");
   if (spec->num_envs < 0) return fail(SWARM_ERR_INVALID_ARG, "num_envs must be >= 0");
   if (spec->n_agents < 2) return fail(SWARM_ERR_INVALID_ARG, "the scenario rewards need at least two agents");
-  if (spec->n_agents > 128) return fail(SWARM_ERR_UNSUPPORTED, "scenario rewards are implemented for n_agents <= 128");
+  if (!large && spec->n_agents > 128)
+    return fail(SWARM_ERR_UNSUPPORTED, "scenario rewards are implemented for n_agents <= 128");
+  if (large && spec->n_agents > kMaxLargeAgents)
+    return fail(SWARM_ERR_UNSUPPORTED, "the large-swarm scenario rewards are implemented for n_agents <= 4096");
   if (spec->env_index < -1 || spec->env_index >= spec->num_envs)
     return fail(SWARM_ERR_INVALID_ARG, "env_index out of range");
-  if ((int64_t)spec->num_envs * spec->n_agents + 128 * 148 * 16 >= (1LL << 31))
+  if ((int64_t)spec->num_envs * spec->n_agents + (large ? 0 : 128 * 148 * 16) >= (1LL << 31))
     return fail(SWARM_ERR_UNSUPPORTED, "num_envs * n_agents must stay below 2^31");
-  if (spec->num_envs == 0) return SWARM_OK;
+  return SWARM_OK;
+}
+
+// the buffer checks of a call with num_envs > 0
+int validate_reward_buffers(const SwarmRewardSpec* spec, const float* state, const float* shaping, const float* reward) {
   if (!state) return fail(SWARM_ERR_INVALID_ARG, "state is NULL");
   if (spec->kind == SWARM_REWARD_FLOCKING) {
     if (!shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
@@ -808,8 +820,35 @@ int swarm_scenario_reward(const SwarmRewardSpec* spec, const float* state, float
     if (!reward) return fail(SWARM_ERR_INVALID_ARG, "reward is NULL");
     if (!(spec->sigma > 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "sigma must be > 0");
   }
+  return SWARM_OK;
+}
+}  // namespace
+
+int swarm_scenario_reward(const SwarmRewardSpec* spec, const float* state, float* shaping, float* reward, float* terms,
+                          void* stream) {
+  if (int rc = validate_reward_spec(spec, false)) return rc;
+  if (spec->num_envs == 0) return SWARM_OK;
+  if (int rc = validate_reward_buffers(spec, state, shaping, reward)) return rc;
   return check_cuda(launch_scenario_reward(*spec, state, shaping, reward, terms, (cudaStream_t)stream),
                     "swarm_scenario_reward");
+}
+
+int64_t swarm_scenario_reward_large_workspace_bytes(const SwarmRewardSpec* spec) {
+  if (validate_reward_spec(spec, true) != SWARM_OK) return 0;
+  return scenario_reward_large_workspace_bytes(*spec);
+}
+
+int swarm_scenario_reward_large(const SwarmRewardSpec* spec, const float* state, float* shaping, float* reward,
+                                float* terms, void* workspace, int64_t workspace_bytes, void* stream) {
+  if (int rc = validate_reward_spec(spec, true)) return rc;
+  if (spec->num_envs == 0) return SWARM_OK;
+  if (int rc = validate_reward_buffers(spec, state, shaping, reward)) return rc;
+  const int64_t need = scenario_reward_large_workspace_bytes(*spec);
+  if (need > 0 && !workspace) return fail(SWARM_ERR_INVALID_ARG, "workspace is NULL");
+  if (workspace_bytes < need) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  return check_cuda(launch_scenario_reward_large(*spec, state, shaping, reward, terms, nullptr, workspace,
+                                                 (cudaStream_t)stream),
+                    "swarm_scenario_reward_large");
 }
 
 namespace {
@@ -957,9 +996,12 @@ static int stack_reward(const SwarmConfig* cfg, const SwarmRewardSpec* reward, c
   return SWARM_OK;
 }
 
-// n_agents > 128: per tick [topk table ->] the large stacked forward (argmax) -> the large world step with returns / hits
+// n_agents > 128: per tick [topk table ->] the large stacked forward (argmax) -> the large world step with returns / hits;
+// rs != nullptr: the world step counts the hits only, and the large scenario reward adds the tick's reward to returns
+// (its per-agent terms in reward_ws)
 static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
-                               int32_t ticks, float* returns, int32_t* hits, void* workspace, cudaStream_t st) {
+                               int32_t ticks, float* returns, int32_t* hits, void* workspace, cudaStream_t st,
+                               const SwarmRewardSpec* rs = nullptr, float* shaping = nullptr, void* reward_ws = nullptr) {
   const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
   const bool knn = cfg->graph_mode == SWARM_GRAPH_KNN;
   uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
@@ -968,7 +1010,7 @@ static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spe
   void* fwd_ws = reinterpret_cast<void*>(base + ((bn * 4 + (knn ? bn * cfg->knn_k * 4 : 0) + 255) & ~(int64_t)255));
   // in place: one CTA owns a whole env and stages its positions first
   SimStepArgs p = step_args(*cfg, state, actions, state);
-  p.returns = returns;
+  p.returns = rs ? nullptr : returns;
   p.hits = hits;
   for (int t = 0; t < ticks; ++t) {
     if (knn)
@@ -978,6 +1020,10 @@ static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spe
         e != cudaSuccess)
       return check_cuda(e, "swarm_rollout_stack (forward)");
     if (cudaError_t e = launch_sim_step_large(p, st); e != cudaSuccess) return check_cuda(e, "swarm_rollout_stack (step)");
+    if (rs)
+      if (cudaError_t e = launch_scenario_reward_large(*rs, state, shaping, nullptr, nullptr, returns, reward_ws, st);
+          e != cudaSuccess)
+        return check_cuda(e, "swarm_rollout_stack_large (reward)");
   }
   return SWARM_OK;
 }
@@ -1000,6 +1046,41 @@ int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, cons
   return check_cuda(launch_gatstack_rollout(*cfg, *spec, weights, state, ticks, world_consts(*cfg), reward ? &rs : nullptr,
                                             shaping, returns, hits, (cudaStream_t)stream),
                     "swarm_rollout_stack");
+}
+
+int64_t swarm_rollout_stack_large_workspace_bytes(const SwarmConfig* cfg, const SwarmRewardSpec* reward) {
+  if (!cfg || cfg->num_envs <= 0 || cfg->n_agents <= kTileThreads || cfg->n_agents > kMaxLargeAgents) return 0;
+  // swarm_rollout_stack's layout, then (reward) the per-agent terms of the large scenario reward, 256-byte aligned
+  const int64_t base = swarm_rollout_stack_workspace_bytes(cfg);
+  if (!reward) return base;
+  SwarmRewardSpec rs = *reward;
+  rs.num_envs = cfg->num_envs;
+  rs.n_agents = cfg->n_agents;
+  return base + 256 + scenario_reward_large_workspace_bytes(rs);
+}
+
+int swarm_rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
+                              int32_t ticks, const SwarmRewardSpec* reward, float* shaping, float* returns,
+                              int32_t* hits, void* workspace, int64_t workspace_bytes, void* stream) {
+  if (int rc = validate_stack(cfg, spec, true)) return rc;
+  if (cfg->n_agents <= kTileThreads)
+    return fail(SWARM_ERR_UNSUPPORTED, "swarm_rollout_stack_large runs 129 <= n_agents <= 4096 (smaller swarms: "
+                                       "swarm_rollout_stack)");
+  if (!weights || !state || !workspace) return fail(SWARM_ERR_INVALID_ARG, "weights/state/workspace is NULL");
+  if (ticks < 0) return fail(SWARM_ERR_INVALID_ARG, "ticks must be >= 0");
+  SwarmRewardSpec rs;
+  if (int rc = stack_reward(cfg, reward, shaping, rs)) return rc;
+  if (reward && (int64_t)cfg->num_envs * cfg->n_agents >= (1LL << 31))
+    return fail(SWARM_ERR_UNSUPPORTED, "num_envs * n_agents must stay below 2^31");
+  if (workspace_bytes < swarm_rollout_stack_large_workspace_bytes(cfg, reward))
+    return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  void* reward_ws = nullptr;
+  if (reward) {
+    const uintptr_t at = reinterpret_cast<uintptr_t>(workspace) + (uintptr_t)swarm_rollout_stack_workspace_bytes(cfg);
+    reward_ws = reinterpret_cast<void*>((at + 255) & ~(uintptr_t)255);
+  }
+  return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, workspace, (cudaStream_t)stream,
+                             reward ? &rs : nullptr, shaping, reward_ws);
 }
 
 int swarm_train_tick_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,

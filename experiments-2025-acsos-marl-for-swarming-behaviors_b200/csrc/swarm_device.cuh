@@ -125,17 +125,86 @@ __device__ __forceinline__ float torch_row_sum(int m, F elem) {
   return fin;
 }
 
+// The same row sum for rows of up to 8 191 non-negative elements, with the cascade of ATen's multi_row_sum that
+// torch_row_sum leaves out.  multi_row_sum keeps four levels of the four vector accumulators, level_power =
+// max(4, CeilLog2(groups) / 4) = 4 below 2^16 groups: after every 16th group of four chunks (512 floats) the level-0
+// accumulators a0..a3 are added into the level-1 accumulators b0..b3 and cleared; after the last group the levels are
+// added back into level 0, and row_sum goes on as torch_row_sum does (leftover chunks, accumulators, tail, lanes).
+// Below 256 groups (m < 8 192) levels 2 and 3 stay zero, and so does level 1 below 16 groups: adding a zero changes no
+// sum of non-negative elements, so those adds are left out.  Up to 17 groups (m < 576) the result equals
+// torch_row_sum's, as float addition is commutative; from m = 576 on the two orders differ
+// (tests/test_torch_sum_order_cascade.py).  elem(k) is called exactly once per k.
+template <typename F>
+__device__ __forceinline__ float torch_row_sum_cascade(int m, F elem) {
+  if (m < 8) {
+    float p0 = 0.0f, p1 = 0.0f, p2 = 0.0f, p3 = 0.0f;
+    int k = 0;
+    if (m >= 4) {
+      p0 = elem(0); p1 = elem(1); p2 = elem(2); p3 = elem(3);
+      k = 4;
+    }
+    for (; k < m; ++k) p0 = __fadd_rn(p0, elem(k));
+    return __fadd_rn(__fadd_rn(__fadd_rn(p0, p1), p2), p3);
+  }
+  const int chunks = m >> 3, groups = chunks >> 2;
+  float a0[8], a1[8], a2[8], a3[8], b0[8], b1[8], b2[8], b3[8];
+#pragma unroll
+  for (int l = 0; l < 8; ++l) a0[l] = a1[l] = a2[l] = a3[l] = b0[l] = b1[l] = b2[l] = b3[l] = 0.0f;
+  int c = 0;
+  for (int gI = 0; gI < groups; ++gI, c += 4) {
+#pragma unroll
+    for (int l = 0; l < 8; ++l) {
+      a0[l] = __fadd_rn(a0[l], elem((c + 0) * 8 + l));
+      a1[l] = __fadd_rn(a1[l], elem((c + 1) * 8 + l));
+      a2[l] = __fadd_rn(a2[l], elem((c + 2) * 8 + l));
+      a3[l] = __fadd_rn(a3[l], elem((c + 3) * 8 + l));
+    }
+    if ((gI & 15) == 15) {                                  // a full block of 16 groups: level 0 -> level 1
+#pragma unroll
+      for (int l = 0; l < 8; ++l) {
+        b0[l] = __fadd_rn(b0[l], a0[l]); a0[l] = 0.0f;
+        b1[l] = __fadd_rn(b1[l], a1[l]); a1[l] = 0.0f;
+        b2[l] = __fadd_rn(b2[l], a2[l]); a2[l] = 0.0f;
+        b3[l] = __fadd_rn(b3[l], a3[l]); a3[l] = 0.0f;
+      }
+    }
+  }
+  if (groups >= 16) {                                       // level 1 -> level 0
+#pragma unroll
+    for (int l = 0; l < 8; ++l) {
+      a0[l] = __fadd_rn(a0[l], b0[l]);
+      a1[l] = __fadd_rn(a1[l], b1[l]);
+      a2[l] = __fadd_rn(a2[l], b2[l]);
+      a3[l] = __fadd_rn(a3[l], b3[l]);
+    }
+  }
+  for (; c < chunks; ++c) {
+#pragma unroll
+    for (int l = 0; l < 8; ++l) a0[l] = __fadd_rn(a0[l], elem(c * 8 + l));
+  }
+  if (groups > 0) {
+#pragma unroll
+    for (int l = 0; l < 8; ++l) a0[l] = __fadd_rn(__fadd_rn(__fadd_rn(a0[l], a1[l]), a2[l]), a3[l]);
+  }
+  float fin = 0.0f;
+  for (int k = chunks * 8; k < m; ++k) fin = __fadd_rn(fin, elem(k));
+#pragma unroll
+  for (int l = 0; l < 8; ++l) fin = __fadd_rn(fin, a0[l]);
+  return fin;
+}
+
 // Flocking's partner sweep of agent i at (px, py) (flocking_scenario.py:109-121,148-168): element k of the stacked
 // distance list is partner j = k + (k >= i) -- the list comprehension skips the agent itself --
-//   sum   = torch sum of (|p_i - p_j| - desired)^2 in torch's CPU row order (see torch_row_sum)
+//   sum   = torch sum of (|p_i - p_j| - desired)^2 in torch's CPU row order (torch_row_sum, exact for N <= 128;
+//           CASCADE = true: torch_row_sum_cascade, exact for N <= 4 096)
 //   close = number of partners with world.get_distance <= min_collision_distance (centre distance minus both radii)
 // pos(j) yields partner j's position.
-template <typename P>
+template <bool CASCADE = false, typename P>
 __device__ __forceinline__ void flocking_partner_sweep(float px, float py, int i, int N, P pos, float desired,
                                                        float radius, float min_collision_distance, float& sum,
                                                        int& close) {
   int cnt = 0;
-  sum = torch_row_sum(N - 1, [&](int k) -> float {
+  auto elem = [&](int k) -> float {
     const int j = k + (k >= i ? 1 : 0);
     const float2 q = pos(j);
     const float dx = __fsub_rn(px, q.x), dy = __fsub_rn(py, q.y);
@@ -144,7 +213,11 @@ __device__ __forceinline__ void flocking_partner_sweep(float px, float py, int i
     const float gap = __fsub_rn(__fsub_rn(d, radius), radius);
     cnt += (gap <= min_collision_distance) ? 1 : 0;
     return __fmul_rn(e, e);
-  });
+  };
+  if constexpr (CASCADE)
+    sum = torch_row_sum_cascade(N - 1, elem);
+  else
+    sum = torch_row_sum(N - 1, elem);
   close = cnt;
 }
 

@@ -323,7 +323,18 @@ def reward_spec(kind: int, num_envs: int, n_agents: int, **overrides) -> _lib.Sw
 def scenario_reward(spec: _lib.SwarmRewardSpec, state: torch.Tensor, shaping: Optional[torch.Tensor] = None, *,
                     reset: bool = False, env_index: Optional[int] = None, want_terms: bool = False):
     """swarm_scenario_reward on state f32[B,N,4].  Flocking: shaping f32[B,N,2] is updated in place; returns the
-    collective reward f32[B] (None for a reset call).  Cohesion: returns f32[B,N].  ``want_terms`` adds f32[B,N,4]."""
+    collective reward f32[B] (None for a reset call).  Cohesion: returns f32[B,N].  ``want_terms`` adds f32[B,N,4].
+    Above 128 agents (up to 4 096) it runs ``scenario_reward_large``."""
+    return _scenario_reward(spec, state, shaping, reset, env_index, want_terms, spec.n_agents > 128)
+
+
+def scenario_reward_large(spec: _lib.SwarmRewardSpec, state: torch.Tensor, shaping: Optional[torch.Tensor] = None, *,
+                          reset: bool = False, env_index: Optional[int] = None, want_terms: bool = False):
+    """``scenario_reward`` through swarm_scenario_reward_large (any 2 <= N <= 4 096; its workspace allocated here)."""
+    return _scenario_reward(spec, state, shaping, reset, env_index, want_terms, True)
+
+
+def _scenario_reward(spec, state, shaping, reset, env_index, want_terms, large):
     B, N = spec.num_envs, spec.n_agents
     _expect(state, torch.float32, B * N * 4, "state")
     dev = state.device
@@ -340,8 +351,14 @@ def scenario_reward(spec: _lib.SwarmRewardSpec, state: torch.Tensor, shaping: Op
         reward = torch.zeros(B, dtype=torch.float32, device=dev) if flocking else \
             torch.zeros(B, N, dtype=torch.float32, device=dev)
     terms = torch.zeros(B, N, 4, dtype=torch.float32, device=dev) if (want_terms and not reset) else None
-    check(lib().swarm_scenario_reward(C.byref(call), ptr(state), ptr(shaping) if flocking else None, ptr(reward),
-                                      ptr(terms), stream_ptr(dev)))
+    if large:
+        wb = int(lib().swarm_scenario_reward_large_workspace_bytes(C.byref(call)))
+        ws = torch.empty(wb, dtype=torch.uint8, device=dev) if wb > 0 else None
+        check(lib().swarm_scenario_reward_large(C.byref(call), ptr(state), ptr(shaping) if flocking else None, ptr(reward),
+                                                ptr(terms), ptr(ws), wb, stream_ptr(dev)))
+    else:
+        check(lib().swarm_scenario_reward(C.byref(call), ptr(state), ptr(shaping) if flocking else None, ptr(reward),
+                                          ptr(terms), stream_ptr(dev)))
     return (reward, terms) if want_terms else reward
 
 
@@ -761,7 +778,22 @@ def rollout_stack(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Te
                   reward: Optional["_lib.SwarmRewardSpec"] = None, shaping: Optional[torch.Tensor] = None,
                   returns: Optional[torch.Tensor] = None, hits: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
     """Greedy rollout of a stacked network, in place on ``state``: per tick forward -> world step -> reward (the world's,
-    or the Flocking / Cohesion reward of ``reward``) -> running totals, all launched from the library."""
+    or the Flocking / Cohesion reward of ``reward``) -> running totals, all launched from the library.  Above 128 agents
+    a Flocking / Cohesion reward runs through ``rollout_stack_large``."""
+    if cfg.n_agents > 128 and reward is not None:
+        return rollout_stack_large(cfg, spec, weights, state, ticks, reward, shaping, returns, hits)
+    return _rollout_stack(cfg, spec, weights, state, ticks, reward, shaping, returns, hits, False)
+
+
+def rollout_stack_large(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Tensor, ticks: int,
+                        reward: Optional["_lib.SwarmRewardSpec"] = None, shaping: Optional[torch.Tensor] = None,
+                        returns: Optional[torch.Tensor] = None, hits: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+    """``rollout_stack`` through swarm_rollout_stack_large (129 <= N <= 4 096, any reward): per tick [topk table ->] the
+    large stacked forward -> world step -> [large scenario reward] with returns += the tick's reward."""
+    return _rollout_stack(cfg, spec, weights, state, ticks, reward, shaping, returns, hits, True)
+
+
+def _rollout_stack(cfg, spec, weights, state, ticks, reward, shaping, returns, hits, large):
     B, N = cfg.num_envs, cfg.n_agents
     _expect(state, torch.float32, B * N * 4, "state")
     _expect(weights, torch.float32, int(lib().swarm_stack_weight_count(C.byref(spec))), "weights")
@@ -772,11 +804,17 @@ def rollout_stack(cfg: SwarmConfig, spec, weights: torch.Tensor, state: torch.Te
         hits = torch.zeros(B, dtype=torch.int32, device=dev)
     if shaping is not None:
         _expect(shaping, torch.float32, B * N * 2, "shaping")
-    wb = int(lib().swarm_rollout_stack_workspace_bytes(C.byref(cfg)))
-    ws = torch.empty(wb, dtype=torch.uint8, device=dev)
-    check(lib().swarm_rollout_stack(C.byref(cfg), C.byref(spec), ptr(weights), ptr(state), int(ticks),
-                                    C.addressof(reward) if reward is not None else None, ptr(shaping), ptr(returns), ptr(hits),
-                                    ptr(ws), wb, stream_ptr(dev)))
+    rptr = C.addressof(reward) if reward is not None else None
+    if large:
+        wb = int(lib().swarm_rollout_stack_large_workspace_bytes(C.byref(cfg), rptr))
+        ws = torch.empty(max(wb, 1), dtype=torch.uint8, device=dev)
+        fn = lib().swarm_rollout_stack_large
+    else:
+        wb = int(lib().swarm_rollout_stack_workspace_bytes(C.byref(cfg)))
+        ws = torch.empty(wb, dtype=torch.uint8, device=dev)
+        fn = lib().swarm_rollout_stack
+    check(fn(C.byref(cfg), C.byref(spec), ptr(weights), ptr(state), int(ticks), rptr, ptr(shaping), ptr(returns), ptr(hits),
+             ptr(ws), wb, stream_ptr(dev)))
     out = {"state": state, "returns": returns, "hits": hits}
     if shaping is not None:
         out["shaping"] = shaping

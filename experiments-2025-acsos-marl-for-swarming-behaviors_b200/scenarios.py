@@ -553,7 +553,8 @@ class FlockingScenario(BaseScenario):
     sphere agents) and is stepped by ``swarm_sim_step``; the collective reward -- shaped goal progress, +50 on the goal,
     -1 per near-contact, shaped spacing progress, with the two ``previous_*`` memories per agent -- is one
     ``swarm_scenario_reward`` launch per tick over all envs.  The reference branches on tensors in Python
-    (flocking:141,169) and so only runs with ``num_envs = 1``; here every env is its own copy of that computation."""
+    (flocking:141,169) and so only runs with ``num_envs = 1``; here every env is its own copy of that computation.
+    Swarms of 2 to 4 096 agents: above 128 agents the reward runs through ``swarm_scenario_reward_large``."""
 
     scenario_id = _lib.SCENARIO_GOTO
 
@@ -663,7 +664,10 @@ class CohesionScenario(BaseScenario):
     (``swarm_scenario_reward``, one launch per tick for all agents and envs).  Stepped by ``swarm_sim_step`` like GoTo.
     The reference takes the min / max over everything ``torch.cat`` returns, i.e. it assumes one env; here the min / max
     are per env.  The Q-network kernels are specialised for 6-float observations, so this scenario is served at the
-    environment level (world step + reward), not by the fused rollout."""
+    environment level (world step + reward), not by the fused rollout.  Its reset keeps the reference's nine-agent start
+    table (and its IndexError beyond nine agents); for larger swarms, up to 4 096 agents, the Cohesion reward is reached
+    through ``ops.scenario_reward`` and ``ops.rollout_stack`` with a ``REWARD_COHESION`` spec on a state the caller
+    places."""
 
     scenario_id = _lib.SCENARIO_GOTO
     _START = [[-1.0, -1.0], [0.0, -1.0], [0.0, 1.0], [0.0, 0.0], [1.0, 1.0], [1.0, -1.0], [-1.0, 1.0], [1.0, 0.0],

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SWARM_ABI_VERSION 7
+#define SWARM_ABI_VERSION 8
 
 enum { SWARM_SCENARIO_GOTO = 0, SWARM_SCENARIO_OBSTACLE_AVOIDANCE = 1 };
 /* SWARM_GRAPH_RADIUS is an EXTENSION (the reference has no radius graph, SURVEY.md Appendix C): the complete-graph
@@ -478,7 +478,8 @@ int swarm_episode_end(const SwarmConfig* cfg, SwarmTrainCtl* ctl, float* returns
  *     (reset_world_at(env_index)).  terms (optional) float[B][N][4] = (pos_rew, avoidance, dist_rew, distance_to_goal).
  *   Cohesion: reward float[B][N] per agent; shaping unused (NULL); terms (optional) float[B][N][4] =
  *     (collision_factor, cohesion_factor, min_distance, max_distance).
- * 2 <= n_agents <= 128 (with one agent the reference's torch.stack / torch.cat of an empty list raises). */
+ * 2 <= n_agents <= 128 (with one agent the reference's torch.stack / torch.cat of an empty list raises); larger swarms:
+ * swarm_scenario_reward_large. */
 #define SWARM_REWARD_FLOCKING 0
 #define SWARM_REWARD_COHESION 1
 typedef struct SwarmRewardSpec {
@@ -502,6 +503,16 @@ typedef struct SwarmRewardSpec {
 void swarm_default_reward_spec(SwarmRewardSpec* spec, int32_t kind, int32_t num_envs, int32_t n_agents);
 int swarm_scenario_reward(const SwarmRewardSpec* spec, const float* state, float* shaping, float* reward, float* terms,
                           void* stream);
+
+/* The same rewards, outputs and arguments for 2 <= n_agents <= 4096 (num_envs * n_agents < 2^31), equal bit for bit to
+ * the reference's float32 CPU computation at every size: the spacing term's mean over the N - 1 partner distances adds
+ * in the order torch's CPU row sum takes, including the cascade ATen starts at 512 floats per row.  One thread per
+ * agent sweeps every partner of its env from shared memory (O(N^2) per env); Flocking's collective reward is then added
+ * in agent order by a second launch.  workspace: swarm_scenario_reward_large_workspace_bytes(spec) bytes (Flocking:
+ * float[B][N] of per-agent terms; Cohesion: 0, workspace may be NULL; 0 as well for arguments the call rejects). */
+int64_t swarm_scenario_reward_large_workspace_bytes(const SwarmRewardSpec* spec);
+int swarm_scenario_reward_large(const SwarmRewardSpec* spec, const float* state, float* shaping, float* reward,
+                                float* terms, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- multi-layer GAT Q-networks (SURVEY.md 8f rank 4) -------------------------------------------------------------
  * The reference's GCN class carries conv2 / conv3 in comments (train_gcn_dqn.py:54-55, 64-67) and ships checkpoints of
@@ -551,12 +562,25 @@ int swarm_gatstack_forward_large(const SwarmConfig* cfg, const SwarmStackSpec* s
  * whole loop is ONE launch (state, running return and Flocking memory in registers across the ticks, same tick as
  * swarm_rollout) that leaves the workspace untouched.  n_agents > 128 (up to 4096): per tick [kNN: the topk table of
  * swarm_graph_build ->] swarm_gatstack_forward_large (argmax) -> swarm_sim_step in place, returns / hits accumulated by
- * the world step; reward must be NULL there (the Flocking / Cohesion rewards are implemented for n_agents <= 128).
+ * the world step; reward must be NULL there (with a Flocking / Cohesion reward above 128 agents:
+ * swarm_rollout_stack_large).
  * No host work or allocation inside (graph capturable).  workspace: swarm_rollout_stack_workspace_bytes(cfg). */
 int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg);
 int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
                         int32_t ticks, const SwarmRewardSpec* reward, float* shaping, float* returns, int32_t* hits,
                         void* workspace, int64_t workspace_bytes, void* stream);
+
+/* swarm_rollout_stack for 129 <= n_agents <= 4096 with any reward: per tick [kNN: the topk table ->]
+ * swarm_gatstack_forward_large (argmax) -> swarm_sim_step in place (hits += as in swarm_rollout_stack) -> with a
+ * SwarmRewardSpec, swarm_scenario_reward_large on the stepped state and returns[b][i] += the tick's reward (Flocking:
+ * the env's collective reward for every agent, shaping required and initialised by a reset call; Cohesion: the agent's
+ * own).  reward == NULL gives exactly what swarm_rollout_stack gives (the world's own reward).  No host work or
+ * allocation inside (graph capturable).  workspace: swarm_rollout_stack_large_workspace_bytes(cfg, reward) bytes, which
+ * is swarm_rollout_stack_workspace_bytes(cfg) for reward == NULL (0 outside 129 <= n_agents <= 4096). */
+int64_t swarm_rollout_stack_large_workspace_bytes(const SwarmConfig* cfg, const SwarmRewardSpec* reward);
+int swarm_rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
+                              int32_t ticks, const SwarmRewardSpec* reward, float* shaping, float* returns,
+                              int32_t* hits, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* One DQN loss + gradient of a stacked network (train_step_dqn, train_gcn_dqn.py:116-124, for the conv1 .. convL form):
  * the contract of swarm_dqn_grad for the network described by `spec`.  Transitions come from `batch` (slot g, or slot
