@@ -23,6 +23,7 @@ FLAG_HIT = 2
 FLAG_PENALTY = 4
 W_COUNT = 1673
 ABI_VERSION = 8
+ERR_UNSUPPORTED = -2     # SWARM_ERR_UNSUPPORTED: the library does not implement this call's shape
 XCHG_STRIDE = 1680
 
 # state-dict tensors in packed order (include/swarm_b200.h SWARM_W_*)

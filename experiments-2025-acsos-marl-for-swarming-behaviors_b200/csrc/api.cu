@@ -5,105 +5,10 @@
 #include <cstring>
 #include <string>
 
+#include "launchers.h"
 #include "tile_kernels.cuh"
 
 namespace swarm {
-cudaError_t launch_tile(int mode, const TileParams& p, cudaStream_t stream);
-cudaError_t launch_sim_step(SimStepArgs p, cudaStream_t stream);
-cudaError_t launch_sim_step_large(const SimStepArgs& p, cudaStream_t stream);
-cudaError_t launch_graph_large(const SwarmConfig& c, const float* state, int32_t* edges, int32_t* nbr, int edges_per_env,
-                               cudaStream_t stream);
-cudaError_t launch_reset_grid(const SwarmConfig& c, int cols, int rows, const float* centers, float* state,
-                              cudaStream_t stream);
-long long gat_layer_workspace_bytes(int n, long long E, int ci, int co, bool backward);
-cudaError_t launch_gat_layer_forward(int n, int ci, int co, const float* W, const float* a_src, const float* a_dst,
-                                     const float* bias, const float* x, const int32_t* row_ptr, const int32_t* src,
-                                     float* out, void* workspace, cudaStream_t stream);
-cudaError_t launch_gat_layer_backward(int n, long long E, int ci, int co, const float* W, const float* a_src,
-                                      const float* a_dst, const float* x, const int32_t* row_ptr, const int32_t* src,
-                                      const int32_t* perm, const int32_t* row_ptr_s, const int32_t* tgt_s,
-                                      const int32_t* perm_s, const float* grad_out, float* gW, float* gas, float* gad,
-                                      float* gb, float* grad_x, void* workspace, cudaStream_t stream);
-cudaError_t launch_scenario_reward(const SwarmRewardSpec& sp, const float* state, float* shaping, float* reward,
-                                   float* terms, cudaStream_t stream);
-long long scenario_reward_large_workspace_bytes(const SwarmRewardSpec& sp);
-cudaError_t launch_scenario_reward_large(const SwarmRewardSpec& sp, const float* state, float* shaping, float* reward,
-                                         float* terms, float* returns, void* workspace, cudaStream_t stream);
-cudaError_t launch_reset_random(const SwarmConfig& c, const SwarmResetSpec& sp, int cols, int rows, const SwarmTrainCtl* ctl,
-                                long long episode, float* centers_out, float* state, cudaStream_t stream);
-cudaError_t launch_episode_end(const SwarmConfig& c, SwarmTrainCtl* ctl, float* returns, int32_t* hits, const float* loss,
-                               float* stats, long long max_episodes, double eps0, double decay, double min_eps,
-                               cudaStream_t stream);
-int stack_weight_count_host(const SwarmStackSpec& s);
-cudaError_t launch_gatstack_forward(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, const float* state,
-                                    float* q, int32_t* actions, cudaStream_t stream);
-cudaError_t launch_gatstack_rollout(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
-                                    int ticks, const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
-                                    float* returns, int32_t* hits, cudaStream_t stream);
-cudaError_t launch_gatstack_train_tick(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, float* state,
-                                       const WorldConsts& step, const SwarmRewardSpec* flock, float* shaping,
-                                       float* returns, int32_t* hits, const SwarmReplay& ring, const SwarmTrainCtl* ctl,
-                                       unsigned long long rng_seed, long long env_offset, cudaStream_t stream);
-int stack_large_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
-long long stack_large_workspace_bytes(const SwarmConfig& c, int hp);
-long long stack_large_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
-cudaError_t launch_gatstack_large(const SwarmConfig& c, const SwarmStackSpec& spec, const float* weights, const float* state,
-                                  const int32_t* nbr, float* q, int32_t* actions, void* workspace, cudaStream_t stream);
-int stack_grad_smem_bytes(const SwarmConfig& c, const SwarmStackSpec& s);
-long long stack_grad_workspace_bytes(const SwarmConfig& c, const SwarmStackSpec& s, int n_graphs);
-cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, const float* w_online, const float* w_target,
-                              const SwarmReplay& batch, const int64_t* indices, int n_graphs, float gamma, float loss_scale,
-                              float* grad, float* loss, float* td, void* workspace, cudaStream_t stream,
-                              SwarmTrainCtl* ctl = nullptr, int64_t* indices_out = nullptr,
-                              unsigned long long sample_seed = 0, int pushed_envs = 0);
-cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const float* grad, float* m, float* v,
-                                   long long step, double lr, double beta1, double beta2, double eps, double max_norm,
-                                   float* target, float* grad_norm, cudaStream_t stream, SwarmTrainCtl* ctl = nullptr,
-                                   int num_envs = 0, long long ring_capacity = 1, int update_target_every = 1);
-bool gatq_knn_large_fits(int N, int K);
-bool gatq_large_x_fits(int N, bool radius);
-cudaError_t launch_gatq_large_x(const SwarmConfig& c, const float* weights, const float* state, float* q, int32_t* actions,
-                                cudaStream_t stream);
-cudaError_t launch_radius_csr(const SwarmConfig& c, const float* state, int32_t* degree, const int32_t* row_ptr,
-                              int32_t* src, cudaStream_t stream);
-bool gatq_knn_large_x_fits(int N, int K);
-cudaError_t launch_gatq_knn_large_x(const SwarmConfig& c, const float* weights, const float* state, const int32_t* nbr,
-                                    float* q, int32_t* actions, cudaStream_t stream);
-cudaError_t launch_gatq_knn_large(const SwarmConfig& c, const float* weights, const float* state, const int32_t* nbr,
-                                  float* q, int32_t* actions, cudaStream_t stream);
-long long csr_workspace_bytes(int n, long long E);
-cudaError_t launch_csr_from_edges(int n, long long E, const int64_t* edge_src, const int64_t* edge_dst, int32_t* row_ptr,
-                                  int32_t* src, int32_t* perm, void* workspace, long long workspace_bytes,
-                                  cudaStream_t stream);
-cudaError_t launch_gatq_csr(int n, const float* weights, const float* x, const int32_t* row_ptr, const int32_t* src,
-                            float* q, int32_t* actions, float* rows, cudaStream_t stream, bool conv_only = false);
-long long gatq_workspace_bytes(int n);
-long long gatq_backward_workspace_bytes(int n, long long E);
-cudaError_t launch_gatq_backward_csr(int n, long long E, const float* weights, const float* x, const int32_t* row_ptr,
-                                     const int32_t* src, const int32_t* perm, const int32_t* row_ptr_s,
-                                     const int32_t* tgt_s, const int32_t* perm_s, const float* grad_q, float* grad_w,
-                                     void* workspace, cudaStream_t stream, bool conv_only = false);
-cudaError_t launch_replay_push(const SwarmReplay& r, long long cursor, int B, int N, const float* state,
-                               const int32_t* actions, const float* rewards, const float* next_state,
-                               cudaStream_t stream);
-cudaError_t launch_replay_gather(const SwarmReplay& r, const int64_t* indices, int G, int N, float* state,
-                                 int32_t* actions, float* rewards, float* next_state, cudaStream_t stream);
-long long dqn_workspace_bytes(const SwarmConfig& c, int n_graphs);
-int dqn_smem_bytes(const SwarmConfig& c);
-bool dqn_fuse_reduce(const SwarmConfig& c, int n_graphs);
-cudaError_t launch_dqn_grad(const SwarmConfig& c, const float* w_online, const float* w_target, const SwarmReplay& batch,
-                            const int64_t* indices, int n_graphs, float gamma, float loss_scale, float* grad, float* loss,
-                            float* td, void* workspace, cudaStream_t stream, SwarmTrainCtl* ctl = nullptr,
-                            int64_t* indices_out = nullptr, unsigned long long sample_seed = 0, int pushed_envs = 0,
-                            bool skip_reduce = false);
-cudaError_t launch_adam_clip(float* w, const float* grad, float* m, float* v, long long step, double lr, double beta1,
-                             double beta2, double eps, double max_norm, float* target, float* grad_norm,
-                             cudaStream_t stream, SwarmTrainCtl* ctl = nullptr, int num_envs = 0,
-                             long long ring_capacity = 1, int update_target_every = 1,
-                             const SwarmPeerExchange* peers = nullptr, float* grad_rw = nullptr,
-                             const SwarmConfig* reduce_cfg = nullptr, const void* reduce_workspace = nullptr,
-                             int reduce_graphs = 0, float loss_scale = 0.0f);
-
 namespace {
 thread_local std::string g_last_error;
 
@@ -146,6 +51,116 @@ int validate(const SwarmConfig* cfg, bool need_graph, bool allow_large = false) 
     }
   }
   return SWARM_OK;
+}
+
+// above 128 agents the kNN table comes from torch.topk's partial_sort branch, the only one implemented
+int validate_large_knn(const SwarmConfig& c) {
+  if (c.graph_mode == SWARM_GRAPH_KNN && c.n_agents > kTileThreads && (int64_t)c.knn_k * 64 > c.n_agents)
+    return fail(SWARM_ERR_UNSUPPORTED,
+                "large-swarm kNN implements torch.topk's partial_sort branch only (needs 64 * k <= n_agents)");
+  return SWARM_OK;
+}
+
+// what: "replay ring" or "batch"; need_capacity: the call writes into the ring
+int validate_ring(const SwarmReplay* r, const char* what, bool need_capacity) {
+  if (!r || !r->state || !r->next_state || !r->actions || !r->rewards || (need_capacity && r->capacity <= 0))
+    return fail(SWARM_ERR_INVALID_ARG,
+                std::string(what) + (need_capacity ? " has NULL arrays or no capacity" : " has NULL arrays"));
+  return SWARM_OK;
+}
+
+// torch.optim.Adam's ValueError checks
+int validate_adam(double lr, double beta1, double beta2, double eps) {
+  if (!(lr >= 0.0) || !(beta1 >= 0.0 && beta1 < 1.0) || !(beta2 >= 0.0 && beta2 < 1.0) || !(eps >= 0.0))
+    return fail(SWARM_ERR_INVALID_ARG, "invalid Adam hyper-parameter");
+  return SWARM_OK;
+}
+
+// the Flocking / Cohesion rewards of a rollout tick on cfg's world; same_shape: the spec must cover cfg's envs and agents
+int validate_reward_cfg(const SwarmConfig* cfg, const SwarmRewardSpec& s, bool same_shape) {
+  if (cfg->scenario != SWARM_SCENARIO_GOTO)
+    return fail(SWARM_ERR_INVALID_ARG,
+                "the Flocking / Cohesion rewards run on the GoTo world (cfg->scenario = SWARM_SCENARIO_GOTO)");
+  if (same_shape && (s.num_envs != cfg->num_envs || s.n_agents != cfg->n_agents))
+    return fail(SWARM_ERR_INVALID_ARG, "reward spec and cfg disagree on num_envs / n_agents");
+  if (cfg->n_agents < 2) return fail(SWARM_ERR_INVALID_ARG, "the scenario rewards need at least two agents");
+  return SWARM_OK;
+}
+
+// Flocking's shaping memory and Cohesion's parameters; per_agent_reward: the call writes the reward array (a rollout
+// adds it to returns instead)
+int validate_reward_buffers(const SwarmRewardSpec& s, const float* shaping, bool per_agent_reward, const float* reward) {
+  if (s.kind == SWARM_REWARD_FLOCKING) {
+    if (!shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
+    if (per_agent_reward && !s.reset && !reward) return fail(SWARM_ERR_INVALID_ARG, "reward is NULL");
+  } else {
+    if (s.reset) return fail(SWARM_ERR_INVALID_ARG, "Cohesion keeps no shaping memory (reset must be 0)");
+    if (per_agent_reward && !reward) return fail(SWARM_ERR_INVALID_ARG, "reward is NULL");
+    if (!(s.sigma > 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "sigma must be > 0");
+  }
+  return SWARM_OK;
+}
+
+template <class T> T align256(T x) { return (x + 255) & ~(T)255; }
+
+// the start grid of reset_grid: math.ceil(math.sqrt(num_points)) columns, math.ceil(num_points / num_cols) rows
+struct GridShape {
+  int cols, rows;
+  explicit GridShape(int n) : cols((int)std::ceil(std::sqrt((double)n))), rows((int)std::ceil((double)n / (double)cols)) {}
+};
+
+// The workspace of a large-swarm rollout: the byte count its *_workspace_bytes call reports and, in a buffer of that
+// size, where each piece starts (256-byte aligned). One function per call computes both, so they cannot disagree.
+struct RolloutWorkspace {
+  int64_t bytes = 0;
+  int32_t* actions = nullptr;
+  int32_t* nbr = nullptr;       // the kNN graph's topk table
+  void* forward = nullptr;      // the large stacked forward's workspace
+  void* reward = nullptr;       // the large scenario reward's per-agent terms
+};
+
+int64_t knn_table_k(const SwarmConfig& c) { return c.graph_mode == SWARM_GRAPH_KNN && c.knn_k > 0 ? c.knn_k : 0; }
+
+// swarm_rollout_large: topk table, then actions
+RolloutWorkspace rollout_large_workspace(const SwarmConfig& c, void* ws = nullptr) {
+  const int64_t bn = (int64_t)c.num_envs * c.n_agents;
+  const uintptr_t base = align256(reinterpret_cast<uintptr_t>(ws));
+  RolloutWorkspace w;
+  w.bytes = bn * knn_table_k(c) * 4 + bn * 4 + 512;
+  w.nbr = reinterpret_cast<int32_t*>(base);
+  w.actions = reinterpret_cast<int32_t*>(base + bn * knn_table_k(c) * 4);
+  return w;
+}
+
+// swarm_rollout_stack above 128 agents: actions, topk table, then the large forward's workspace at the widest layer
+// (hidden 32). The n_agents <= 128 rollout is one launch that does not touch the workspace; its size is kept as the
+// ABI states it.
+RolloutWorkspace rollout_stack_workspace(const SwarmConfig& c, void* ws = nullptr) {
+  const int64_t bn = (int64_t)c.num_envs * c.n_agents;
+  RolloutWorkspace w;
+  if (c.n_agents <= kTileThreads) {
+    w.bytes = bn * 4 + bn * 4 + bn + 1024;
+    return w;
+  }
+  const int64_t tables = align256(bn * 4 + bn * knn_table_k(c) * 4);
+  const uintptr_t base = align256(reinterpret_cast<uintptr_t>(ws));
+  w.bytes = 256 + tables + stack_large_workspace_bytes(c, 32);
+  w.actions = reinterpret_cast<int32_t*>(base);
+  w.nbr = reinterpret_cast<int32_t*>(base + bn * 4);
+  w.forward = reinterpret_cast<void*>(base + tables);
+  return w;
+}
+
+// swarm_rollout_stack_large: the stacked layout, then (reward) the large scenario reward's per-agent terms
+RolloutWorkspace rollout_stack_large_workspace(const SwarmConfig& c, const SwarmRewardSpec* reward, void* ws = nullptr) {
+  RolloutWorkspace w = rollout_stack_workspace(c, ws);
+  if (!reward) return w;
+  SwarmRewardSpec rs = *reward;
+  rs.num_envs = c.num_envs;
+  rs.n_agents = c.n_agents;
+  w.reward = reinterpret_cast<void*>(align256(reinterpret_cast<uintptr_t>(ws) + (uintptr_t)w.bytes));
+  w.bytes += 256 + scenario_reward_large_workspace_bytes(rs);
+  return w;
 }
 
 int fill_params(TileParams& p, const SwarmConfig* cfg, int mode) {
@@ -225,10 +240,8 @@ int64_t swarm_edges_per_env(const SwarmConfig* cfg) {
 int swarm_reset_grid(const SwarmConfig* cfg, const float* centers, float* state, void* stream) {
   if (int rc = validate(cfg, false, true)) return rc;
   if (!centers || !state) return fail(SWARM_ERR_INVALID_ARG, "centers/state is NULL");
-  const int n = cfg->n_agents;
-  const int cols = (int)std::ceil(std::sqrt((double)n));     // math.ceil(math.sqrt(num_points))
-  const int rows = (int)std::ceil((double)n / (double)cols);  // math.ceil(num_points / num_cols)
-  return check_cuda(launch_reset_grid(*cfg, cols, rows, centers, state, (cudaStream_t)stream), "swarm_reset_grid");
+  const GridShape g(cfg->n_agents);
+  return check_cuda(launch_reset_grid(*cfg, g.cols, g.rows, centers, state, (cudaStream_t)stream), "swarm_reset_grid");
 }
 
 int swarm_sim_step(const SwarmConfig* cfg, const float* state_in, const int32_t* actions, float* state_out,
@@ -255,9 +268,7 @@ int swarm_graph_build(const SwarmConfig* cfg, const float* state, int32_t* edges
   if (cfg->graph_mode == SWARM_GRAPH_RADIUS)
     return fail(SWARM_ERR_INVALID_ARG, "radius graphs have a per-env edge count: use swarm_graph_build_radius");
   if (cfg->n_agents > kTileThreads) {
-    if (cfg->graph_mode == SWARM_GRAPH_KNN && (int64_t)cfg->knn_k * 64 > cfg->n_agents)
-      return fail(SWARM_ERR_UNSUPPORTED,
-                  "kNN for n_agents > 128 implements torch.topk's partial_sort branch only (needs 64 * k <= n_agents)");
+    if (int rc = validate_large_knn(*cfg)) return rc;
     if (cfg->graph_mode == SWARM_GRAPH_KNN && cfg->knn_k > 64) return fail(SWARM_ERR_UNSUPPORTED, "knn_k > 64");
     return check_cuda(launch_graph_large(*cfg, state, edges, neighbours, (int)swarm_edges_per_env(cfg), (cudaStream_t)stream),
                       "swarm_graph_build");
@@ -306,7 +317,7 @@ int swarm_gatq_forward_csr(int32_t n_nodes, const float* weights, const float* x
   if (!weights || !x || !row_ptr || !workspace) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
   if (!q && !actions) return fail(SWARM_ERR_INVALID_ARG, "no output requested");
   if (workspace_bytes < gatq_workspace_bytes(n_nodes)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  float* rows = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
+  float* rows = reinterpret_cast<float*>(align256(reinterpret_cast<uintptr_t>(workspace)));
   return check_cuda(launch_gatq_csr(n_nodes, weights, x, row_ptr, src, q, actions, rows, (cudaStream_t)stream),
                     "swarm_gatq_forward_csr");
 }
@@ -351,9 +362,7 @@ int swarm_gatq_forward_large(const SwarmConfig* cfg, const float* weights, const
 
 int64_t swarm_rollout_large_workspace_bytes(const SwarmConfig* cfg) {
   if (!cfg || cfg->num_envs <= 0 || cfg->n_agents <= 0) return 0;
-  const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
-  const int64_t k = cfg->graph_mode == SWARM_GRAPH_KNN ? (cfg->knn_k > 0 ? cfg->knn_k : 0) : 0;
-  return bn * k * 4 + bn * 4 + 512;
+  return rollout_large_workspace(*cfg).bytes;
 }
 
 int swarm_rollout_large(const SwarmConfig* cfg, const float* weights, float* state, int32_t ticks, float* returns,
@@ -362,9 +371,8 @@ int swarm_rollout_large(const SwarmConfig* cfg, const float* weights, float* sta
   if (cfg->n_agents <= kTileThreads) return fail(SWARM_ERR_INVALID_ARG, "n_agents <= 128: use swarm_rollout");
   if (!weights || !state || !workspace) return fail(SWARM_ERR_INVALID_ARG, "weights/state/workspace is NULL");
   if (ticks < 0) return fail(SWARM_ERR_INVALID_ARG, "ticks must be >= 0");
+  if (int rc = validate_large_knn(*cfg)) return rc;
   const bool knn = cfg->graph_mode == SWARM_GRAPH_KNN;
-  if (knn && (int64_t)cfg->knn_k * 64 > cfg->n_agents)
-    return fail(SWARM_ERR_UNSUPPORTED, "large-swarm kNN implements torch.topk's partial_sort branch (64 k <= n)");
   // attention in input space (no projected-feature tile: envs up to 4 096 agents fit) unless SWARM_TC=0 asks for the
   // bit-faithful forward of swarm_gatq_forward_knn_large (kNN only; the radius / complete graph of a large swarm has
   // the input-space forward alone -- their bit-faithful path is the CSR one)
@@ -376,11 +384,9 @@ int swarm_rollout_large(const SwarmConfig* cfg, const float* weights, float* sta
   if (!fits)
     return fail(SWARM_ERR_UNSUPPORTED, "the env does not fit shared memory: step it with swarm_graph_build + "
                                        "swarm_csr_from_edges + swarm_gatq_forward_csr + swarm_sim_step");
-  if (workspace_bytes < swarm_rollout_large_workspace_bytes(cfg)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
-  uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
-  int32_t* nbr = reinterpret_cast<int32_t*>(base);
-  int32_t* actions = nbr + (knn ? bn * cfg->knn_k : 0);
+  const RolloutWorkspace w = rollout_large_workspace(*cfg, workspace);
+  if (workspace_bytes < w.bytes) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  int32_t *nbr = w.nbr, *actions = w.actions;
   // in place: one CTA owns a whole env and stages its positions first
   SimStepArgs p = step_args(*cfg, state, actions, state);
   p.returns = returns;
@@ -412,7 +418,7 @@ int swarm_gatconv_forward_csr(int32_t n_nodes, const float* weights, const float
   if (n_nodes == 0) return SWARM_OK;
   if (!weights || !x || !row_ptr || !out || !workspace) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
   if (workspace_bytes < gatq_workspace_bytes(n_nodes)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  float* rows = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
+  float* rows = reinterpret_cast<float*>(align256(reinterpret_cast<uintptr_t>(workspace)));
   return check_cuda(launch_gatq_csr(n_nodes, weights, x, row_ptr, src, out, nullptr, rows, (cudaStream_t)stream, true),
                     "swarm_gatconv_forward_csr");
 }
@@ -527,10 +533,8 @@ int swarm_csr_from_edges(int32_t n_nodes, int64_t n_edges, const int64_t* edge_s
 static int attach_flocking(TileParams& p, const SwarmConfig* cfg, const SwarmRewardSpec* fs, float* shaping) {
   if (!fs) return SWARM_OK;
   if (fs->kind != SWARM_REWARD_FLOCKING) return fail(SWARM_ERR_INVALID_ARG, "`flocking` must be a Flocking reward spec");
-  if (cfg->scenario != SWARM_SCENARIO_GOTO)
-    return fail(SWARM_ERR_INVALID_ARG, "the Flocking reward runs on the GoTo world (cfg->scenario = SWARM_SCENARIO_GOTO)");
-  if (cfg->n_agents < 2) return fail(SWARM_ERR_INVALID_ARG, "the scenario rewards need at least two agents");
-  if (!shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
+  if (int rc = validate_reward_cfg(cfg, *fs, false)) return rc;
+  if (int rc = validate_reward_buffers(*fs, shaping, false, nullptr)) return rc;
   p.flock = *fs;
   p.shaping = reinterpret_cast<float2*>(shaping);
   p.use_flock = 1;
@@ -563,9 +567,8 @@ int swarm_rollout(const SwarmConfig* cfg, const float* weights, float* state, in
     p.rng_tick0 = opts->rng_tick0;
     p.env_offset = opts->env_offset;
     if (opts->replay) {
+      if (int rc = validate_ring(opts->replay, "replay ring", true)) return rc;
       const SwarmReplay& r = *opts->replay;
-      if (!r.state || !r.next_state || !r.actions || !r.rewards || r.capacity <= 0)
-        return fail(SWARM_ERR_INVALID_ARG, "replay ring has NULL arrays or no capacity");
       if ((int64_t)ticks * cfg->num_envs > r.capacity)
         return fail(SWARM_ERR_INVALID_ARG, "ticks * num_envs exceeds the replay capacity (slots would be overwritten inside one call)");
       p.replay = r;
@@ -587,8 +590,7 @@ int swarm_rollout(const SwarmConfig* cfg, const float* weights, float* state, in
 int swarm_replay_push(const SwarmConfig* cfg, const SwarmReplay* replay, int64_t cursor, const float* state,
                       const int32_t* actions, const float* rewards, const float* next_state, void* stream) {
   if (int rc = validate(cfg, false)) return rc;
-  if (!replay || !replay->state || !replay->next_state || !replay->actions || !replay->rewards || replay->capacity <= 0)
-    return fail(SWARM_ERR_INVALID_ARG, "replay ring has NULL arrays or no capacity");
+  if (int rc = validate_ring(replay, "replay ring", true)) return rc;
   if (!state || !actions || !rewards || !next_state) return fail(SWARM_ERR_INVALID_ARG, "NULL transition array");
   if (cfg->num_envs > replay->capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
   if (cursor < 0) return fail(SWARM_ERR_INVALID_ARG, "cursor must be >= 0");
@@ -600,8 +602,7 @@ int swarm_replay_push(const SwarmConfig* cfg, const SwarmReplay* replay, int64_t
 int swarm_replay_gather(const SwarmConfig* cfg, const SwarmReplay* replay, const int64_t* indices, int32_t n_graphs,
                         float* state, int32_t* actions, float* rewards, float* next_state, void* stream) {
   if (!cfg || cfg->n_agents <= 0) return fail(SWARM_ERR_INVALID_ARG, "cfg is NULL or n_agents <= 0");
-  if (!replay || !replay->state || !replay->next_state || !replay->actions || !replay->rewards)
-    return fail(SWARM_ERR_INVALID_ARG, "replay ring has NULL arrays");
+  if (int rc = validate_ring(replay, "replay ring", false)) return rc;
   if (n_graphs < 0) return fail(SWARM_ERR_INVALID_ARG, "n_graphs must be >= 0");
   if (n_graphs == 0) return SWARM_OK;
   if (!indices || !state || !actions || !rewards || !next_state) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
@@ -631,8 +632,7 @@ int swarm_dqn_grad(const SwarmConfig* cfg, const float* online_weights, const fl
                    float* grad, float* loss, float* td, void* workspace, int64_t workspace_bytes, void* stream) {
   if (int rc = validate_dqn(cfg, n_graphs)) return rc;
   if (!online_weights || !target_weights || !grad || !loss || !workspace) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
-  if (!batch || !batch->state || !batch->next_state || !batch->actions || !batch->rewards)
-    return fail(SWARM_ERR_INVALID_ARG, "batch has NULL arrays");
+  if (int rc = validate_ring(batch, "batch", false)) return rc;
   if (workspace_bytes < dqn_workspace_bytes(*cfg, n_graphs)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
   return check_cuda(launch_dqn_grad(*cfg, online_weights, target_weights, *batch, indices, n_graphs, gamma, loss_scale,
                                     grad, loss, td, workspace, (cudaStream_t)stream),
@@ -644,8 +644,7 @@ int swarm_adam_clip_step(float* weights, const float* grad, float* exp_avg, floa
                          float* grad_norm, void* stream) {
   if (!weights || !grad || !exp_avg || !exp_avg_sq) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
   if (step < 1) return fail(SWARM_ERR_INVALID_ARG, "step is 1-based");
-  if (!(lr >= 0.0) || !(beta1 >= 0.0 && beta1 < 1.0) || !(beta2 >= 0.0 && beta2 < 1.0) || !(eps >= 0.0))
-    return fail(SWARM_ERR_INVALID_ARG, "invalid Adam hyper-parameter");     // torch.optim.Adam's ValueError checks
+  if (int rc = validate_adam(lr, beta1, beta2, eps)) return rc;
   return check_cuda(launch_adam_clip(weights, grad, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_norm,
                                      target_weights, grad_norm, (cudaStream_t)stream),
                     "swarm_adam_clip_step");
@@ -655,9 +654,7 @@ static int validate_hyper(const SwarmTrainHyper* h) {
   if (!h) return fail(SWARM_ERR_INVALID_ARG, "hyper is NULL");
   if (h->graphs_per_update <= 0) return fail(SWARM_ERR_INVALID_ARG, "graphs_per_update must be positive");
   if (h->update_target_every <= 0) return fail(SWARM_ERR_INVALID_ARG, "update_target_every must be positive");
-  if (!(h->lr >= 0.0) || !(h->beta1 >= 0.0 && h->beta1 < 1.0) || !(h->beta2 >= 0.0 && h->beta2 < 1.0) || !(h->eps >= 0.0))
-    return fail(SWARM_ERR_INVALID_ARG, "invalid Adam hyper-parameter");
-  return SWARM_OK;
+  return validate_adam(h->lr, h->beta1, h->beta2, h->eps);
 }
 
 // shared argument checks and rollout-tick parameters of swarm_train_tick_grad / swarm_train_tick
@@ -670,8 +667,7 @@ static int train_tick_rollout(const SwarmConfig* cfg, const SwarmTrainHyper* hyp
   if (int rc = validate_dqn(cfg, hyper->graphs_per_update)) return rc;
   if (!ctl || !weights || !target_weights || !state || !grad || !loss || !workspace)
     return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
-  if (!ring || !ring->state || !ring->next_state || !ring->actions || !ring->rewards || ring->capacity <= 0)
-    return fail(SWARM_ERR_INVALID_ARG, "replay ring has NULL arrays or no capacity");
+  if (int rc = validate_ring(ring, "replay ring", true)) return rc;
   if (cfg->num_envs > ring->capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
   if (workspace_bytes < dqn_workspace_bytes(*cfg, hyper->graphs_per_update))
     return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
@@ -761,10 +757,8 @@ int swarm_reset_random(const SwarmConfig* cfg, const SwarmResetSpec* spec, const
   if (!spec || !state) return fail(SWARM_ERR_INVALID_ARG, "spec/state is NULL");
   if (!(spec->std_x >= 0.0f) || !(spec->std_y >= 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "std must be >= 0");
   if (!ctl && episode < 0) return fail(SWARM_ERR_INVALID_ARG, "episode must be >= 0");
-  const int n = cfg->n_agents;
-  const int cols = (int)std::ceil(std::sqrt((double)n));
-  const int rows = (int)std::ceil((double)n / (double)cols);
-  return check_cuda(launch_reset_random(*cfg, *spec, cols, rows, ctl, episode, centers_out, state, (cudaStream_t)stream),
+  const GridShape g(cfg->n_agents);
+  return check_cuda(launch_reset_random(*cfg, *spec, g.cols, g.rows, ctl, episode, centers_out, state, (cudaStream_t)stream),
                     "swarm_reset_random");
 }
 
@@ -808,27 +802,14 @@ int validate_reward_spec(const SwarmRewardSpec* spec, bool large) {
     return fail(SWARM_ERR_UNSUPPORTED, "num_envs * n_agents must stay below 2^31");
   return SWARM_OK;
 }
-
-// the buffer checks of a call with num_envs > 0
-int validate_reward_buffers(const SwarmRewardSpec* spec, const float* state, const float* shaping, const float* reward) {
-  if (!state) return fail(SWARM_ERR_INVALID_ARG, "state is NULL");
-  if (spec->kind == SWARM_REWARD_FLOCKING) {
-    if (!shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
-    if (!spec->reset && !reward) return fail(SWARM_ERR_INVALID_ARG, "reward is NULL");
-  } else {
-    if (spec->reset) return fail(SWARM_ERR_INVALID_ARG, "Cohesion keeps no shaping memory (reset must be 0)");
-    if (!reward) return fail(SWARM_ERR_INVALID_ARG, "reward is NULL");
-    if (!(spec->sigma > 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "sigma must be > 0");
-  }
-  return SWARM_OK;
-}
 }  // namespace
 
 int swarm_scenario_reward(const SwarmRewardSpec* spec, const float* state, float* shaping, float* reward, float* terms,
                           void* stream) {
   if (int rc = validate_reward_spec(spec, false)) return rc;
   if (spec->num_envs == 0) return SWARM_OK;
-  if (int rc = validate_reward_buffers(spec, state, shaping, reward)) return rc;
+  if (!state) return fail(SWARM_ERR_INVALID_ARG, "state is NULL");
+  if (int rc = validate_reward_buffers(*spec, shaping, true, reward)) return rc;
   return check_cuda(launch_scenario_reward(*spec, state, shaping, reward, terms, (cudaStream_t)stream),
                     "swarm_scenario_reward");
 }
@@ -842,7 +823,8 @@ int swarm_scenario_reward_large(const SwarmRewardSpec* spec, const float* state,
                                 float* terms, void* workspace, int64_t workspace_bytes, void* stream) {
   if (int rc = validate_reward_spec(spec, true)) return rc;
   if (spec->num_envs == 0) return SWARM_OK;
-  if (int rc = validate_reward_buffers(spec, state, shaping, reward)) return rc;
+  if (!state) return fail(SWARM_ERR_INVALID_ARG, "state is NULL");
+  if (int rc = validate_reward_buffers(*spec, shaping, true, reward)) return rc;
   const int64_t need = scenario_reward_large_workspace_bytes(*spec);
   if (need > 0 && !workspace) return fail(SWARM_ERR_INVALID_ARG, "workspace is NULL");
   if (workspace_bytes < need) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
@@ -854,20 +836,25 @@ int swarm_scenario_reward_large(const SwarmRewardSpec* spec, const float* state,
 namespace {
 // large = false: the env-tile kernels (n_agents <= 128, kNN n_agents <= 16); large = true: the one-CTA-per-env kernel
 // (any n_agents <= 4096; above 128 agents the kNN table comes from the partial_sort branch of swarm_graph_build)
-int validate_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, bool large = false) {
-  if (int rc = validate(cfg, true, large)) return rc;
+int validate_spec(const SwarmStackSpec* spec) {
   if (!spec) return fail(SWARM_ERR_INVALID_ARG, "spec is NULL");
   if (spec->n_layers < 1 || spec->n_layers > 4) return fail(SWARM_ERR_INVALID_ARG, "n_layers must be 1 .. 4");
   if (spec->hidden < 1 || spec->hidden > 32) return fail(SWARM_ERR_UNSUPPORTED, "hidden must be 1 .. 32");
   if (spec->in_features != 7 && spec->in_features != 5) return fail(SWARM_ERR_INVALID_ARG, "in_features must be 7 or 5");
+  return SWARM_OK;
+}
+
+// large = false: the env-tile kernels (n_agents <= 128, kNN n_agents <= 16); large = true: the one-CTA-per-env kernel
+// (any n_agents <= 4096; above 128 agents the kNN table comes from the partial_sort branch of swarm_graph_build)
+int validate_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, bool large = false) {
+  if (int rc = validate(cfg, true, large)) return rc;
+  if (int rc = validate_spec(spec)) return rc;
   for (int l = 0; l < spec->n_layers; ++l)
     if (spec->activation[l] != SWARM_ACT_TANH && spec->activation[l] != SWARM_ACT_RELU)
       return fail(SWARM_ERR_INVALID_ARG, "unknown activation");
   if (!large && cfg->graph_mode == SWARM_GRAPH_KNN && cfg->n_agents > 16)
     return fail(SWARM_ERR_UNSUPPORTED, "stacked networks on the kNN graph are implemented for n_agents <= 16");
-  if (large && cfg->graph_mode == SWARM_GRAPH_KNN && cfg->n_agents > kTileThreads &&
-      (int64_t)cfg->knn_k * 64 > cfg->n_agents)
-    return fail(SWARM_ERR_UNSUPPORTED, "large-swarm kNN implements torch.topk's partial_sort branch (64 k <= n_agents)");
+  if (int rc = validate_large_knn(*cfg)) return rc;
   if (large && stack_large_smem_bytes(*cfg, *spec) > 227 * 1024)
     return fail(SWARM_ERR_UNSUPPORTED, "the large stacked forward needs more than 227 KB of shared memory for this (N, spec)");
   return SWARM_OK;
@@ -908,15 +895,15 @@ int swarm_gatstack_forward_large(const SwarmConfig* cfg, const SwarmStackSpec* s
 }
 
 namespace {
-int validate_spec(const SwarmStackSpec* spec) {
-  if (!spec) return fail(SWARM_ERR_INVALID_ARG, "spec is NULL");
-  if (spec->n_layers < 1 || spec->n_layers > 4) return fail(SWARM_ERR_INVALID_ARG, "n_layers must be 1 .. 4");
-  if (spec->hidden < 1 || spec->hidden > 32) return fail(SWARM_ERR_UNSUPPORTED, "hidden must be 1 .. 32");
-  if (spec->in_features != 7 && spec->in_features != 5) return fail(SWARM_ERR_INVALID_ARG, "in_features must be 7 or 5");
+// the stacked DQN gradient tile's own limits, for a cfg and spec that validate_stack accepts
+int validate_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec) {
+  if (c.n_agents < 2) return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN update needs n_agents >= 2");
+  if (stack_grad_smem_bytes(c, spec) > 227 * 1024)
+    return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN gradient tile exceeds 227 KB of shared memory for this (N, k, spec)");
   return SWARM_OK;
 }
 
-// the checks of swarm_gatstack_forward on a batch of n_graphs transitions, then the gradient tile's shared memory
+// the checks of swarm_gatstack_forward on a batch of n_graphs transitions, then the gradient tile's
 int validate_dqn_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, int32_t n_graphs) {
   if (!cfg) return fail(SWARM_ERR_INVALID_ARG, "cfg is NULL");
   if (n_graphs <= 0) return fail(SWARM_ERR_INVALID_ARG, "n_graphs must be positive");
@@ -925,10 +912,7 @@ int validate_dqn_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, int32
   SwarmConfig c = *cfg;
   c.num_envs = n_graphs;
   if (int rc = validate_stack(&c, spec)) return rc;
-  if (c.n_agents < 2) return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN update needs n_agents >= 2");
-  if (stack_grad_smem_bytes(c, *spec) > 227 * 1024)
-    return fail(SWARM_ERR_UNSUPPORTED, "the stacked DQN gradient tile exceeds 227 KB of shared memory for this (N, k, spec)");
-  return SWARM_OK;
+  return validate_stack_grad(c, *spec);
 }
 }  // namespace
 
@@ -943,8 +927,7 @@ int swarm_dqn_stack_grad(const SwarmConfig* cfg, const SwarmStackSpec* spec, con
                          int64_t workspace_bytes, void* stream) {
   if (int rc = validate_dqn_stack(cfg, spec, n_graphs)) return rc;
   if (!online_weights || !target_weights || !grad || !loss || !workspace) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
-  if (!batch || !batch->state || !batch->next_state || !batch->actions || !batch->rewards)
-    return fail(SWARM_ERR_INVALID_ARG, "batch has NULL arrays");
+  if (int rc = validate_ring(batch, "batch", false)) return rc;
   if (workspace_bytes < stack_grad_workspace_bytes(*cfg, *spec, n_graphs))
     return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
   return check_cuda(launch_stack_grad(*cfg, *spec, online_weights, target_weights, *batch, indices, n_graphs, gamma,
@@ -958,8 +941,7 @@ int swarm_adam_clip_stack_step(const SwarmStackSpec* spec, float* weights, const
   if (int rc = validate_spec(spec)) return rc;
   if (!weights || !grad || !exp_avg || !exp_avg_sq) return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
   if (step < 1) return fail(SWARM_ERR_INVALID_ARG, "step is 1-based");
-  if (!(lr >= 0.0) || !(beta1 >= 0.0 && beta1 < 1.0) || !(beta2 >= 0.0 && beta2 < 1.0) || !(eps >= 0.0))
-    return fail(SWARM_ERR_INVALID_ARG, "invalid Adam hyper-parameter");     // torch.optim.Adam's ValueError checks
+  if (int rc = validate_adam(lr, beta1, beta2, eps)) return rc;
   return check_cuda(launch_stack_adam_clip(*spec, weights, grad, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_norm,
                                            target_weights, grad_norm, (cudaStream_t)stream),
                     "swarm_adam_clip_stack_step");
@@ -967,14 +949,7 @@ int swarm_adam_clip_stack_step(const SwarmStackSpec* spec, float* weights, const
 
 int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg) {
   if (!cfg || cfg->num_envs <= 0 || cfg->n_agents <= 0) return 0;
-  const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
-  if (cfg->n_agents > kTileThreads) {
-    // actions, topk table (kNN), then the large forward's workspace at the widest layer (hidden 32)
-    const int64_t k = cfg->graph_mode == SWARM_GRAPH_KNN ? (cfg->knn_k > 0 ? cfg->knn_k : 0) : 0;
-    return 256 + ((bn * 4 + bn * k * 4 + 255) & ~(int64_t)255) + stack_large_workspace_bytes(*cfg, 32);
-  }
-  // the n_agents <= 128 rollout is one launch that does not touch the workspace; this size is kept as the ABI states it
-  return bn * 4 + bn * 4 + bn + 1024;
+  return rollout_stack_workspace(*cfg).bytes;
 }
 
 // the Flocking / Cohesion reward of the n_agents <= 128 stacked tick (reward == NULL: the world's own): checked, and
@@ -982,32 +957,22 @@ int64_t swarm_rollout_stack_workspace_bytes(const SwarmConfig* cfg) {
 static int stack_reward(const SwarmConfig* cfg, const SwarmRewardSpec* reward, const float* shaping, SwarmRewardSpec& rs) {
   if (!reward) return SWARM_OK;
   rs = *reward;
-  if (rs.kind != SWARM_REWARD_FLOCKING && rs.kind != SWARM_REWARD_COHESION)
-    return fail(SWARM_ERR_INVALID_ARG, "unknown reward kind");
-  if (cfg->scenario != SWARM_SCENARIO_GOTO)
-    return fail(SWARM_ERR_INVALID_ARG, "the Flocking / Cohesion rewards run on the GoTo world (cfg->scenario)");
-  if (rs.num_envs != cfg->num_envs || rs.n_agents != cfg->n_agents)
-    return fail(SWARM_ERR_INVALID_ARG, "reward spec and cfg disagree on num_envs / n_agents");
-  if (rs.n_agents < 2) return fail(SWARM_ERR_INVALID_ARG, "the scenario rewards need at least two agents");
-  if (rs.kind == SWARM_REWARD_FLOCKING && !shaping) return fail(SWARM_ERR_INVALID_ARG, "Flocking needs the shaping buffer");
-  if (rs.kind == SWARM_REWARD_COHESION && !(rs.sigma > 0.0f)) return fail(SWARM_ERR_INVALID_ARG, "sigma must be > 0");
   rs.reset = 0;
   rs.env_index = -1;
-  return SWARM_OK;
+  if (rs.kind != SWARM_REWARD_FLOCKING && rs.kind != SWARM_REWARD_COHESION)
+    return fail(SWARM_ERR_INVALID_ARG, "unknown reward kind");
+  if (int rc = validate_reward_cfg(cfg, rs, true)) return rc;
+  return validate_reward_buffers(rs, shaping, false, nullptr);
 }
 
 // n_agents > 128: per tick [topk table ->] the large stacked forward (argmax) -> the large world step with returns / hits;
 // rs != nullptr: the world step counts the hits only, and the large scenario reward adds the tick's reward to returns
-// (its per-agent terms in reward_ws)
+// (its per-agent terms in w.reward)
 static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
-                               int32_t ticks, float* returns, int32_t* hits, void* workspace, cudaStream_t st,
-                               const SwarmRewardSpec* rs = nullptr, float* shaping = nullptr, void* reward_ws = nullptr) {
-  const int64_t bn = (int64_t)cfg->num_envs * cfg->n_agents;
+                               int32_t ticks, float* returns, int32_t* hits, const RolloutWorkspace& w, cudaStream_t st,
+                               const SwarmRewardSpec* rs = nullptr, float* shaping = nullptr) {
   const bool knn = cfg->graph_mode == SWARM_GRAPH_KNN;
-  uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
-  int32_t* actions = reinterpret_cast<int32_t*>(base);
-  int32_t* nbr = actions + bn;
-  void* fwd_ws = reinterpret_cast<void*>(base + ((bn * 4 + (knn ? bn * cfg->knn_k * 4 : 0) + 255) & ~(int64_t)255));
+  int32_t *actions = w.actions, *nbr = w.nbr;
   // in place: one CTA owns a whole env and stages its positions first
   SimStepArgs p = step_args(*cfg, state, actions, state);
   p.returns = rs ? nullptr : returns;
@@ -1016,12 +981,12 @@ static int rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spe
     if (knn)
       if (cudaError_t e = launch_graph_large(*cfg, state, nullptr, nbr, (int)swarm_edges_per_env(cfg), st); e != cudaSuccess)
         return check_cuda(e, "swarm_rollout_stack (graph)");
-    if (cudaError_t e = launch_gatstack_large(*cfg, *spec, weights, state, knn ? nbr : nullptr, nullptr, actions, fwd_ws, st);
+    if (cudaError_t e = launch_gatstack_large(*cfg, *spec, weights, state, knn ? nbr : nullptr, nullptr, actions, w.forward, st);
         e != cudaSuccess)
       return check_cuda(e, "swarm_rollout_stack (forward)");
     if (cudaError_t e = launch_sim_step_large(p, st); e != cudaSuccess) return check_cuda(e, "swarm_rollout_stack (step)");
     if (rs)
-      if (cudaError_t e = launch_scenario_reward_large(*rs, state, shaping, nullptr, nullptr, returns, reward_ws, st);
+      if (cudaError_t e = launch_scenario_reward_large(*rs, state, shaping, nullptr, nullptr, returns, w.reward, st);
           e != cudaSuccess)
         return check_cuda(e, "swarm_rollout_stack_large (reward)");
   }
@@ -1038,8 +1003,9 @@ int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, cons
                                        "(larger swarms: reward = NULL, the world's own reward)");
   if (!weights || !state || !workspace) return fail(SWARM_ERR_INVALID_ARG, "weights/state/workspace is NULL");
   if (ticks < 0) return fail(SWARM_ERR_INVALID_ARG, "ticks must be >= 0");
-  if (workspace_bytes < swarm_rollout_stack_workspace_bytes(cfg)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  if (large) return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, workspace, (cudaStream_t)stream);
+  const RolloutWorkspace w = rollout_stack_workspace(*cfg, workspace);
+  if (workspace_bytes < w.bytes) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  if (large) return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, w, (cudaStream_t)stream);
   SwarmRewardSpec rs;
   if (int rc = stack_reward(cfg, reward, shaping, rs)) return rc;
   // the whole loop is ONE launch with the state in registers (stack_kernels.cu gatstack_kernel<HP, true>)
@@ -1050,13 +1016,7 @@ int swarm_rollout_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, cons
 
 int64_t swarm_rollout_stack_large_workspace_bytes(const SwarmConfig* cfg, const SwarmRewardSpec* reward) {
   if (!cfg || cfg->num_envs <= 0 || cfg->n_agents <= kTileThreads || cfg->n_agents > kMaxLargeAgents) return 0;
-  // swarm_rollout_stack's layout, then (reward) the per-agent terms of the large scenario reward, 256-byte aligned
-  const int64_t base = swarm_rollout_stack_workspace_bytes(cfg);
-  if (!reward) return base;
-  SwarmRewardSpec rs = *reward;
-  rs.num_envs = cfg->num_envs;
-  rs.n_agents = cfg->n_agents;
-  return base + 256 + scenario_reward_large_workspace_bytes(rs);
+  return rollout_stack_large_workspace(*cfg, reward).bytes;
 }
 
 int swarm_rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec, const float* weights, float* state,
@@ -1072,15 +1032,10 @@ int swarm_rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec
   if (int rc = stack_reward(cfg, reward, shaping, rs)) return rc;
   if (reward && (int64_t)cfg->num_envs * cfg->n_agents >= (1LL << 31))
     return fail(SWARM_ERR_UNSUPPORTED, "num_envs * n_agents must stay below 2^31");
-  if (workspace_bytes < swarm_rollout_stack_large_workspace_bytes(cfg, reward))
-    return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  void* reward_ws = nullptr;
-  if (reward) {
-    const uintptr_t at = reinterpret_cast<uintptr_t>(workspace) + (uintptr_t)swarm_rollout_stack_workspace_bytes(cfg);
-    reward_ws = reinterpret_cast<void*>((at + 255) & ~(uintptr_t)255);
-  }
-  return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, workspace, (cudaStream_t)stream,
-                             reward ? &rs : nullptr, shaping, reward_ws);
+  const RolloutWorkspace w = rollout_stack_large_workspace(*cfg, reward, workspace);
+  if (workspace_bytes < w.bytes) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  return rollout_stack_large(cfg, spec, weights, state, ticks, returns, hits, w, (cudaStream_t)stream,
+                             reward ? &rs : nullptr, shaping);
 }
 
 int swarm_train_tick_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
@@ -1089,15 +1044,14 @@ int swarm_train_tick_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, c
                            int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
                            int64_t workspace_bytes, void* stream) {
   if (int rc = validate_hyper(hyper)) return rc;
-  if (int rc = validate_stack(cfg, spec)) return rc;
+  if (int rc = validate_stack(cfg, spec)) return rc;      // the caller's cfg: its own num_envs must be positive
+  if (int rc = validate_stack_grad(*cfg, *spec)) return rc;
   const int G = hyper->graphs_per_update;
-  if (int rc = validate_dqn_stack(cfg, spec, G)) return rc;
   if (hyper->flocking)
     return fail(SWARM_ERR_INVALID_ARG, "hyper->flocking must be NULL: the stacked tick takes its reward as `reward`");
   if (!ctl || !weights || !target_weights || !exp_avg || !exp_avg_sq || !state || !grad || !workspace)
     return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
-  if (!ring || !ring->state || !ring->next_state || !ring->actions || !ring->rewards || ring->capacity <= 0)
-    return fail(SWARM_ERR_INVALID_ARG, "replay ring has NULL arrays or no capacity");
+  if (int rc = validate_ring(ring, "replay ring", true)) return rc;
   if (cfg->num_envs > ring->capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
   if (workspace_bytes < stack_grad_workspace_bytes(*cfg, *spec, G)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
   SwarmRewardSpec rs;

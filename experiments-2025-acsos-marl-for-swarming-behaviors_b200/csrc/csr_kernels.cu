@@ -6,6 +6,7 @@
 #include <string>
 
 #include "gatq_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

@@ -8,6 +8,7 @@
 #include <cooperative_groups.h>
 
 #include "dqn_common.cuh"
+#include "launchers.h"
 
 namespace swarm {
 
@@ -779,8 +780,6 @@ __global__ void __launch_bounds__(kTileThreads) csr_bwd_source_kernel(const __gr
   }
 }
 
-cudaError_t launch_csr_project(int n, const float* weights, const float* x, float* rows, cudaStream_t stream);
-
 static size_t bwd_align(size_t v) { return (v + 255) & ~(size_t)255; }
 
 long long gatq_backward_workspace_bytes(int n, long long E) {
@@ -866,8 +865,6 @@ long long dqn_workspace_bytes(const SwarmConfig& c, int n_graphs) {
   const long long ctas = (n_graphs + epb - 1) / epb;
   return ctas * kPartialStride * 4 + 256;
 }
-
-cudaError_t launch_dqn_grad_tc(DqnParams& p, cudaStream_t stream);
 
 cudaError_t launch_dqn_grad(const SwarmConfig& c, const float* w_online, const float* w_target, const SwarmReplay& batch,
                             const int64_t* indices, int n_graphs, float gamma, float loss_scale, float* grad, float* loss,

@@ -21,6 +21,7 @@
 // the CTA needs 2 x 5 KB of staging per warp instead of six 18 KB tiles.
 #include "dqn_common.cuh"
 #include "tile_tc_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

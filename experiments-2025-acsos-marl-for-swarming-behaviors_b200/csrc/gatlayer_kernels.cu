@@ -17,6 +17,7 @@
 
 #include "gatq_device.cuh"
 #include "swarm_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

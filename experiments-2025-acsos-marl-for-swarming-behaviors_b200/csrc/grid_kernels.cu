@@ -19,6 +19,7 @@
 
 #include "gatq_device.cuh"
 #include "grid_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

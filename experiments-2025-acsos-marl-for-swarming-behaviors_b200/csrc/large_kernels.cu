@@ -15,6 +15,7 @@
 #include "knn_select.h"
 #include "knn_small.h"
 #include "gatq_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 
@@ -596,9 +597,6 @@ cudaError_t launch_gatq_knn_large(const SwarmConfig& c, const float* weights, co
 }
 
 // ---- launchers ------------------------------------------------------------------------------
-bool sim_step_grid_enabled(int n_agents);
-cudaError_t launch_sim_step_grid(const SimStepArgs& p, cudaStream_t stream);
-
 cudaError_t launch_sim_step_large(const SimStepArgs& p, cudaStream_t stream) {
   const SwarmConfig& c = p.cfg;
   // contact partners from the uniform grid (grid_kernels.cu; same bits) unless SWARM_STEP_GRID=0 asks for the full sweep

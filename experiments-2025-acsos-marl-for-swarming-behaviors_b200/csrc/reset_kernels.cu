@@ -1,6 +1,7 @@
 // reset_kernels.cu -- generate_grid + reset_world_at (go_to_position_scenario.py:52-106,
 // obstacle_avoidance_scenario.py:63-133): one thread per agent, float4 state writes.
 #include "tile_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

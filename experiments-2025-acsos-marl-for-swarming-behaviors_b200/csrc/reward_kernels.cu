@@ -12,6 +12,7 @@
 #include <cstdint>
 
 #include "swarm_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

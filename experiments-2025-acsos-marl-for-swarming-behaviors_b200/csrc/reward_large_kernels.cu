@@ -13,6 +13,7 @@
 #include <cstdint>
 
 #include "swarm_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

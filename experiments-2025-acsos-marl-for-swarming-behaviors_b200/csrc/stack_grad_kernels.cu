@@ -15,6 +15,7 @@
 
 #include "dqn_common.cuh"
 #include "stack_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

@@ -15,6 +15,7 @@
 #include <cstring>
 
 #include "stack_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

@@ -22,6 +22,7 @@
 
 #include "grid_device.cuh"
 #include "stack_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

@@ -18,6 +18,7 @@
 //                           16-byte-aligned bursts only.
 #include "tile_kernels.cuh"
 #include "tc_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

@@ -11,6 +11,7 @@
 // so the stand-alone kernels and the fused rollout are consistent by construction.  The rollout's world step is the
 // agent_step of swarm_device.cuh, which the stand-alone world-step kernels (step_kernels.cu) run as well.
 #include "tile_tc_device.cuh"
+#include "launchers.h"
 
 namespace swarm {
 

@@ -7,7 +7,6 @@ is computed in PyTorch.
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import Dict, Optional, Tuple
 
 import torch
@@ -921,27 +920,30 @@ def rollout_large(cfg: SwarmConfig, weights: torch.Tensor, state: torch.Tensor, 
     offs = (torch.arange(B, device=dev, dtype=torch.int64) * N).view(B, 1, 1)
     trace = []
     static_csr = None
-    fused_knn = cfg.graph_mode == _lib.GRAPH_KNN and N * (144 + 4 * cfg.knn_k) + 8192 <= 227 * 1024 and fused
-    # swarm_rollout_large attends in input space unless SWARM_TC=0 (no projected-feature tile: envs up to 4 096 agents)
-    xspace = os.environ.get("SWARM_TC", "1")[:1] != "0"
-    lib_loop = fused and cfg.graph_mode == _lib.GRAPH_KNN and N > 128 and 64 * cfg.knn_k <= N and not trace_state and \
-        (N * (28 + 2 * cfg.knn_k) + 8400 <= 227 * 1024 if xspace else fused_knn)
-    # radius / complete graph: the library forward finds its own sources (uniform grid / every other agent), no edge list
-    lib_loop = lib_loop or (fused and cfg.graph_mode != _lib.GRAPH_KNN and 128 < N <= 4096 and not trace_state)
-    if lib_loop:
-        # the whole tick sequence from the library (swarm_rollout_large): topk table -> per-env Q + argmax -> world step
-        # with returns / hits accumulated by the step kernel; no tensor op between the launches
+    if fused and not trace_state and 128 < N <= 4096:
+        # the whole tick sequence from the library (swarm_rollout_large): [topk table ->] per-env Q + argmax -> world
+        # step with returns / hits accumulated by the step kernel; no tensor op between the launches.  The library
+        # refuses a swarm its kernels do not take (SWARM_ERR_UNSUPPORTED) before it launches anything.
         wb = int(lib().swarm_rollout_large_workspace_bytes(C.byref(cfg)))
         ws = torch.empty(wb, dtype=torch.uint8, device=dev)
-        check(lib().swarm_rollout_large(C.byref(cfg), ptr(weights), ptr(state), int(ticks), ptr(returns), ptr(hits), ptr(ws),
-                                        wb, stream_ptr(dev)))
-        return {"state": state, "returns": returns, "hits": hits}
+        rc = lib().swarm_rollout_large(C.byref(cfg), ptr(weights), ptr(state), int(ticks), ptr(returns), ptr(hits), ptr(ws),
+                                       wb, stream_ptr(dev))
+        if rc != _lib.ERR_UNSUPPORTED:
+            check(rc)
+            return {"state": state, "returns": returns, "hits": hits}
+    # kNN: the per-env fused forward straight from the topk table while the library takes the env, else the CSR path
+    fused_knn = fused and cfg.graph_mode == _lib.GRAPH_KNN
     nbr = torch.empty(B, N, cfg.knn_k, dtype=torch.int32, device=dev) if fused_knn else None
+    act = torch.empty(B, N, dtype=torch.int32, device=dev) if fused_knn else None
     for _ in range(ticks):
         if fused_knn:
             # topk table only (no edge list), then the per-env fused forward
             check(lib().swarm_graph_build(C.byref(cfg), ptr(state), None, ptr(nbr), stream_ptr(dev)))
-            act = gatq_forward_knn_large(cfg, weights, state, nbr, want_q=False, want_actions=True)
+            rc = lib().swarm_gatq_forward_knn_large(C.byref(cfg), ptr(weights), ptr(state), ptr(nbr), None, ptr(act),
+                                                    stream_ptr(dev))
+            fused_knn = rc != _lib.ERR_UNSUPPORTED
+        if fused_knn:
+            check(rc)
             out = sim_step(cfg, state, act, state_out=state, want_obs=False)
             returns += out["rewards"]
             hits += ((out["flags"] & _lib.FLAG_HIT) != 0).sum(dim=1, dtype=torch.int32)
