@@ -22,9 +22,10 @@ FLAG_OBSTACLE_CONTACT = 1
 FLAG_HIT = 2
 FLAG_PENALTY = 4
 W_COUNT = 1673
-ABI_VERSION = 8
+ABI_VERSION = 9
 ERR_UNSUPPORTED = -2     # SWARM_ERR_UNSUPPORTED: the library does not implement this call's shape
 XCHG_STRIDE = 1680
+XCHG_STACK_STRIDE = 5040
 
 # state-dict tensors in packed order (include/swarm_b200.h SWARM_W_*)
 WEIGHT_KEYS = ("conv1.lin.weight", "conv1.att_src", "conv1.att_dst", "conv1.bias",
@@ -189,6 +190,11 @@ _SIGNATURES = {
     "swarm_train_tick_stack": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.POINTER(SwarmTrainHyper)]
                                + [C.c_void_p] * 10 + [C.POINTER(SwarmReplay)] + [C.c_void_p] * 3
                                + [C.c_int64, C.c_void_p]),
+    "swarm_train_tick_stack_grad": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec), C.POINTER(SwarmTrainHyper)]
+                                    + [C.c_void_p] * 8 + [C.POINTER(SwarmReplay)] + [C.c_void_p] * 3
+                                    + [C.c_int64, C.POINTER(SwarmPeerExchange), C.c_void_p]),
+    "swarm_train_tick_stack_apply": (C.c_int, [C.POINTER(SwarmConfig), C.POINTER(SwarmStackSpec),
+                                               C.POINTER(SwarmTrainHyper)] + [C.c_void_p] * 6 + [C.c_int64, C.c_void_p]),
 }
 
 

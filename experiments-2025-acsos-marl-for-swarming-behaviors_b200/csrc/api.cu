@@ -1038,40 +1038,100 @@ int swarm_rollout_stack_large(const SwarmConfig* cfg, const SwarmStackSpec* spec
                              reward ? &rs : nullptr, shaping);
 }
 
+// the checks of swarm_train_tick_stack and of its grad phase, in swarm_train_tick_stack's order (no_moments: the apply
+// phase's exp_avg / exp_avg_sq are missing, reported with the other NULL arguments), and the reward spec copied into rs
+static int validate_tick_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                               const SwarmRewardSpec* reward, const float* shaping, const SwarmTrainCtl* ctl,
+                               const float* weights, const float* target_weights, bool no_moments, const float* state,
+                               const SwarmReplay* ring, const float* grad, const void* workspace, int64_t workspace_bytes,
+                               SwarmRewardSpec& rs) {
+  if (int rc = validate_hyper(hyper)) return rc;
+  if (int rc = validate_stack(cfg, spec)) return rc;      // the caller's cfg: its own num_envs must be positive
+  if (int rc = validate_stack_grad(*cfg, *spec)) return rc;
+  if (hyper->flocking)
+    return fail(SWARM_ERR_INVALID_ARG, "hyper->flocking must be NULL: the stacked tick takes its reward as `reward`");
+  if (!ctl || !weights || !target_weights || no_moments || !state || !grad || !workspace)
+    return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
+  if (int rc = validate_ring(ring, "replay ring", true)) return rc;
+  if (cfg->num_envs > ring->capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
+  if (workspace_bytes < stack_grad_workspace_bytes(*cfg, *spec, hyper->graphs_per_update))
+    return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
+  return stack_reward(cfg, reward, shaping, rs);
+}
+
+// launches 1-3 of the stacked tick (peers != NULL: the reduce launch sums grad / loss over the ranks)
+static int tick_stack_grad(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                           const SwarmRewardSpec* rs, float* shaping, SwarmTrainCtl* ctl, const float* weights,
+                           const float* target_weights, float* state, float* returns, int32_t* hits, const SwarmReplay* ring,
+                           int64_t* indices, float* grad, void* workspace, const SwarmPeerExchange* peers, cudaStream_t st,
+                           const char* what_rollout, const char* what_grad) {
+  float* loss = grad + stack_weight_count_host(*spec);
+  if (int rc = check_cuda(launch_gatstack_train_tick(*cfg, *spec, weights, state, world_consts(*cfg), rs, shaping, returns,
+                                                     hits, *ring, ctl, hyper->rng_seed, hyper->env_offset, st),
+                          what_rollout))
+    return rc;
+  return check_cuda(launch_stack_grad(*cfg, *spec, weights, target_weights, *ring, nullptr, hyper->graphs_per_update,
+                                      hyper->gamma, hyper->loss_scale, grad, loss, nullptr, workspace, st, ctl, indices,
+                                      hyper->sample_seed, cfg->num_envs, peers),
+                    what_grad);
+}
+
+// launch 4 of the stacked tick
+static int tick_stack_apply(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                            SwarmTrainCtl* ctl, float* weights, float* target_weights, float* exp_avg, float* exp_avg_sq,
+                            const float* grad, int64_t ring_capacity, cudaStream_t st, const char* what) {
+  return check_cuda(launch_stack_adam_clip(*spec, weights, grad, exp_avg, exp_avg_sq, 1, hyper->lr, hyper->beta1,
+                                           hyper->beta2, hyper->eps, hyper->max_norm, target_weights, nullptr, st, ctl,
+                                           cfg->num_envs, ring_capacity, hyper->update_target_every),
+                    what);
+}
+
 int swarm_train_tick_stack(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
                            const SwarmRewardSpec* reward, float* shaping, SwarmTrainCtl* ctl, float* weights,
                            float* target_weights, float* exp_avg, float* exp_avg_sq, float* state, float* returns,
                            int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
                            int64_t workspace_bytes, void* stream) {
+  SwarmRewardSpec rs;
+  if (int rc = validate_tick_stack(cfg, spec, hyper, reward, shaping, ctl, weights, target_weights, !exp_avg || !exp_avg_sq,
+                                   state, ring, grad, workspace, workspace_bytes, rs))
+    return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = tick_stack_grad(cfg, spec, hyper, reward ? &rs : nullptr, shaping, ctl, weights, target_weights, state,
+                               returns, hits, ring, indices, grad, workspace, nullptr, st, "swarm_train_tick_stack(rollout)",
+                               "swarm_train_tick_stack(grad)"))
+    return rc;
+  return tick_stack_apply(cfg, spec, hyper, ctl, weights, target_weights, exp_avg, exp_avg_sq, grad, ring->capacity, st,
+                          "swarm_train_tick_stack(apply)");
+}
+
+int swarm_train_tick_stack_grad(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                                const SwarmRewardSpec* reward, float* shaping, SwarmTrainCtl* ctl, const float* weights,
+                                const float* target_weights, float* state, float* returns, int32_t* hits,
+                                const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
+                                int64_t workspace_bytes, const SwarmPeerExchange* peers, void* stream) {
+  SwarmRewardSpec rs;
+  if (int rc = validate_tick_stack(cfg, spec, hyper, reward, shaping, ctl, weights, target_weights, false, state, ring,
+                                   grad, workspace, workspace_bytes, rs))
+    return rc;
+  if (int rc = validate_peers(peers)) return rc;
+  return tick_stack_grad(cfg, spec, hyper, reward ? &rs : nullptr, shaping, ctl, weights, target_weights, state, returns,
+                         hits, ring, indices, grad, workspace, peers, (cudaStream_t)stream,
+                         "swarm_train_tick_stack_grad(rollout)", "swarm_train_tick_stack_grad(grad)");
+}
+
+int swarm_train_tick_stack_apply(const SwarmConfig* cfg, const SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                                 SwarmTrainCtl* ctl, float* weights, float* target_weights, float* exp_avg,
+                                 float* exp_avg_sq, const float* grad, int64_t ring_capacity, void* stream) {
   if (int rc = validate_hyper(hyper)) return rc;
-  if (int rc = validate_stack(cfg, spec)) return rc;      // the caller's cfg: its own num_envs must be positive
+  if (int rc = validate_stack(cfg, spec)) return rc;
   if (int rc = validate_stack_grad(*cfg, *spec)) return rc;
-  const int G = hyper->graphs_per_update;
   if (hyper->flocking)
     return fail(SWARM_ERR_INVALID_ARG, "hyper->flocking must be NULL: the stacked tick takes its reward as `reward`");
-  if (!ctl || !weights || !target_weights || !exp_avg || !exp_avg_sq || !state || !grad || !workspace)
+  if (!ctl || !weights || !target_weights || !exp_avg || !exp_avg_sq || !grad)
     return fail(SWARM_ERR_INVALID_ARG, "NULL argument");
-  if (int rc = validate_ring(ring, "replay ring", true)) return rc;
-  if (cfg->num_envs > ring->capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
-  if (workspace_bytes < stack_grad_workspace_bytes(*cfg, *spec, G)) return fail(SWARM_ERR_INVALID_ARG, "workspace too small");
-  SwarmRewardSpec rs;
-  if (int rc = stack_reward(cfg, reward, shaping, rs)) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  float* loss = grad + stack_weight_count_host(*spec);
-  if (int rc = check_cuda(launch_gatstack_train_tick(*cfg, *spec, weights, state, world_consts(*cfg), reward ? &rs : nullptr,
-                                                     shaping, returns, hits, *ring, ctl, hyper->rng_seed, hyper->env_offset,
-                                                     st),
-                          "swarm_train_tick_stack(rollout)"))
-    return rc;
-  if (int rc = check_cuda(launch_stack_grad(*cfg, *spec, weights, target_weights, *ring, nullptr, G, hyper->gamma,
-                                            hyper->loss_scale, grad, loss, nullptr, workspace, st, ctl, indices,
-                                            hyper->sample_seed, cfg->num_envs),
-                          "swarm_train_tick_stack(grad)"))
-    return rc;
-  return check_cuda(launch_stack_adam_clip(*spec, weights, grad, exp_avg, exp_avg_sq, 1, hyper->lr, hyper->beta1,
-                                           hyper->beta2, hyper->eps, hyper->max_norm, target_weights, nullptr, st, ctl,
-                                           cfg->num_envs, ring->capacity, hyper->update_target_every),
-                    "swarm_train_tick_stack(apply)");
+  if (cfg->num_envs > ring_capacity) return fail(SWARM_ERR_INVALID_ARG, "num_envs exceeds the replay capacity");
+  return tick_stack_apply(cfg, spec, hyper, ctl, weights, target_weights, exp_avg, exp_avg_sq, grad, ring_capacity,
+                          (cudaStream_t)stream, "swarm_train_tick_stack_apply");
 }
 
 int swarm_episode_end(const SwarmConfig* cfg, SwarmTrainCtl* ctl, float* returns, int32_t* hits, const float* loss,

@@ -65,5 +65,17 @@ __device__ __forceinline__ void adam_element(const AdamScalars& a, float g, floa
   v_io = v;
 }
 
+// the peer-memory gradient exchange of the data-parallel ticks (adam_clip_kernel<true> / reduce_clip_adam_kernel<true>
+// in dqn_kernels.cu, stack_reduce_peers_kernel in stack_grad_kernels.cu): one naturally aligned 64-bit word =
+// (epoch << 32 | float bits) is single-copy atomic, so the word itself is the flag
+__device__ __forceinline__ void st_relaxed_sys_u64(uint64_t* p, uint64_t v) {
+  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ uint64_t ld_relaxed_sys_u64(const uint64_t* p) {
+  uint64_t v;
+  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+
 }  // namespace swarm
 #endif

@@ -217,16 +217,6 @@ __device__ __forceinline__ float clip_coefficient(const float (&g_)[kAdamPer], d
   return s_coef;
 }
 
-// one naturally aligned 64-bit word = (epoch << 32 | float bits): single-copy atomic, so the word itself is the flag
-__device__ __forceinline__ void st_relaxed_sys_u64(uint64_t* p, uint64_t v) {
-  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint64_t ld_relaxed_sys_u64(const uint64_t* p) {
-  uint64_t v;
-  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-
 // PEERS: with the fused peer-memory all-reduce (its register arrays and system-scope loads would otherwise slow the
 // single-GPU kernel from 5.4 to 7.6 us)
 template <bool PEERS>

@@ -121,7 +121,8 @@ cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, 
                               const SwarmReplay& batch, const int64_t* indices, int n_graphs, float gamma, float loss_scale,
                               float* grad, float* loss, float* td, void* workspace, cudaStream_t stream,
                               SwarmTrainCtl* ctl = nullptr, int64_t* indices_out = nullptr,
-                              unsigned long long sample_seed = 0, int pushed_envs = 0);
+                              unsigned long long sample_seed = 0, int pushed_envs = 0,
+                              const SwarmPeerExchange* peers = nullptr);
 cudaError_t launch_stack_adam_clip(const SwarmStackSpec& spec, float* w, const float* grad, float* m, float* v,
                                    long long step, double lr, double beta1, double beta2, double eps, double max_norm,
                                    float* target, float* grad_norm, cudaStream_t stream, SwarmTrainCtl* ctl = nullptr,

@@ -404,13 +404,19 @@ __global__ void __launch_bounds__(kTileThreads, HP == 8 ? 5 : 0) stack_grad_ctl_
   stack_grad_body<HP, true>(p);
 }
 
-// grad[o] = sum over CTAs (in CTA order) of partials[cta][o]; loss = loss_scale * sum of squared TD errors
+// sum over CTAs (in CTA order) of partials[cta][o]
+__device__ __forceinline__ float stack_partial_sum(const float* __restrict__ partials, int n_ctas, int stride, int o) {
+  float acc = 0.0f;
+  for (int b = 0; b < n_ctas; ++b) acc = __fadd_rn(acc, partials[(long long)b * stride + o]);
+  return acc;
+}
+
+// grad[o] = the CTA-order sum of the partials; loss = loss_scale * sum of squared TD errors
 __device__ __forceinline__ void stack_reduce_element(const float* __restrict__ partials, int n_ctas, int stride, int count,
                                                      float loss_scale, float* __restrict__ grad, float* __restrict__ loss,
                                                      int o) {
   if (o > count) return;
-  float acc = 0.0f;
-  for (int b = 0; b < n_ctas; ++b) acc = __fadd_rn(acc, partials[(long long)b * stride + o]);
+  const float acc = stack_partial_sum(partials, n_ctas, stride, o);
   if (o < count) grad[o] = acc;
   else loss[0] = __fmul_rn(acc, loss_scale);
 }
@@ -422,16 +428,72 @@ __global__ void __launch_bounds__(256) stack_reduce_kernel(const float* __restri
 }
 
 // device-driven tick: publishes whether this tick updates (read by the clip + Adam kernel) and leaves grad / loss
-// untouched when it does not (as dqn_reduce_kernel)
-__global__ void __launch_bounds__(256) stack_reduce_ctl_kernel(const float* __restrict__ partials, int n_ctas, int stride,
-                                                               int count, float loss_scale, float* __restrict__ grad,
-                                                               float* __restrict__ loss, SwarmTrainCtl* __restrict__ ctl,
-                                                               int pushed_envs, long long capacity, int n_graphs) {
+// untouched when it does not (as dqn_reduce_kernel).
+// PEERS: the data-parallel tick -- the one-shot PUSH all-reduce of reduce_clip_adam_kernel<true> (dqn_kernels.cu) over
+// NVLink peer memory, one gradient element per thread after the CTA-order sum: the thread writes its word
+// (epoch = tick + 1 << 32 | float bits) into slot [parity of the epoch][own rank][o] of every rank's buffer, own buffer
+// first, then in ring order; polls its own buffer's [parity][r][o] for every rank r; and sums the ranks in rank order,
+// so every rank holds the same bits.  Every rank agrees on `upd` (equal shards, same ring fill), so either all ranks
+// exchange this tick or none does.  A separate template value so that the one-GPU kernel keeps its code.
+template <bool PEERS>
+__device__ __forceinline__ void stack_reduce_ctl_body(const float* __restrict__ partials, int n_ctas, int stride, int count,
+                                                      float loss_scale, float* __restrict__ grad, float* __restrict__ loss,
+                                                      SwarmTrainCtl* __restrict__ ctl, int pushed_envs, long long capacity,
+                                                      int n_graphs, const SwarmPeerExchange* peers) {
   const int o = blockIdx.x * blockDim.x + threadIdx.x;
   const bool upd = train_ring_size(ctl, pushed_envs, capacity) >= n_graphs;
   if (o == 0) ctl->updating = upd ? 1 : 0;
   if (!upd) return;
-  stack_reduce_element(partials, n_ctas, stride, count, loss_scale, grad, loss, o);
+  if (!PEERS) {
+    stack_reduce_element(partials, n_ctas, stride, count, loss_scale, grad, loss, o);
+    return;
+  }
+  if (o > count) return;
+  float g = stack_partial_sum(partials, n_ctas, stride, o);
+  if (o == count) g = __fmul_rn(g, loss_scale);
+  const uint32_t epoch = (uint32_t)(ctl->tick + 1);
+  const int W = peers->world_size, rank = peers->rank;
+  const size_t par_base = (size_t)(epoch & 1u) * W * SWARM_XCHG_STACK_STRIDE;
+  const uint64_t word = ((uint64_t)epoch << 32) | (uint64_t)__float_as_uint(g);
+  for (int q = 0; q < W; ++q) {
+    const int peer = (rank + q) % W;                      // own buffer first, then ring order: spreads the links
+    st_relaxed_sys_u64(peers->data[peer] + par_base + (size_t)rank * SWARM_XCHG_STACK_STRIDE + o, word);
+  }
+  const uint64_t* mine = peers->data[rank] + par_base + o;
+  uint64_t got[SWARM_MAX_PEERS];
+  bool ok = false;
+  for (long long it = 0; it < (1ll << 26) && !ok; ++it) {      // bounded: a lost peer traps instead of hanging
+    ok = true;
+#pragma unroll
+    for (int r = 0; r < SWARM_MAX_PEERS; ++r)
+      got[r] = (r < W) ? ld_relaxed_sys_u64(mine + (size_t)r * SWARM_XCHG_STACK_STRIDE) : ((uint64_t)epoch << 32);
+#pragma unroll
+    for (int r = 0; r < SWARM_MAX_PEERS; ++r) ok = ok && ((uint32_t)(got[r] >> 32) == epoch);
+  }
+  if (!ok) __trap();
+  g = 0.0f;
+#pragma unroll
+  for (int r = 0; r < SWARM_MAX_PEERS; ++r)
+    if (r < W) g = __fadd_rn(g, __uint_as_float((uint32_t)got[r]));     // rank order
+  if (o < count) grad[o] = g;
+  else loss[0] = g;
+}
+
+__global__ void __launch_bounds__(256) stack_reduce_ctl_kernel(const float* __restrict__ partials, int n_ctas, int stride,
+                                                               int count, float loss_scale, float* __restrict__ grad,
+                                                               float* __restrict__ loss, SwarmTrainCtl* __restrict__ ctl,
+                                                               int pushed_envs, long long capacity, int n_graphs) {
+  stack_reduce_ctl_body<false>(partials, n_ctas, stride, count, loss_scale, grad, loss, ctl, pushed_envs, capacity,
+                               n_graphs, nullptr);
+}
+
+__global__ void __launch_bounds__(256) stack_reduce_peers_kernel(const float* __restrict__ partials, int n_ctas, int stride,
+                                                                 int count, float loss_scale, float* __restrict__ grad,
+                                                                 float* __restrict__ loss, SwarmTrainCtl* __restrict__ ctl,
+                                                                 int pushed_envs, long long capacity, int n_graphs,
+                                                                 const __grid_constant__ SwarmPeerExchange peers) {
+  stack_reduce_ctl_body<true>(partials, n_ctas, stride, count, loss_scale, grad, loss, ctl, pushed_envs, capacity,
+                              n_graphs, &peers);
 }
 
 // ---- launchers -------------------------------------------------------------------------------------------------------
@@ -479,7 +541,8 @@ static cudaError_t launch_stack_grad_hp(const StackGradParams& p, int ctas, cuda
 cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, const float* w_online, const float* w_target,
                               const SwarmReplay& batch, const int64_t* indices, int n_graphs, float gamma, float loss_scale,
                               float* grad, float* loss, float* td, void* workspace, cudaStream_t stream,
-                              SwarmTrainCtl* ctl, int64_t* indices_out, unsigned long long sample_seed, int pushed_envs) {
+                              SwarmTrainCtl* ctl, int64_t* indices_out, unsigned long long sample_seed, int pushed_envs,
+                              const SwarmPeerExchange* peers) {
   StackGradParams p;
   std::memset(&p, 0, sizeof(p));
   p.ctl = ctl;
@@ -511,7 +574,10 @@ cudaError_t launch_stack_grad(const SwarmConfig& c, const SwarmStackSpec& spec, 
   }
   if (err != cudaSuccess) return err;
   const int blocks = (p.count + 1 + 255) / 256;
-  if (ctl)
+  if (ctl && peers)
+    stack_reduce_peers_kernel<<<blocks, 256, 0, stream>>>(p.partials, ctas, p.stride, p.count, loss_scale, grad, loss, ctl,
+                                                          pushed_envs, batch.capacity, n_graphs, *peers);
+  else if (ctl)
     stack_reduce_ctl_kernel<<<blocks, 256, 0, stream>>>(p.partials, ctas, p.stride, p.count, loss_scale, grad, loss, ctl,
                                                         pushed_envs, batch.capacity, n_graphs);
   else

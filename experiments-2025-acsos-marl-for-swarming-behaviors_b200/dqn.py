@@ -16,7 +16,8 @@ Two drivers:
 data/models/experiment_Flocking-seed_*.pth) instead of the one-layer GCN: ``train_model`` and ``train_model_stepwise``
 then run the stack's gradient kernel (``swarm_dqn_stack_grad``) and clip + Adam (``swarm_adam_clip_stack_step``), and
 ``train_model_stack_device`` is the stack's whole-run device loop -- one ``swarm_train_tick_stack`` call (four launches)
-per tick, one CUDA-graph replay per episode -- for the GoTo, ObstacleAvoidance, Flocking and Cohesion rewards on one GPU.
+per tick, one CUDA-graph replay per episode -- for the GoTo, ObstacleAvoidance, Flocking and Cohesion rewards, on one GPU
+or data-parallel over several (the gradient summed over the ranks through NVLink peer memory, or NCCL).
 """
 from __future__ import annotations
 
@@ -496,14 +497,15 @@ class DQNTrainer:
         False runs every episode eagerly), four launches per tick and no host synchronisation until the run ends.  The
         reward is the world's own (GoTo / ObstacleAvoidance), Flocking's (its shaping memory reset on the device with
         the world) or Cohesion's.  GoTo / ObstacleAvoidance / Flocking start from ``swarm_reset_random``; Cohesion starts
-        from its fixed table, so its reset is a device copy of the state one ``env.reset()`` leaves.  One GPU.  Returns
-        stats f32[episodes, 4] = (mean agent-0 return / N, hits per env, last loss, epsilon)."""
+        from its fixed table, so its reset is a device copy of the state one ``env.reset()`` leaves.  Data-parallel (one
+        process per GPU, envs sharded as in ``train_model_device``): G graphs per rank, the loss is the mean over the
+        global batch, and each tick is ``swarm_train_tick_stack_grad`` (which sums the gradient over the ranks through
+        NVLink peer memory) + ``swarm_train_tick_stack_apply``, with an NCCL all-reduce in between where peer memory is
+        unavailable or SWARM_PEER_ALLREDUCE=0; the weights stay identical on every rank.  Returns stats
+        f32[episodes, 4] = (mean agent-0 return / N, hits per env, last loss, epsilon)."""
         if self.stack_spec is None:
             raise NotImplementedError("train_model_stack_device trains a StackedGCN; the one-layer GCN has "
                                       "train_model_device")
-        if parallel.world_size() > 1:
-            raise NotImplementedError("train_model_stack_device runs on one GPU (data-parallel stacked training is not "
-                                      "implemented)")
         env, world = self.env, self.env.world
         flock = isinstance(env.scenario, FlockingScenario)
         cohesion = isinstance(env.scenario, CohesionScenario)
@@ -511,21 +513,24 @@ class DQNTrainer:
             raise NotImplementedError("the stacked device loop covers the GoTo, ObstacleAvoidance, Flocking and Cohesion "
                                       "rewards; train other scenarios with train_model_stepwise")
         B, n, dev = env.num_envs, env.n_agents, env.device
+        G = int(config.get("graphs_per_update", 32))
         episodes = int(config["episodes"])
+        ring = self.replay_buffer.ring
         cfg = ops.clone_config(self.graph_cfg, num_envs=B)
+        rank = torch.distributed.get_rank() if parallel.world_size() > 1 else 0
+        multi = parallel.world_size() > 1
         reward = shaping = None
         if flock:
             reward, shaping = env.scenario._spec(), env.scenario.shaping
         elif cohesion:
             reward = ops.reward_spec(_lib.REWARD_COHESION, B, n, agent_radius=world.cfg.agent_radius,
                                      sigma=env.scenario.sigma)
-        tt = ops.StackTrainTick(cfg, self.stack_spec, self.replay_buffer.ring,
-                                graphs_per_update=int(config.get("graphs_per_update", 32)),
+        tt = ops.StackTrainTick(cfg, self.stack_spec, ring, graphs_per_update=G,
                                 update_target_every=int(config.get("update_target_every", 200)),
-                                gamma=float(config.get("gamma", 0.99)), lr=self.lr, betas=self.betas, eps=self.eps,
-                                max_norm=self.max_norm, rng_seed=self.seed,
-                                sample_seed=int(config.get("sample_seed", self.seed)),
-                                env_offset=int(config.get("env_offset", 0)), reward=reward, shaping=shaping)
+                                gamma=float(config.get("gamma", 0.99)), loss_scale=parallel.global_loss_scale(G, n),
+                                lr=self.lr, betas=self.betas, eps=self.eps, max_norm=self.max_norm, rng_seed=self.seed,
+                                sample_seed=int(config.get("sample_seed", self.seed)) + 7919 * rank,
+                                env_offset=int(config.get("env_offset", rank * B)), reward=reward, shaping=shaping)
         if cohesion:
             env.reset()
             start = world.state.clone()
@@ -541,16 +546,26 @@ class DQNTrainer:
                 ops.reset_random(cfg, spec, world.state, ctl=tt.ctl)
                 if flock:
                     ops.scenario_reward(reward, world.state, shaping, reset=True)
+        parallel.require_equal_shards(B, ring.size, ring.position, ring.capacity, G)
+        parallel.broadcast_weights(self.w)
         self.w_target.copy_(self.w)
         tt.load_cursor(int(config.get("start_tick", 0)), self.opt_step, config["epsilon"], 0)
         returns = torch.zeros(B, n, dtype=torch.float32, device=dev)
         hits = torch.zeros(B, dtype=torch.int32, device=dev)
         stats = torch.zeros(episodes, 4, dtype=torch.float32, device=dev)
+        tt.peers = parallel.make_peer_exchange(dev, stride=_lib.XCHG_STACK_STRIDE)
+        nccl = multi and tt.peers is None
 
         def episode():
             reset()
             for _ in range(env.max_steps):
-                tt.tick(self.w, self.w_target, self.exp_avg, self.exp_avg_sq, world.state, returns, hits)
+                if not multi:
+                    tt.tick(self.w, self.w_target, self.exp_avg, self.exp_avg_sq, world.state, returns, hits)
+                    continue
+                tt.grad_phase(self.w, self.w_target, world.state, returns, hits)
+                if nccl:
+                    torch.distributed.all_reduce(tt.grad_loss)
+                tt.apply_phase(self.w, self.w_target, self.exp_avg, self.exp_avg_sq)
             tt.episode_end(returns, hits, stats, config["epsilon"], config["epsilon_decay"], config["min_epsilon"])
 
         _run_episodes(episode, episodes, bool(config.get("cuda_graph", True)), dev)

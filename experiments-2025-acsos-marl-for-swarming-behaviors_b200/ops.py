@@ -496,7 +496,10 @@ class StackTrainTick(_TrainCursor):
     draw + gradient, the partial-sum reduce and clip + Adam (+ target sync) with the cursor on the device, so the ticks
     of an episode capture into a CUDA graph.  ``reward``: None for the world's own reward (GoTo / ObstacleAvoidance), or
     a Flocking / Cohesion ``reward_spec`` on the GoTo world (Flocking: ``shaping`` f32[B,N,2] is its memory, in / out).
-    One GPU: no phase split, no peer exchange."""
+    Data-parallel trainers run the tick as ``grad_phase`` + ``apply_phase`` (swarm_train_tick_stack_grad /
+    swarm_train_tick_stack_apply): with ``self.peers`` set (``parallel.PeerExchange`` of ``_lib.XCHG_STACK_STRIDE``
+    words) the gradient phase sums ``grad_loss`` over the ranks itself, otherwise the trainer all-reduces ``grad_loss``
+    between the phases."""
 
     def __init__(self, cfg: SwarmConfig, spec, ring: ReplayRing, *, graphs_per_update: int = 32,
                  update_target_every: int = 200, gamma: float = 0.99, loss_scale: Optional[float] = None, lr: float = 1e-3,
@@ -518,11 +521,44 @@ class StackTrainTick(_TrainCursor):
         self.loss = self.grad_loss[self.count:]
         self._ws_bytes = int(lib().swarm_dqn_stack_workspace_bytes(C.byref(cfg), C.byref(spec), G))
         self.workspace = torch.empty(max(self._ws_bytes, 256), dtype=torch.uint8, device=dev)
+        self.peers = None          # parallel.PeerExchange: sum grad_loss over the ranks inside grad_phase
+
+    def _expect_weights(self, **tensors) -> None:
+        for name, t in tensors.items():
+            _expect(t, torch.float32, self.count, name)
+
+    # -- the two phases -------------------------------------------------------------------------------
+    def grad_phase(self, weights: torch.Tensor, target: torch.Tensor, state: torch.Tensor, returns: torch.Tensor,
+                   hits: torch.Tensor) -> None:
+        """Rollout tick, slot draw + gradient and the partial-sum reduce; with ``self.peers`` set, ``grad_loss`` then
+        holds the sum over the ranks."""
+        self._expect_weights(weights=weights, target=target)
+        peers = None
+        if self.peers is not None:
+            if self.peers.stride != _lib.XCHG_STACK_STRIDE:        # the kernel writes SWARM_XCHG_STACK_STRIDE-word slots
+                raise ValueError(f"a stacked tick exchanges through a PeerExchange of stride {_lib.XCHG_STACK_STRIDE}, "
+                                 f"got {self.peers.stride}")
+            peers = C.byref(self.peers.struct)
+        check(lib().swarm_train_tick_stack_grad(C.byref(self.cfg), C.byref(self.spec), C.byref(self.hyper),
+                                                C.addressof(self._reward) if self._reward is not None else None,
+                                                ptr(self._shaping), ptr(self.ctl), ptr(weights), ptr(target), ptr(state),
+                                                ptr(returns), ptr(hits), C.byref(self._rstruct), ptr(self.indices),
+                                                ptr(self.grad_loss), ptr(self.workspace), self._ws_bytes, peers,
+                                                stream_ptr(state.device)))
+
+    def apply_phase(self, weights: torch.Tensor, target: torch.Tensor, exp_avg: torch.Tensor,
+                    exp_avg_sq: torch.Tensor) -> None:
+        """clip + Adam on ``grad_loss`` (+ target sync) and the cursor advance."""
+        self._expect_weights(weights=weights, target=target, exp_avg=exp_avg, exp_avg_sq=exp_avg_sq)
+        check(lib().swarm_train_tick_stack_apply(C.byref(self.cfg), C.byref(self.spec), C.byref(self.hyper), ptr(self.ctl),
+                                                 ptr(weights), ptr(target), ptr(exp_avg), ptr(exp_avg_sq),
+                                                 ptr(self.grad_loss), self.ring.capacity, stream_ptr(weights.device)))
 
     def tick(self, weights: torch.Tensor, target: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor,
              state: torch.Tensor, returns: torch.Tensor, hits: torch.Tensor) -> None:
-        for name, t in (("weights", weights), ("target", target), ("exp_avg", exp_avg), ("exp_avg_sq", exp_avg_sq)):
-            _expect(t, torch.float32, self.count, name)
+        """Both phases as one library call (swarm_train_tick_stack), without the peer exchange: the same bits as
+        ``grad_phase`` + ``apply_phase``, for one GPU."""
+        self._expect_weights(weights=weights, target=target, exp_avg=exp_avg, exp_avg_sq=exp_avg_sq)
         check(lib().swarm_train_tick_stack(C.byref(self.cfg), C.byref(self.spec), C.byref(self.hyper),
                                            C.addressof(self._reward) if self._reward is not None else None,
                                            ptr(self._shaping), ptr(self.ctl), ptr(weights), ptr(target), ptr(exp_avg),

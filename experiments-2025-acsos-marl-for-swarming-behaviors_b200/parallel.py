@@ -14,6 +14,8 @@ from typing import Optional, Tuple
 import torch
 import torch.distributed as dist
 
+from . import _lib
+
 
 @dataclass(frozen=True)
 class EnvShard:
@@ -102,20 +104,21 @@ def require_equal_shards(num_envs: int, ring_size: int, ring_position: int, ring
 
 
 class PeerExchange:
-    """Symmetric (peer-mapped) receive buffers for the fused one-shot PUSH all-reduce of ``swarm_train_tick_apply``:
-    every rank allocates uint64[2][world][1680] with ``torch.distributed._symmetric_memory`` and maps all peers' copies
-    over NVLink; the clip + Adam kernel writes its partial gradient (value + epoch per 8-byte word) into its slot of
-    every peer's buffer, polls its own local buffer for the peers' words and sums the partials in rank order.  PyTorch
-    only provides the allocation / rendezvous plumbing."""
+    """Symmetric (peer-mapped) receive buffers for the fused one-shot PUSH all-reduce of the data-parallel ticks: every
+    rank allocates uint64[2][world][stride] with ``torch.distributed._symmetric_memory`` and maps all peers' copies over
+    NVLink; the exchanging kernel writes its partial gradient (value + epoch per 8-byte word) into its slot of every
+    peer's buffer, polls its own local buffer for the peers' words and sums the partials in rank order.  ``stride`` is
+    ``_lib.XCHG_STRIDE`` for the one-layer GCN (``swarm_train_tick_apply``) and ``_lib.XCHG_STACK_STRIDE`` for stacked
+    networks (``swarm_train_tick_stack_grad``).  PyTorch only provides the allocation / rendezvous plumbing."""
 
-    def __init__(self, device, group=None):
+    def __init__(self, device, group=None, stride: int = _lib.XCHG_STRIDE):
         import torch.distributed._symmetric_memory as symm_mem
-        from . import _lib
         group = group if group is not None else dist.group.WORLD
         world = dist.get_world_size(group)
         if world > 16:
             raise ValueError("PeerExchange supports up to 16 ranks")
-        self.buf = symm_mem.empty(2 * world * _lib.XCHG_STRIDE, dtype=torch.int64, device=device)
+        self.stride = int(stride)
+        self.buf = symm_mem.empty(2 * world * self.stride, dtype=torch.int64, device=device)
         self.buf.zero_()
         self.handle = symm_mem.rendezvous(self.buf, group)
         st = _lib.SwarmPeerExchange()
@@ -127,13 +130,14 @@ class PeerExchange:
         dist.barrier(group)            # every rank's buffer is zeroed before anybody's kernel can write into it
 
 
-def make_peer_exchange(device) -> Optional["PeerExchange"]:
-    """PeerExchange when data-parallel on GPUs with symmetric memory available, else None (the trainer then keeps the
-    NCCL all-reduce between the two tick phases).  SWARM_PEER_ALLREDUCE=0 forces the NCCL path."""
+def make_peer_exchange(device, stride: int = _lib.XCHG_STRIDE) -> Optional["PeerExchange"]:
+    """PeerExchange (of ``stride`` words per rank and parity) when data-parallel on GPUs with symmetric memory
+    available, else None (the trainer then keeps the NCCL all-reduce between the two tick phases).
+    SWARM_PEER_ALLREDUCE=0 forces the NCCL path."""
     if world_size() <= 1 or os.environ.get("SWARM_PEER_ALLREDUCE", "1") == "0":
         return None
     try:
-        return PeerExchange(device)
+        return PeerExchange(device, stride=stride)
     except Exception as exc:           # no NVLink peer mapping / symmetric memory on this box
         import warnings
         warnings.warn(f"peer-memory gradient exchange unavailable ({exc!r}); using the NCCL all-reduce")

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SWARM_ABI_VERSION 8
+#define SWARM_ABI_VERSION 9
 
 enum { SWARM_SCENARIO_GOTO = 0, SWARM_SCENARIO_OBSTACLE_AVOIDANCE = 1 };
 /* SWARM_GRAPH_RADIUS is an EXTENSION (the reference has no radius graph, SURVEY.md Appendix C): the complete-graph
@@ -431,13 +431,46 @@ int swarm_train_tick(const SwarmConfig* cfg, const SwarmTrainHyper* hyper, Swarm
  * (shaping float[B][N][2] required, read and written back) or a Cohesion spec selects that reward on the GoTo world;
  * hyper->flocking must be NULL.  grad float[count + 1] = gradient (count = swarm_stack_weight_count(spec)), then the
  * loss.  2 <= n_agents <= 128, graphs and spec as for swarm_dqn_stack_grad.  workspace:
- * swarm_dqn_stack_workspace_bytes(cfg, spec, G).  One GPU: there is no two-phase split and no peer exchange. */
+ * swarm_dqn_stack_workspace_bytes(cfg, spec, G).  A data-parallel trainer calls the same tick as its two phases,
+ * swarm_train_tick_stack_grad (launches 1-3, with the gradient exchange) and swarm_train_tick_stack_apply (launch 4). */
 struct SwarmStackSpec;
 int swarm_train_tick_stack(const SwarmConfig* cfg, const struct SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
                            const struct SwarmRewardSpec* reward, float* shaping, SwarmTrainCtl* ctl, float* weights,
                            float* target_weights, float* exp_avg, float* exp_avg_sq, float* state, float* returns,
                            int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
                            int64_t workspace_bytes, void* stream);
+
+/* swarm_train_tick_stack as two calls, for data-parallel training: swarm_train_tick_stack_grad followed by
+ * swarm_train_tick_stack_apply gives the same bits as swarm_train_tick_stack.
+ *
+ * Phase 1 runs launches 1-3 of swarm_train_tick_stack (rollout tick, slot draw + gradient, partial-sum reduce) and takes
+ * the same arguments, with the same checks, minus exp_avg / exp_avg_sq.  grad is float[count + 1] (gradient, then the
+ * loss), so a trainer without peer memory all-reduces one buffer between the phases.  With peers != NULL the reduce
+ * launch also sums grad and loss over the ranks: the peer exchange of swarm_train_tick_apply (word = epoch << 32 | float
+ * bits, own buffer first, polls of the local buffer, rank-order sums), on a buffer of
+ * uint64[2][world_size][SWARM_XCHG_STACK_STRIDE], zero-initialised; when the call returns on the stream, grad holds
+ * the sum over the ranks on every rank.  Ticks that do not update exchange nothing.
+ *
+ * The exchange sits in the grad phase here, while the one-layer tick's sits in swarm_train_tick_apply: the stacked
+ * reduce launch runs one gradient element per thread over ceil((count + 1) / 256) CTAs (2 for the Flocking
+ * checkpoint's 409 weights, 20 for the largest stack), so every thread pushes one word per peer and polls world_size
+ * words -- the shape of the one-layer exchange that measured fastest.  The stacked clip + Adam kernel is one CTA holding
+ * up to 20 elements per thread; polling there would put 20 x world_size loads in one thread's registers.
+ *
+ * All ranks must run the same number of envs, start from the same ring fill and call the phases for the same ticks. */
+enum { SWARM_XCHG_STACK_STRIDE = 5040 };     /* >= 5 033 weights of the largest stack + the loss, a multiple of 8 */
+int swarm_train_tick_stack_grad(const SwarmConfig* cfg, const struct SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                                const struct SwarmRewardSpec* reward, float* shaping, SwarmTrainCtl* ctl,
+                                const float* weights, const float* target_weights, float* state, float* returns,
+                                int32_t* hits, const SwarmReplay* ring, int64_t* indices, float* grad, void* workspace,
+                                int64_t workspace_bytes, const SwarmPeerExchange* peers, void* stream);
+
+/* Phase 2: launch 4 of swarm_train_tick_stack -- clip_grad_norm_ + Adam on grad (the gradient phase's, reduced over the
+ * ranks), the target sync and the cursor advance; ring_capacity as ring->capacity of phase 1.  Rejects every cfg, spec
+ * and hyper that swarm_train_tick_stack rejects. */
+int swarm_train_tick_stack_apply(const SwarmConfig* cfg, const struct SwarmStackSpec* spec, const SwarmTrainHyper* hyper,
+                                 SwarmTrainCtl* ctl, float* weights, float* target_weights, float* exp_avg,
+                                 float* exp_avg_sq, const float* grad, int64_t ring_capacity, void* stream);
 
 /* ---- device-side episode boundary (SURVEY.md 8f rank 2) -------------------------------------------------------
  * The reference resets with one CPU torch.normal draw per episode (go_to:84-88, oa:100-102) and does its episode
